@@ -2,7 +2,7 @@
 """Benchmark of the RoadSurf per-point simulation loop on B200.
 
     python bench.py --gpus N --steps K --warmup W [--impl reference]
-                    [--workload c4|c3|c5] [--scaling weak|strong] [--inproc]
+                    [--workload c4|c3|c5] [--scaling weak|strong] [--inproc] [--dump-outputs DIR]
 
 Workloads (BASELINE.json configs; `config.workload` in the output names the one that ran):
   c4 (default)  "synthetic 10^7-point km-scale road grid, 24 h forecast, sharded across 1/2/4/8 B200":
@@ -29,6 +29,12 @@ e2e     same metric through the C ABI with HOST buffers (roadsurf_run_host_soa):
         it exists) on all host cores, on the first 10240 points of the very workload the GPU arm runs.
 --inproc  one process drives all N GPUs through the library's own `ngpus` argument
         (roadsurf_run_host_soa(..., ngpus=N)) and compares the result with the one-GPU run.
+--dump-outputs DIR  after the timed steps, write what the last one computed as DIR/<name>.npy (float64):
+        every output variable [points, hourly slots], the status words [points], for the coupled workloads
+        (c3, c2) the end-of-run state planes [points, planes] (ground-layer temperatures first), and the
+        indices of the points written [points].  Points are a fixed, seeded sample of rank 0's points (with
+        --inproc: of all points), all of them when they fit 64 MB.  The inputs depend on the arguments alone,
+        so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -73,7 +79,14 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-full-config", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU paths only")
+    return args
 
 
 def rank_points(args, world):
@@ -311,6 +324,38 @@ def kernel_traffic_per_point_step():
         return None, None
 
 
+DUMP_LIMIT_BYTES = 64_000_000
+DUMP_SEED = 20191206
+
+
+def dump_outputs(directory, out, status, npoints, state=None, limit=DUMP_LIMIT_BYTES):
+    """Writes out [O_NVAR, n_out, >= npoints], status [>= npoints] and, when given, the end-of-run state
+    [planes, >= npoints] of a fixed, seeded sample of the points (all of them when they fit `limit` bytes) as
+    directory/<output name>.npy [points, n_out], status.npy, state.npy [points, planes] and point_index.npy
+    [points], all float64 (status words and indices are exact there)."""
+    import numpy as np
+    import torch
+    from roadsurf_b200 import lib
+    n_out = out.shape[1]
+    planes = 0 if state is None else state.shape[0]
+    headers = 128 * (len(lib.O_NAMES) + 3)
+    n = min(npoints, (limit - headers) // ((len(lib.O_NAMES) * n_out + planes + 2) * 8))
+    if n < npoints:
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(npoints, n, replace=False))
+    else:
+        idx = np.arange(npoints)
+    sel = torch.from_numpy(idx).to(out.device)
+    o = out[:len(lib.O_NAMES)].index_select(2, sel).cpu().numpy()
+    arrays = {name: np.ascontiguousarray(o[v].T) for v, name in enumerate(lib.O_NAMES)}
+    arrays["status"] = status.index_select(0, sel.to(status.device)).cpu().numpy().astype(np.float64)
+    if state is not None:
+        arrays["state"] = np.ascontiguousarray(state.index_select(1, sel.to(state.device)).cpu().numpy().T)
+    arrays["point_index"] = idx.astype(np.float64)
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def run_inproc(args):
     """One process, N GPUs through the product's own `ngpus` argument; compared with the 1-GPU result."""
     import torch
@@ -343,6 +388,8 @@ def run_inproc(args):
         call(n, out, status, statics=handle)
     dt = time.perf_counter() - t0
     st = lib.last_batch_stats()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out, status, total)
     same = all(bool(torch.equal(out[:, :, k * P:(k + 1) * P], ref_out)) and bool(torch.equal(status[k * P:(k + 1) * P], ref_status))
                for k in range(n))
     lib.release_statics(handle)
@@ -420,6 +467,8 @@ def main():
     bl_per_step = float(cnt[lib.CNT_BL_ITERATIONS]) / max(1.0, float(cnt[lib.CNT_EXECUTED_STEPS]))
     launch = lib.last_launch()
     gpu_launches = launch["launches_total"] - launches_before
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, db.out, db.status, P, state=db.state)
 
     # ---- end to end through the C ABI with host buffers ------------------------------------------
     e2e = None
