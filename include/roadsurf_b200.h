@@ -148,7 +148,9 @@ enum
   RS_ST_BL_NOT_CONVERGED = 32,/* BLCond iteration hit MaxIter (src/BoundaryLayer.f90:98-101) */
   RS_ST_SOLAR_GEOMETRY = 64,  /* the reference would `stop` (src/SunPosition.f90:144-146,176-178) */
   RS_ST_BAD_WINDOW = 128,     /* device SoA entry: coupling windows differ inside one warp */
-  RS_ST_NOT_RUN = 256         /* point was skipped (bad settings) */
+  RS_ST_NOT_RUN = 256,        /* point was skipped (bad settings) */
+  RS_ST_BAD_FORK = 512        /* ensemble member: its relaxation targets differ from the ones the shared
+                                 analysis already used (see roadsurf_run_ensemble_device); with RS_ST_NOT_RUN */
 };
 
 /* Return codes. */
@@ -563,6 +565,152 @@ void roadsurf_last_launch(RsLaunchInfo* info);
 
 /* Library version string. */
 const char* roadsurf_version(void);
+
+/* ------------------------------------------------------------------------------------------ */
+/* Part 3: ensemble runs                                                                        */
+/* ------------------------------------------------------------------------------------------ */
+
+/* An ensemble over P stations and M members shares the analysis period: the steps [1, F - 1] run once
+ * per station, the state is then forked on the device into P * M member lanes, the forecast [F, SimLen]
+ * runs per member, and the member outputs are reduced to ensemble statistics on the device.  F
+ * (`fork_step`, 1-based) is the first step that reads member forcing.  The results are bit for bit
+ * those of P * M independent roadsurf_run_device runs in which lane p * M + m gets station p's forcing
+ * before F and member m's from F on: every output slot, status word and end-of-run state plane.
+ *
+ * Member lanes are station-major: lane = p * M + m, `ld_members` a multiple of 32 >= P * M.
+ *
+ * Where F may sit:
+ *   - coupling: the whole window [start, end + 1] of every coupled station lies before F
+ *     (F >= couplingIndexI + 2), and coupled stations share ONE window (members of different stations
+ *     share warps; a lane whose window differs from its warp's is flagged RS_ST_BAD_WINDOW);
+ *   - forcing_mode 1: F - 1 or F - 2 (0-based steps) is a record time, so that no record feeds both the
+ *     shared and the member part with different values.  r_f = the last record at or before step F - 1;
+ *     member record tensors start at r_f, and their slot 0 is written by the library from the shared
+ *     records (the caller fills records r_f + 1 ...).  F = forecast step + 2 (example1's shape: the
+ *     coupling window ends at the forecast-start record) is admissible;
+ *   - forcing_mode 0: any F in [2, SimLen]; member forcing is [SimLen - F + 1][nvar][ld_members]
+ *     (record 0 = step F);
+ *   - forcing_mode 2: RS_ERR_UNSUPPORTED (example2's rule interpolates across up to 180 minutes, which
+ *     would reach across F).
+ * Relaxation targets are read at the first forecast step, so they are per member (`member_relax`).
+ *   - The prefix runs on a library-owned copy of the station targets; where the station's fail the
+ *     kernel's range test and a member's pass, the copy takes the first passing member's targets, so that
+ *     the latch at InitLenI happens wherever a member will relax.
+ *   - After the fork, member lanes whose own targets fail the test get the three latch planes reset to
+ *     their initial value (the independent run never latched).
+ *   - A station with InitLenI <= F - 2 has applied its targets inside the shared part already: its
+ *     members whose targets differ from those get RS_ST_BAD_FORK | RS_ST_NOT_RUN and are not run. */
+
+#define RS_ENS_MAX_MEMBERS 128
+#define RS_ENS_MAX_QUANTILES 8
+#define RS_ENS_MAX_THRESHOLDS 8
+
+/* Planes of the statistics tensor, followed by one plane per requested quantile. */
+enum
+{
+  RS_ENS_NVALID = 0, /* number of valid members (value == value and > -9000), as a double */
+  RS_ENS_MEAN,       /* left-to-right sum in member order from +0.0, divided by n */
+  RS_ENS_STD,        /* population standard deviation (ddof = 0), two passes in member order */
+  RS_ENS_MIN,
+  RS_ENS_MAX,
+  RS_ENS_NFIXED = 5
+};
+
+/* Comparison of an exceedance probability. */
+enum
+{
+  RS_ENS_LT = 0,
+  RS_ENS_LE,
+  RS_ENS_GT,
+  RS_ENS_GE
+};
+
+typedef struct RsEnsembleThreshold
+{
+  int plane;    /* output plane (RS_O_*) */
+  int op;       /* RS_ENS_LT / LE / GT / GE */
+  double value; /* P(member value op value) = count / n */
+} RsEnsembleThreshold;
+
+/* What the statistics kernel computes per (station, output slot, plane) besides the fixed planes.
+ * Quantile q of the valid values sorted y_0 <= ... <= y_{n-1}: h = (n - 1) q, i = floor(h), t = h - i;
+ * y_i if t == 0 or i == n - 1, else y_i + t (y_{i+1} - y_i).  Where n == 0 every value but RS_ENS_NVALID (0.0)
+ * is -9999.0, the probabilities too. */
+typedef struct RsEnsembleStatsSpec
+{
+  int n_quantiles;  /* 0 .. RS_ENS_MAX_QUANTILES */
+  int n_thresholds; /* 0 .. RS_ENS_MAX_THRESHOLDS */
+  double quantiles[RS_ENS_MAX_QUANTILES];
+  RsEnsembleThreshold thresholds[RS_ENS_MAX_THRESHOLDS];
+} RsEnsembleStatsSpec;
+
+/* A device-resident ensemble (DEVICE pointers on the current device). */
+typedef struct RsEnsembleBatch
+{
+  RsDeviceBatch shared;          /* the P stations, as for roadsurf_run_device with the whole run's time axis:
+                                    `state` is required, `scratch` too when coupled, `out` holds the output
+                                    slots of the steps before F (out_slot0 = 0), forcing is the stations'
+                                    forcing up to F - 1 (forcing_mode 1: the full record axis; the values of
+                                    records after r_f + 1 are never read).  step_begin, step_end,
+                                    forcing_step0, out_slot0 and expand_* must be 0.  `local` is not modified */
+  int members;                   /* M, 1 .. RS_ENS_MAX_MEMBERS */
+  int fork_step;                 /* F, 1-based, 2 <= F <= sim_len */
+  int ld_members;                /* multiple of 32, >= P * M */
+  double* member_forcing;        /* mode 1: [n_records - r_f][nvar][ld_members], slot 0 written by the library;
+                                    mode 0: [sim_len - F + 1][nvar][ld_members] */
+  const double* member_relax;    /* [3][ld_members]: tair, VZ, RH relaxation targets per member, or NULL
+                                    (the station's targets for every member) */
+  double* member_local;          /* [RS_L_NLOCAL][ld_members]                        (written) */
+  double* member_horizons;       /* [360][ld_members] when shared.horizons != NULL    (written) */
+  double* member_state;          /* [RS_STATE_NPLANES(NLayers)][ld_members]; also the work space of the
+                                    prefix's copy of shared.local, so it needs RS_L_NLOCAL * shared.ld
+                                    doubles at least                                  (written) */
+  double* member_scratch;        /* [RS_SCRATCH_NPLANES(NLayers)][ld_members] when coupled (written) */
+  int* member_status;            /* [ld_members]                                      (written) */
+  double* member_out;            /* [out_nvar][n_out_members][ld_members]: slot 0 = the first output slot of
+                                    a step >= F                                       (written) */
+  int n_out_members;             /* slot dimension of member_out, stats and prob: >= the number of output slots of
+                                    the steps [F, sim_len]; the statistics cover those slots, later ones are
+                                    neither read nor written */
+  const int* member_order;       /* optional [ld_members] thread permutation, as RsDeviceBatch.order */
+  RsEnsembleStatsSpec spec;
+  double* stats;                 /* [RS_ENS_NFIXED + n_quantiles][out_nvar][n_out_members][shared.ld], or NULL */
+  double* prob;                  /* [n_thresholds][n_out_members][shared.ld], or NULL */
+} RsEnsembleBatch;
+
+/* Runs an ensemble asynchronously on `stream`: (1) the prefix [1, F - 1] of the P stations (with lane
+ * compaction between coupling iterations when shared.coupling_window_end is set, under the rules of
+ * roadsurf_run_device), (2) the fork into the member lanes, (3) the member launch [F, sim_len], a resumed
+ * launch of the step kernel, (4) the statistics (when stats or prob is given).  shared.counters, if
+ * given, accumulate both launches.  forcing_mode 1 reads record_step back once (a small synchronous
+ * copy on `stream`) to check F against the record grid.  Returns RS_OK or an error code. */
+int roadsurf_run_ensemble_device(const RsEnsembleBatch* batch, void* stream);
+
+/* The statistics kernel on its own, over any station-major member tensor member_out
+ * [out_nvar][n_out][ld_members] (lane p * members + m): stats [RS_ENS_NFIXED + n_quantiles][out_nvar][n_out][ld],
+ * prob [n_thresholds][n_out][ld] (either may be NULL).  Device pointers; asynchronous on `stream`. */
+int roadsurf_ensemble_stats(const double* member_out, int out_nvar, int n_out, int ld_members, int npoints,
+                            int members, const RsEnsembleStatsSpec* spec, double* stats, double* prob, int ld,
+                            void* stream);
+
+/* Host form on the current device, forcing_mode 1 only.  `shared` is the stations' host SoA batch
+ * (as for roadsurf_run_host_soa, with the full record axis); its `out`, if not NULL, receives the
+ * station outputs of the steps before F, [RS_O_NVAR][n_out_pre][P] with n_out_pre = ceil((F - 1) /
+ * out_stride); `status` is not written.  member_records [n_records - r_f - 1][nvar][P * M] are the
+ * members' records r_f + 1 ... (lane p * M + m).  With use_relaxation == 1 the member relaxation targets are
+ * derived by the rule of roadsurf_read_input_derive_records from each member's records (the station's up to r_f)
+ * and `latest_obs_index` (per station, as passed to that call; NULL = no observation anywhere, targets
+ * -9999.9); shared->local is expected to hold what that call derived for the stations.
+ * Coupled stations must share one window (RS_ERR_UNSUPPORTED otherwise).  Outputs: stats
+ * [RS_ENS_NFIXED + n_quantiles][RS_O_NVAR][n_out_m][P], prob [n_thresholds][n_out_m][P] and, when not NULL,
+ * member_out [RS_O_NVAR][n_out_m][P * M] and member_status [P * M], with n_out_m the output slots of the
+ * steps [F, sim_len].  Stations are processed in chunks that fit device memory and the option
+ * "max_points_per_device_batch" (counted in member lanes).  Synchronous; roadsurf_last_batch_stats reports
+ * the phases (kernel_ms: prefix, fork, members and statistics). */
+int roadsurf_run_ensemble_host_soa(const RsHostBatch* shared, const double* member_records, int members,
+                                   int fork_step, const int* latest_obs_index, const RsEnsembleStatsSpec* spec, double* stats, double* prob,
+                                   double* member_out, int* member_status, const InputSettings* settings,
+                                   const InputParameters* params);
 
 #ifdef __cplusplus
 }

@@ -6,7 +6,7 @@ import subprocess
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, os.environ.get("ROADSURF_B200_LIBNAME", "libroadsurf_b200.so"))
-SOURCES = ("rs_kernel.cu", "rs_host.cu", "rs_model.cpp")
+SOURCES = ("rs_kernel.cu", "rs_host.cu", "rs_ensemble.cu", "rs_model.cpp")
 
 # -fmad=false: no FMA contraction, like a generic x86-64 gfortran build of the reference, so that
 # threshold decisions (freeze/melt limits, minimum storages) are taken on identically rounded values.

@@ -60,6 +60,25 @@ enum
                          // once and stop after step window_end (state written)
 };
 
+// Per-point state planes (RsArgsCold.state, RS_STATE_NPLANES(N) of them): Tmp(0:N+1) in planes 0 .. N+1, then,
+// as offsets from plane N + 2: Ts, Wat, Snow, Ice, Ice2, Dep, Q2Melt, T4Melt, Evap, Alb (0 .. 9), the relaxation
+// latches TairInitEnd, VZInitEnd, RhzInitEnd (RS_SP_LATCH + 0 .. 2), SwCof, LwCof, SWcorr, LWcorr, lastObs, and the
+// flag word (RS_SP_FLAGS).
+enum
+{
+  RS_SP_LATCH = 10,
+  RS_SP_FLAGS = 18
+};
+// Flag word: coupling iterations + 1 in bits 0..7, then these bits.
+enum
+{
+  RS_FL_CPL_FAILED = 8,
+  RS_FL_START_AGAIN = 9,
+  RS_FL_IN_CPL = 10,
+  RS_FL_ALIVE = 11,
+  RS_FL_FAILED = 12
+};
+
 // Host-callable launchers (rs_kernel.cu).  Return a cudaError_t as int.
 int rs_upload_model(const RsModel* m);
 int rs_launch_solar(const int* tf, int sim_len, double* table, void* stream);

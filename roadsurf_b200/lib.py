@@ -17,6 +17,7 @@ LIB_PATH = os.path.join(HERE, os.environ.get("ROADSURF_B200_LIBNAME", "libroadsu
 # enums of include/roadsurf_b200.h
 ST_FAILED, ST_BAD_INPUT, ST_ABNORMAL_TSURF, ST_COUPLING_USED, ST_COUPLING_FAILED = 1, 2, 4, 8, 16
 ST_BL_NOT_CONVERGED, ST_SOLAR_GEOMETRY, ST_BAD_WINDOW, ST_NOT_RUN = 32, 64, 128, 256
+ST_BAD_FORK = 512
 F_NVAR, F_NVAR_DEPTH = 11, 12
 F_NAMES = ("tair", "tdew", "VZ", "Rhz", "prec", "SW", "LW", "SW_dir", "LW_net", "TSurfObs", "PrecPhase",
            "Depth")
@@ -38,7 +39,12 @@ EXPORTS = ("runsimulation", "roadsurf_last_error", "roadsurf_device_count", "roa
            "roadsurf_session_open", "roadsurf_step", "roadsurf_session_fetch", "roadsurf_session_set_chunk",
            "roadsurf_session_done", "roadsurf_session_close", "roadsurf_expand_records",
            "roadsurf_sun_position",
-           "roadsurf_version")
+           "roadsurf_version",
+           "roadsurf_run_ensemble_device", "roadsurf_ensemble_stats", "roadsurf_run_ensemble_host_soa")
+ENS_MAX_MEMBERS, ENS_MAX_QUANTILES, ENS_MAX_THRESHOLDS = 128, 8, 8
+ENS_NVALID, ENS_MEAN, ENS_STD, ENS_MIN, ENS_MAX, ENS_NFIXED = range(6)
+ENS_LT, ENS_LE, ENS_GT, ENS_GE = range(4)
+ENS_OPS = {"<": ENS_LT, "<=": ENS_LE, ">": ENS_GT, ">=": ENS_GE}
 
 
 def state_nplanes(nlayers):
@@ -81,6 +87,38 @@ class RsHostBatch(C.Structure):
                 ("forcing", C.c_void_p), ("record_step", C.c_void_p), ("time_fields", C.c_void_p),
                 ("local", C.c_void_p), ("horizons", C.c_void_p), ("out", C.c_void_p), ("status", C.c_void_p),
                 ("coupling_window_end", C.c_int), ("statics", C.c_void_p)]
+
+
+class RsEnsembleThreshold(C.Structure):
+    _fields_ = [("plane", C.c_int), ("op", C.c_int), ("value", C.c_double)]
+
+
+class RsEnsembleStatsSpec(C.Structure):
+    _fields_ = [("n_quantiles", C.c_int), ("n_thresholds", C.c_int), ("quantiles", C.c_double * 8),
+                ("thresholds", RsEnsembleThreshold * 8)]
+
+
+class RsEnsembleBatch(C.Structure):
+    _fields_ = [("shared", RsDeviceBatch), ("members", C.c_int), ("fork_step", C.c_int), ("ld_members", C.c_int),
+                ("member_forcing", C.c_void_p), ("member_relax", C.c_void_p), ("member_local", C.c_void_p),
+                ("member_horizons", C.c_void_p), ("member_state", C.c_void_p), ("member_scratch", C.c_void_p),
+                ("member_status", C.c_void_p), ("member_out", C.c_void_p), ("n_out_members", C.c_int),
+                ("member_order", C.c_void_p), ("spec", RsEnsembleStatsSpec), ("stats", C.c_void_p),
+                ("prob", C.c_void_p)]
+
+
+def stats_spec(quantiles=(), thresholds=()):
+    """RsEnsembleStatsSpec from quantiles [q, ...] and thresholds [(plane, op, value), ...], op one of
+    "<", "<=", ">", ">=" (or an ENS_* code)."""
+    quantiles, thresholds = list(quantiles), list(thresholds)
+    if len(quantiles) > ENS_MAX_QUANTILES or len(thresholds) > ENS_MAX_THRESHOLDS:
+        raise ValueError("at most 8 quantiles and 8 thresholds")
+    sp = RsEnsembleStatsSpec(n_quantiles=len(quantiles), n_thresholds=len(thresholds))
+    for j, q in enumerate(quantiles):
+        sp.quantiles[j] = float(q)
+    for j, (plane, op, value) in enumerate(thresholds):
+        sp.thresholds[j] = RsEnsembleThreshold(int(plane), ENS_OPS.get(op, op), float(value))
+    return sp
 
 
 class RoadSurfError(RuntimeError):
@@ -147,6 +185,15 @@ def load():
     lib.roadsurf_default_settings.argtypes = [P(IS), C.c_int, C.c_double]
     lib.roadsurf_default_settings.restype = None
     lib.roadsurf_last_launch.argtypes = [P(RsLaunchInfo)]
+    lib.roadsurf_run_ensemble_device.argtypes = [P(RsEnsembleBatch), C.c_void_p]
+    lib.roadsurf_run_ensemble_device.restype = C.c_int
+    lib.roadsurf_ensemble_stats.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                                            P(RsEnsembleStatsSpec), C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
+    lib.roadsurf_ensemble_stats.restype = C.c_int
+    lib.roadsurf_run_ensemble_host_soa.argtypes = [P(RsHostBatch), C.c_void_p, C.c_int, C.c_int, C.c_void_p,
+                                                   P(RsEnsembleStatsSpec), C.c_void_p, C.c_void_p, C.c_void_p,
+                                                   C.c_void_p, P(IS), P(IPa)]
+    lib.roadsurf_run_ensemble_host_soa.restype = C.c_int
     _lib = lib
     return lib
 
@@ -528,3 +575,181 @@ def read_input_derive_records(forcing, record_step, settings, forecast_step, loc
 
 def release_workspace():
     load().roadsurf_release_workspace()
+
+
+# ---- ensemble runs (include/roadsurf_b200.h, part 3) ---------------------------------------------------
+
+def _ptr(x):
+    if x is None:
+        return None
+    return x.data_ptr() if hasattr(x, "data_ptr") else x.ctypes.data
+
+
+def ensemble_stats(member_out, npoints, members, spec, stream=None):
+    """roadsurf_ensemble_stats on a torch CUDA tensor member_out [out_nvar, n_out, ld_members] (lane
+    p * members + m).  Returns (stats [5 + n_quantiles, out_nvar, n_out, npoints],
+    prob [n_thresholds, n_out, npoints]) as CUDA tensors (synchronised)."""
+    import torch
+    out_nvar, n_out, ldm = member_out.shape
+    ld = max(32, (npoints + 31) // 32 * 32)
+    f64 = dict(dtype=torch.float64, device=member_out.device)
+    stats = torch.full((ENS_NFIXED + spec.n_quantiles, out_nvar, n_out, ld), 12345.0, **f64)
+    prob = torch.full((max(1, spec.n_thresholds), n_out, ld), 12345.0, **f64)
+    st = stream if stream is not None else torch.cuda.current_stream()
+    _check(load().roadsurf_ensemble_stats(member_out.data_ptr(), out_nvar, n_out, ldm, int(npoints), int(members),
+                                          C.byref(spec), stats.data_ptr(), prob.data_ptr(), ld,
+                                          C.c_void_p(st.cuda_stream)))
+    torch.cuda.synchronize()
+    return stats[..., :npoints], prob[:spec.n_thresholds, :, :npoints]
+
+
+def fork_record(record_step, fork_step):
+    """r_f: the last record at or before 0-based step fork_step - 1."""
+    rs = np.asarray(record_step)
+    return int(np.nonzero(rs <= fork_step - 1)[0][-1])
+
+
+class EnsembleBatch:
+    """Device-resident ensemble (RsEnsembleBatch): a shared DeviceBatch of the P stations (it needs
+    state=True, and coupling=True when the model couples) plus the member tensors of P * M lanes,
+    station-major (lane p * M + m).  Fill `shared` as usual (records / full-resolution forcing, time axis,
+    statics), then the members' forcing with load_member_records / load_member_forcing, and run()."""
+
+    def __init__(self, shared, members, fork_step, stats_spec=None, member_relax=False, extra_slots=0):
+        import torch
+        self.torch = torch
+        self.shared = shared
+        self.members, self.fork_step = int(members), int(fork_step)
+        P, M = shared.npoints, self.members
+        self.ld_members = max(32, (P * M + 31) // 32 * 32)
+        ldm, dev = self.ld_members, shared.local.device
+        f64 = dict(dtype=torch.float64, device=dev)
+        if shared.coarse:
+            rs = shared.record_step.cpu().numpy()
+            self.r_f = fork_record(rs, self.fork_step)
+            n_rec_m = shared.n_records - self.r_f
+        else:
+            self.r_f = None
+            n_rec_m = shared.sim_len - self.fork_step + 1
+        self.member_forcing = torch.zeros((n_rec_m, shared.nvar, ldm), **f64)
+        self.member_relax = torch.full((3, ldm), -9999.0, **f64) if member_relax else None
+        self.member_local = torch.zeros((L_NLOCAL, ldm), **f64)
+        self.member_horizons = torch.zeros((360, ldm), **f64) if shared.horizons is not None else None
+        self.member_state = torch.zeros((state_nplanes(shared.nlayers), ldm), **f64)
+        self.member_scratch = (torch.zeros((scratch_nplanes(shared.nlayers), ldm), **f64)
+                               if shared.scratch is not None else None)
+        self.member_status = torch.zeros(ldm, dtype=torch.int32, device=dev)
+        # output slots: the steps before F in shared.out, the steps [F, sim_len] in member_out
+        k0 = self.fork_step - 1 - shared.out_start
+        self.slot0 = (k0 + shared.out_stride - 1) // shared.out_stride if k0 > 0 else 0
+        self.n_slots = max(1, shared.n_out - self.slot0)      # output slots of the steps [F, sim_len]
+        self.n_out_members = self.n_slots + int(extra_slots)  # slot dimension of member_out / stats / prob
+        self.member_out = torch.empty((shared.out_nvar, self.n_out_members, ldm), **f64)
+        self.member_order = None
+        self.spec = stats_spec if stats_spec is not None else RsEnsembleStatsSpec()
+        ld = shared.ld
+        self.stats_t = torch.empty((ENS_NFIXED + self.spec.n_quantiles, shared.out_nvar, self.n_out_members, ld), **f64)
+        self.prob_t = torch.empty((max(1, self.spec.n_thresholds), self.n_out_members, ld), **f64)
+
+    def load_member_records(self, member_recs):
+        """Coarse records of every member (synth.Records with the full record axis, one per member, equal
+        to the station records up to r_f): records r_f + 1 ... go into the member tensor (slot 0 is
+        written by the library)."""
+        P, M = self.shared.npoints, self.members
+        assert self.shared.coarse and len(member_recs) == M
+        names = ("tair", "tdew", "VZ", "Rhz", "prec", "SW", "LW", "SW_dir", "LW_net", "TSurfObs", "PrecPhase")
+        host = np.zeros(tuple(self.member_forcing.shape))
+        for m, rec in enumerate(member_recs):
+            for v, name in enumerate(names):
+                host[1:, v, m:P * M:M] = getattr(rec, name)[:, self.r_f + 1:].T
+        if self.shared.nvar > F_NVAR:
+            host[:, F_NVAR, :] = -9999.9
+        self.member_forcing.copy_(self.torch.from_numpy(host))
+
+    def load_member_forcing(self, lane_arrays):
+        """Full-resolution member forcing: steps F ... of a PointArrays whose point p * M + m is member m of
+        station p (abi.PointArrays with P * M points)."""
+        P, M, F = self.shared.npoints, self.members, self.fork_step
+        assert not self.shared.coarse and lane_arrays.npoints == P * M
+        host = np.zeros(tuple(self.member_forcing.shape))
+        for v in range(self.shared.nvar):
+            host[:, v, :P * M] = getattr(lane_arrays, F_NAMES[v])[:, F - 1:].T
+        self.member_forcing.copy_(self.torch.from_numpy(host))
+
+    def set_member_relax(self, relax):
+        """relax [3, P * M]: tair, VZ, RH relaxation targets per member lane."""
+        assert self.member_relax is not None
+        self.member_relax[:, :relax.shape[1]] = self.torch.as_tensor(np.asarray(relax, dtype=np.float64))
+
+    def build_member_order(self, stream=None):
+        """roadsurf_order_points over the member statics (needs a first run for member_local)."""
+        st = stream if stream is not None else self.torch.cuda.current_stream()
+        self.member_order = self.torch.empty(self.ld_members, dtype=self.torch.int32, device=self.member_local.device)
+        _check(load().roadsurf_order_points(C.c_void_p(self.member_local.data_ptr()), self.ld_members,
+                                            self.shared.npoints * self.members,
+                                            C.c_void_p(self.member_order.data_ptr()), C.c_void_p(st.cuda_stream)))
+
+    def descriptor(self, stats=True):
+        s = self.shared
+        sd = s.descriptor()
+        sd.coupling_window_end = s.coupling_window_end
+        return RsEnsembleBatch(shared=sd, members=self.members, fork_step=self.fork_step,
+                               ld_members=self.ld_members, member_forcing=_ptr(self.member_forcing),
+                               member_relax=_ptr(self.member_relax), member_local=_ptr(self.member_local),
+                               member_horizons=_ptr(self.member_horizons), member_state=_ptr(self.member_state),
+                               member_scratch=_ptr(self.member_scratch), member_status=_ptr(self.member_status),
+                               member_out=_ptr(self.member_out), n_out_members=self.n_out_members,
+                               member_order=_ptr(self.member_order), spec=self.spec,
+                               stats=_ptr(self.stats_t) if stats else None,
+                               prob=_ptr(self.prob_t) if (stats and self.spec.n_thresholds) else None)
+
+    def run(self, stream=None, stats=True):
+        """Asynchronous: prefix, fork, members, statistics on `stream` (default: the current stream)."""
+        st = stream if stream is not None else self.torch.cuda.current_stream()
+        desc = self.descriptor(stats)
+        _check(load().roadsurf_run_ensemble_device(C.byref(desc), C.c_void_p(st.cuda_stream)))
+
+    def member_outputs(self):
+        """dict name -> numpy [P, M, n_out_members] of the member slots."""
+        P, M = self.shared.npoints, self.members
+        o = self.member_out.cpu().numpy()[:, :self.n_slots, :P * M]
+        names = O_NAMES + (O_NAMES_EXT if self.shared.out_nvar == O_NVAR_EXT else ())
+        return {name: np.ascontiguousarray(o[v].T.reshape(P, M, -1)) for v, name in enumerate(names)}
+
+    def stats(self):
+        """(stats [5 + n_quantiles, out_nvar, n_slots, P], prob [n_thresholds, n_slots, P]) numpy: the slots of the
+        steps [F, sim_len]."""
+        P, n = self.shared.npoints, self.n_slots
+        return (self.stats_t.cpu().numpy()[:, :, :n, :P],
+                self.prob_t.cpu().numpy()[:self.spec.n_thresholds, :n, :P])
+
+
+def run_ensemble_host_soa(settings, params, forcing, record_step, time_fields, local, member_records, members,
+                          fork_step, spec, horizons=None, out_stride=1, coupling_window_end=0, out=None,
+                          member_out=False, member_status=False, latest_obs_index=None):
+    """roadsurf_run_ensemble_host_soa on host arrays: forcing [n_records, nvar, P], record_step [n_records],
+    local [L_NLOCAL, P], member_records [n_records - r_f - 1, nvar, P * members], latest_obs_index [P] int32 (the
+    relaxation rule of read_input_derive_records; None = no observations).  Returns a dict with
+    stats [5 + nq, 6, n_out_m, P], prob [nt, n_out_m, P] and, when asked for, member_out [6, n_out_m, P * M]
+    and member_status [P * M]."""
+    n_records, nvar, npoints = forcing.shape
+    sim_len = time_fields.shape[1]
+    k0 = fork_step - 1
+    slot0 = (k0 + out_stride - 1) // out_stride
+    n_m = (sim_len + out_stride - 1) // out_stride - slot0
+    res = dict(stats=np.zeros((ENS_NFIXED + spec.n_quantiles, O_NVAR, n_m, npoints)),
+               prob=np.zeros((spec.n_thresholds, n_m, npoints)))
+    if member_out:
+        res["member_out"] = np.zeros((O_NVAR, n_m, npoints * members))
+    if member_status:
+        res["member_status"] = np.zeros(npoints * members, dtype=np.int32)
+    hb = RsHostBatch(npoints=npoints, sim_len=sim_len, forcing_mode=1, n_records=n_records, nvar=nvar,
+                     out_stride=out_stride, forcing=_ptr(forcing), record_step=_ptr(record_step),
+                     time_fields=_ptr(time_fields), local=_ptr(local), horizons=_ptr(horizons), out=_ptr(out),
+                     coupling_window_end=int(coupling_window_end))
+    lat = None if latest_obs_index is None else np.ascontiguousarray(latest_obs_index, dtype=np.int32)
+    _check(load().roadsurf_run_ensemble_host_soa(C.byref(hb), _ptr(member_records), int(members), int(fork_step),
+                                                 _ptr(lat), C.byref(spec), _ptr(res["stats"]), _ptr(res["prob"]),
+                                                 _ptr(res.get("member_out")), _ptr(res.get("member_status")),
+                                                 C.byref(settings), C.byref(params)))
+    return res

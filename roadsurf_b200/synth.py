@@ -258,3 +258,49 @@ def make_case(npoints, hours, seed, analysis_hours=0, use_coupling=0, use_relaxa
     pa, settings, params = case_from_records(rec, hours, analysis_hours, use_coupling, use_relaxation, dt,
                                              nlayers, start, **(settings_kw or {}))
     return pa, settings, params, rec
+
+
+def member_records(base, members, r_f, seed, start, dt_secs=30.0, sky_view_fraction=0.3):
+    """`members` record sets of an ensemble forked after record r_f: member m equals `base` (drawn by
+    draw_records with the same seed, start, spacing and sky-view fraction) in every record up to r_f and
+    in its observations, and is a perturbed draw (draw_records(..., member_perturbation=m)) after r_f.
+    Each is a full record set: it is what an independent run of member m reads."""
+    record_secs = float(base.record_step[1] - base.record_step[0]) * dt_secs
+    out = []
+    for m in range(members):
+        r = draw_records(base.npoints, base.nrec, seed, start, record_secs, dt_secs, int(base.record_step[0]),
+                         sky_view_fraction, member_perturbation=m)
+        for v in RECORD_VARS:
+            getattr(r, v)[:, :r_f + 1] = getattr(base, v)[:, :r_f + 1]
+        r.TSurfObs[:] = base.TSurfObs
+        r.lat[:], r.lon[:], r.sky_view[:], r.horizons[:] = base.lat, base.lon, base.sky_view, base.horizons
+        r.record_step[:] = base.record_step
+        r.obs_bias = None
+        out.append(r)
+    return out
+
+
+def member_record_tensor(member_recs, r_f):
+    """The members' records r_f + 1 ... as [n_records - r_f - 1][11][P * M] (lane p * M + m), the layout of
+    roadsurf_run_ensemble_host_soa's member_records."""
+    M, P, nrec = len(member_recs), member_recs[0].npoints, member_recs[0].nrec
+    out = np.zeros((nrec - r_f - 1, len(RECORD_VARS), P * M))
+    for m, r in enumerate(member_recs):
+        for v, name in enumerate(RECORD_VARS):
+            out[:, v, m::M] = getattr(r, name)[:, r_f + 1:].T
+    return out
+
+
+def lane_records(member_recs):
+    """One Records object whose point p * M + m is member m of station p: the input of P * M independent
+    runs."""
+    M, P, nrec = len(member_recs), member_recs[0].npoints, member_recs[0].nrec
+    r = Records(P * M, nrec)
+    for v in RECORD_VARS:
+        a = getattr(r, v)
+        for m, mr in enumerate(member_recs):
+            a[m::M] = getattr(mr, v)
+    for m, mr in enumerate(member_recs):
+        r.lat[m::M], r.lon[m::M], r.sky_view[m::M], r.horizons[m::M] = mr.lat, mr.lon, mr.sky_view, mr.horizons
+    r.record_step[:] = member_recs[0].record_step
+    return r
