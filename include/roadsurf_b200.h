@@ -468,14 +468,19 @@ int roadsurf_session_set_chunk(void* session, int steps);
 int roadsurf_session_done(void* session);
 void roadsurf_session_close(void* session);
 
-/* Pack kernels for callers that hold point-major data on the device:
- * src[point][n] (row stride `src_ld` elements) -> dst plane [n][ld].  Asynchronous. */
+/* Pack kernels for callers that hold point-major data on the device (device pointers, asynchronous):
+ * to_soa:   src[point][n] (row stride `src_ld` elements) -> dst[n][ld];
+ * from_soa: src[n][ld] -> dst[point][n] (row stride `dst_ld` elements).
+ * Values are copied bit for bit; elements outside [0, npoints) x [0, n) are not touched.  Any npoints and n
+ * that fit the int arguments are accepted.  RS_ERR_BAD_ARGUMENT for null pointers, npoints < 0, n < 0,
+ * ld < npoints or a point-major row stride < n; npoints == 0 or n == 0 is RS_OK without a launch. */
 int roadsurf_transpose_to_soa(const double* src, int64_t src_ld, int npoints, int n, double* dst,
                               int ld, void* stream);
 int roadsurf_transpose_from_soa(const double* src, int ld, int npoints, int n, double* dst,
                                 int64_t dst_ld, void* stream);
 
-/* Fill n doubles with `value` (used for the -9999.0 output pre-fill).  Asynchronous. */
+/* Fill n doubles with `value` (used for the -9999.0 output pre-fill).  Asynchronous.  RS_ERR_BAD_ARGUMENT
+ * for a null dst or n < 0; n == 0 is RS_OK without a launch. */
 int roadsurf_fill(double* dst, int64_t n, double value, void* stream);
 
 /* Measure the fp64 FMA throughput of the current device (TFLOP/s, FMA = 2 flop) with a
@@ -496,6 +501,30 @@ int roadsurf_expand_records(const RsDeviceBatch* records, int rule, int step_beg
  * reference would `stop`.  Asynchronous on `stream`. */
 int roadsurf_sun_position(const int* time_fields, int n_steps, const double* lat, const double* lon, int npoints,
                           double* elevation, double* azimuth, void* stream);
+
+/* Math primitives of the step kernel, for roadsurf_eval_primitive. */
+enum
+{
+  RS_PRIM_EXP = 0,                 /* exp: libm's algorithm, device-library exp outside its fast path */
+  RS_PRIM_EXP_SMEM = 1,            /*   ... tables read from shared memory (latency body) */
+  RS_PRIM_LOG = 2,                 /* log: libm's algorithm, device-library log outside its fast path */
+  RS_PRIM_LOG_SMEM = 3,            /*   ... tables read from shared memory */
+  RS_PRIM_EXP_FLAT = 4,            /* the branch-free exp of the early saturation pressures, with its fallback */
+  RS_PRIM_EXP_FLAT_SMEM = 5,       /*   ... tables read from shared memory */
+  RS_PRIM_PSIH_UNSTABLE = 6,       /* -2 log((1 + sqrt(1 - 16 a)) / 2), the unstable stability correction */
+  RS_PRIM_PSIH_UNSTABLE_SMEM = 7,  /*   ... tables read from shared memory */
+  RS_PRIM_FRCP = 8,                /* 1 / b (the values of a are ignored) */
+  RS_PRIM_FDIV = 9,                /* a / b */
+  RS_PRIM_DIV_CONST = 10,          /* a / b through the constant-divisor form, reciprocal RN(1 / b) */
+  RS_PRIM_N = 11
+};
+
+/* Diagnostic: out[k] = fn(a[k]) or fn(a[k], b[k]) for k < n, exactly as the step kernel evaluates the primitive
+ * (same code, same build flags).  Device pointers; b is read by RS_PRIM_FRCP, _FDIV and _DIV_CONST only and may be
+ * NULL otherwise.  Asynchronous on `stream`.  RS_ERR_BAD_ARGUMENT for an unknown fn, n < 0, a null a / out, or a
+ * null b where fn reads it; n == 0 is RS_OK without a launch.  The domains on which the results equal the host's
+ * libm and IEEE division bit for bit are listed in DESIGN.md section 4. */
+int roadsurf_eval_primitive(int fn, const double* a, const double* b, double* out, int64_t n, void* stream);
 
 /* Builds RsDeviceBatch.order on the device: the slots of points without sky-view radiation first, those
  * with it last, original order kept inside both classes.  `local` is the batch's [RS_L_NLOCAL][ld]

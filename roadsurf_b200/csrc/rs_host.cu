@@ -1721,6 +1721,9 @@ int roadsurf_order_points(const double* local, int ld, int npoints, int* order, 
 int roadsurf_transpose_to_soa(const double* src, int64_t src_ld, int npoints, int n, double* dst, int ld,
                               void* stream)
 {
+  if (!src || !dst || npoints < 0 || n < 0 || ld < npoints || src_ld < n)
+    return fail(RS_ERR_BAD_ARGUMENT, "bad arguments (ld >= npoints >= 0, src_ld >= n >= 0)");
+  if (npoints == 0 || n == 0) return RS_OK;
   CU(static_cast<cudaError_t>(rs_launch_transpose_to_soa(src, src_ld, npoints, n, dst, ld, stream)));
   ++g_launches_total;
   return RS_OK;
@@ -1729,13 +1732,29 @@ int roadsurf_transpose_to_soa(const double* src, int64_t src_ld, int npoints, in
 int roadsurf_transpose_from_soa(const double* src, int ld, int npoints, int n, double* dst, int64_t dst_ld,
                                 void* stream)
 {
+  if (!src || !dst || npoints < 0 || n < 0 || ld < npoints || dst_ld < n)
+    return fail(RS_ERR_BAD_ARGUMENT, "bad arguments (ld >= npoints >= 0, dst_ld >= n >= 0)");
+  if (npoints == 0 || n == 0) return RS_OK;
   CU(static_cast<cudaError_t>(rs_launch_transpose_from_soa(src, ld, npoints, n, dst, dst_ld, stream)));
+  ++g_launches_total;
+  return RS_OK;
+}
+
+int roadsurf_eval_primitive(int fn, const double* a, const double* b, double* out, int64_t n, void* stream)
+{
+  const bool binary = fn == RS_PRIM_FRCP || fn == RS_PRIM_FDIV || fn == RS_PRIM_DIV_CONST;
+  if (fn < 0 || fn >= RS_PRIM_N || n < 0 || !a || !out || (binary && !b))
+    return fail(RS_ERR_BAD_ARGUMENT, "bad arguments (fn one of RS_PRIM_*, n >= 0, b where fn reads it)");
+  if (n == 0) return RS_OK;
+  CU(static_cast<cudaError_t>(rs_launch_eval_primitive(fn, a, b, out, n, stream)));
   ++g_launches_total;
   return RS_OK;
 }
 
 int roadsurf_fill(double* dst, int64_t n, double value, void* stream)
 {
+  if (!dst || n < 0) return fail(RS_ERR_BAD_ARGUMENT, "bad arguments (dst, n >= 0)");
+  if (n == 0) return RS_OK;
   CU(static_cast<cudaError_t>(rs_launch_fill(dst, n, value, stream)));
   ++g_launches_total;
   return RS_OK;

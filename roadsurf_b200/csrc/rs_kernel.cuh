@@ -102,6 +102,7 @@ int rs_launch_transpose_to_soa(const double* src, long long src_ld, int npoints,
 int rs_launch_transpose_from_soa(const double* src, int ld, int npoints, int n, double* dst,
                                  long long dst_ld, void* stream);
 int rs_launch_fill(double* dst, long long n, double value, void* stream);
+int rs_launch_eval_primitive(int fn, const double* a, const double* b, double* out, long long n, void* stream);
 int rs_launch_pack_forcing(const double* stage, int npoints_chunk, int p0, int sim_len, int nvar,
                            double* forcing, int ld, void* stream);
 int rs_launch_unpack_out(const double* out, int ld, int n_out, int p0, int npoints_chunk,

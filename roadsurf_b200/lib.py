@@ -38,9 +38,11 @@ EXPORTS = ("runsimulation", "roadsurf_last_error", "roadsurf_device_count", "roa
            "roadsurf_last_launch", "roadsurf_prepare_statics", "roadsurf_release_statics",
            "roadsurf_session_open", "roadsurf_step", "roadsurf_session_fetch", "roadsurf_session_set_chunk",
            "roadsurf_session_done", "roadsurf_session_close", "roadsurf_expand_records",
-           "roadsurf_sun_position",
+           "roadsurf_sun_position", "roadsurf_eval_primitive",
            "roadsurf_version",
            "roadsurf_run_ensemble_device", "roadsurf_ensemble_stats", "roadsurf_run_ensemble_host_soa")
+(PRIM_EXP, PRIM_EXP_SMEM, PRIM_LOG, PRIM_LOG_SMEM, PRIM_EXP_FLAT, PRIM_EXP_FLAT_SMEM, PRIM_PSIH_UNSTABLE,
+ PRIM_PSIH_UNSTABLE_SMEM, PRIM_FRCP, PRIM_FDIV, PRIM_DIV_CONST, PRIM_N) = range(12)
 ENS_MAX_MEMBERS, ENS_MAX_QUANTILES, ENS_MAX_THRESHOLDS = 128, 8, 8
 ENS_NVALID, ENS_MEAN, ENS_STD, ENS_MIN, ENS_MAX, ENS_NFIXED = range(6)
 ENS_LT, ENS_LE, ENS_GT, ENS_GE = range(4)
@@ -168,6 +170,8 @@ def load():
     lib.roadsurf_transpose_from_soa.restype = C.c_int
     lib.roadsurf_fill.argtypes = [C.c_void_p, C.c_int64, C.c_double, C.c_void_p]
     lib.roadsurf_fill.restype = C.c_int
+    lib.roadsurf_eval_primitive.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]
+    lib.roadsurf_eval_primitive.restype = C.c_int
     lib.roadsurf_measure_fp64_tflops.argtypes = [C.c_int]
     lib.roadsurf_measure_fp64_tflops.restype = C.c_double
     lib.roadsurf_set_option.argtypes = [C.c_char_p, C.c_int]
@@ -533,6 +537,23 @@ def sun_position(time_fields, lat, lon):
     _check(lib.roadsurf_sun_position(time_fields.data_ptr(), n, lat.data_ptr(), lon.data_ptr(), npts, elev.data_ptr(),
                                      azim.data_ptr(), C.c_void_p(torch.cuda.current_stream().cuda_stream)))
     return elev, azim
+
+
+def eval_primitive(fn, a, b=None):
+    """roadsurf_eval_primitive: one of the step kernel's math primitives (PRIM_*) elementwise on float64 torch
+    CUDA tensors a (and b for PRIM_FRCP / _FDIV / _DIV_CONST, same shape).  Returns the result tensor
+    (synchronised)."""
+    import torch
+    a = a.contiguous()
+    if b is not None:
+        b = b.contiguous()
+        assert b.shape == a.shape and b.dtype == torch.float64
+    assert a.dtype == torch.float64 and a.is_cuda
+    out = torch.empty_like(a)
+    _check(load().roadsurf_eval_primitive(int(fn), a.data_ptr(), None if b is None else b.data_ptr(), out.data_ptr(),
+                                          a.numel(), C.c_void_p(torch.cuda.current_stream().cuda_stream)))
+    torch.cuda.synchronize()
+    return out
 
 
 def set_option(name, value):

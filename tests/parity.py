@@ -6,10 +6,25 @@ S_TOL = 1e-3   # mm  (storage terms within 1e-3 mm water equivalent)
 STORAGES = ("SnowOut", "WaterOut", "IceOut", "DepositOut", "Ice2Out")
 
 
+def bit_mismatch(a, b):
+    """Elementwise: True where two float64 arrays differ as bit patterns.  Zeros must carry the same sign;
+    any two NaNs are equal (the device and x86 produce different NaN payloads for invalid operations)."""
+    a = np.ascontiguousarray(a, dtype=np.float64)
+    b = np.ascontiguousarray(b, dtype=np.float64)
+    return (a.view(np.uint64) != b.view(np.uint64)) & ~(np.isnan(a) & np.isnan(b))
+
+
+def same_bits(a, b):
+    """Two float64 arrays of one shape are equal bit for bit (under the NaN rule of bit_mismatch)."""
+    a, b = np.asarray(a), np.asarray(b)
+    return a.shape == b.shape and not bit_mismatch(a, b).any()
+
+
 def compare(out_a, out_b):
     """Per-point comparison of two output dicts name -> [npoints, n].  Returns a dict with the max
     temperature / storage differences over matching points, the mismatch fraction (points with any
-    value beyond tolerance: threshold-induced state flips) and the index of the worst point."""
+    value beyond tolerance: threshold-induced state flips), the index of the worst point and the number of
+    values that differ as bit patterns (bit_identical: none does)."""
     dT = np.abs(out_a["TsurfOut"] - out_b["TsurfOut"])
     dS = np.zeros_like(dT)
     for n in STORAGES:
@@ -18,7 +33,7 @@ def compare(out_a, out_b):
     good = ~bad
     differing = 0
     for n in ("TsurfOut",) + STORAGES:
-        differing += int((~((out_a[n] == out_b[n]) | (np.isnan(out_a[n]) & np.isnan(out_b[n])))).sum())
+        differing += int(bit_mismatch(out_a[n], out_b[n]).sum())
     res = {
         "bit_identical": differing == 0,
         "differing_values": differing,

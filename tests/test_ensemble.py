@@ -11,6 +11,7 @@ import tempfile
 import numpy as np
 import pytest
 
+from parity import same_bits
 from roadsurf_b200 import abi, lib, synth
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -264,12 +265,11 @@ def _assert_equivalent(ens, db, lanes=None):
     s0 = ens.slot0
     ind = db.out.cpu().numpy()
     pre = ens.shared.out.cpu().numpy()[:, :s0, :P]
-    assert np.array_equal(ind[:, :s0, lanes], pre[:, :, lanes // M], equal_nan=True), "slots before the fork"
+    assert same_bits(ind[:, :s0, lanes], pre[:, :, lanes // M]), "slots before the fork"
     mo = ens.member_out.cpu().numpy()
-    assert np.array_equal(ind[:, s0:, lanes], mo[:, :ind.shape[1] - s0, lanes], equal_nan=True), "member slots"
+    assert same_bits(ind[:, s0:, lanes], mo[:, :ind.shape[1] - s0, lanes]), "member slots"
     assert np.array_equal(db.status.cpu().numpy()[lanes], ens.member_status.cpu().numpy()[lanes])
-    assert np.array_equal(db.state.cpu().numpy()[:, lanes], ens.member_state.cpu().numpy()[:, lanes],
-                          equal_nan=True), "state planes"
+    assert same_bits(db.state.cpu().numpy()[:, lanes], ens.member_state.cpu().numpy()[:, lanes]), "state planes"
 
 
 @pytest.mark.gpu

@@ -11,7 +11,7 @@ import numpy as np
 import pytest
 
 from golden_io import CASE_NAMES, load_case
-from parity import S_TOL, T_TOL, compare
+from parity import S_TOL, T_TOL, compare, same_bits
 from roadsurf_b200 import abi, synth
 
 pytestmark = pytest.mark.gpu
@@ -846,14 +846,14 @@ def _assert_outputs_and_ground_state_exact(rslib, oracle, arrays, settings, para
     db = _coarse_run_with_state(rslib, arrays, rec, coupling)
     got = db.outputs()
     for k in ref.out:
-        assert np.array_equal(got[k], ref.out[k], equal_nan=True), k
+        assert same_bits(got[k], ref.out[k]), k
     assert np.array_equal(db.status.cpu().numpy()[:n], st_cpu)
     state = db.state.cpu().numpy()
     ok = (st_cpu & rslib.ST_FAILED) == 0
     assert ok.sum() > 0.9 * n
     # a failed point stops before its last step: its state is not the end-of-run state on either side
-    assert np.array_equal(state[:nl + 2, :n].T[ok], tmp_cpu[ok]), "ground temperatures Tmp(0:N+1)"
-    assert np.array_equal(state[nl + 2:nl + 12, :n].T[ok], surf_cpu[ok]), "surface state"
+    assert same_bits(state[:nl + 2, :n].T[ok], tmp_cpu[ok]), "ground temperatures Tmp(0:N+1)"
+    assert same_bits(state[nl + 2:nl + 12, :n].T[ok], surf_cpu[ok]), "surface state"
     return db, ref
 
 
@@ -869,7 +869,7 @@ def test_48h_coupled_forecast_config3_like_exact_including_ground_temperatures(r
     # the same through the reference-facing batched entry (full-resolution host arrays)
     st = rslib.run_batch(arrays, settings, params)
     for k in ref.out:
-        assert np.array_equal(arrays.out[k], ref.out[k], equal_nan=True), k
+        assert same_bits(arrays.out[k], ref.out[k]), k
 
 
 def test_74h_example1_span_401_points_exact(rslib, oracle):
@@ -893,7 +893,7 @@ def test_ground_temperatures_match_for_other_layer_counts(rslib, oracle):
         db.load_point_arrays(arrays)
         db.run()
         torch.cuda.synchronize()
-        assert np.array_equal(db.state.cpu().numpy()[:nl + 2, :96].T, tmp_cpu), nl
+        assert same_bits(db.state.cpu().numpy()[:nl + 2, :96].T, tmp_cpu), nl
 
 
 def test_records_that_end_inside_the_run_are_not_extrapolated(rslib, oracle):
