@@ -633,6 +633,8 @@ const char* roadsurf_version(void);
 #define RS_ENS_MAX_MEMBERS 128
 #define RS_ENS_MAX_QUANTILES 8
 #define RS_ENS_MAX_THRESHOLDS 8
+#define RS_ENS_MAX_EVENTS 8
+#define RS_ENS_MAX_CONDITIONS 4
 
 /* Planes of the statistics tensor, followed by one plane per requested quantile. */
 enum
@@ -661,16 +663,39 @@ typedef struct RsEnsembleThreshold
   double value; /* P(member value op value) = count / n */
 } RsEnsembleThreshold;
 
+/* A compound event over a window of output slots: "the conditions all hold at one slot or more of the
+ * window".  Let S be the member output slots the statistics cover (the output slots of the steps [F, sim_len];
+ * slots from S to n_out_members are neither read nor written).  For station p, member m, slot s < S:
+ *   - valid: member m is valid for the event at s when every plane referenced by the conditions holds a valid
+ *     value (value == value and > -9000) at every slot of the window W(s) = [s, min(s + window, S) - 1].  The
+ *     window is truncated at the last member slot, not padded;
+ *   - hit: the conjunction of the conditions holds at one slot or more of W(s), the comparisons those of
+ *     RsEnsembleThreshold;
+ *   - result: prob[n_thresholds + e][s][p] = (valid members that hit) / (valid members), computed as
+ *     (double)count / (double)n like the thresholds; -9999.0 where no member is valid.
+ * A one-condition event with window 1 equals the threshold with the same (plane, op, value) bit for bit.
+ * Example, "wet road freezing within the next 3 h" at hourly output slots: window 3, conditions
+ * {RS_O_TSURF, RS_ENS_LT, 0.0} and {RS_O_WATER, RS_ENS_GT, x}. */
+typedef struct RsEnsembleEvent
+{
+  int n_conditions;                                      /* 1 .. RS_ENS_MAX_CONDITIONS, combined with AND */
+  int window;                                            /* >= 1 output slots */
+  RsEnsembleThreshold conditions[RS_ENS_MAX_CONDITIONS]; /* plane, op, value: as for thresholds */
+} RsEnsembleEvent;
+
 /* What the statistics kernel computes per (station, output slot, plane) besides the fixed planes.
  * Quantile q of the valid values sorted y_0 <= ... <= y_{n-1}: h = (n - 1) q, i = floor(h), t = h - i;
  * y_i if t == 0 or i == n - 1, else y_i + t (y_{i+1} - y_i).  Where n == 0 every value but RS_ENS_NVALID (0.0)
- * is -9999.0, the probabilities too. */
+ * is -9999.0, the probabilities too.  The event probabilities follow the thresholds in `prob`: event j is
+ * plane n_thresholds + j. */
 typedef struct RsEnsembleStatsSpec
 {
   int n_quantiles;  /* 0 .. RS_ENS_MAX_QUANTILES */
   int n_thresholds; /* 0 .. RS_ENS_MAX_THRESHOLDS */
   double quantiles[RS_ENS_MAX_QUANTILES];
   RsEnsembleThreshold thresholds[RS_ENS_MAX_THRESHOLDS];
+  int n_events;     /* 0 .. RS_ENS_MAX_EVENTS */
+  RsEnsembleEvent events[RS_ENS_MAX_EVENTS];
 } RsEnsembleStatsSpec;
 
 /* A device-resident ensemble (DEVICE pointers on the current device). */
@@ -704,20 +729,22 @@ typedef struct RsEnsembleBatch
   const int* member_order;       /* optional [ld_members] thread permutation, as RsDeviceBatch.order */
   RsEnsembleStatsSpec spec;
   double* stats;                 /* [RS_ENS_NFIXED + n_quantiles][out_nvar][n_out_members][shared.ld], or NULL */
-  double* prob;                  /* [n_thresholds][n_out_members][shared.ld], or NULL */
+  double* prob;                  /* [n_thresholds + n_events][n_out_members][shared.ld], or NULL */
 } RsEnsembleBatch;
 
 /* Runs an ensemble asynchronously on `stream`: (1) the prefix [1, F - 1] of the P stations (with lane
  * compaction between coupling iterations when shared.coupling_window_end is set, under the rules of
  * roadsurf_run_device), (2) the fork into the member lanes, (3) the member launch [F, sim_len], a resumed
- * launch of the step kernel, (4) the statistics (when stats or prob is given).  shared.counters, if
+ * launch of the step kernel, (4) the statistics (when stats or prob is given) and, when prob is given and
+ * spec.n_events > 0, the event probabilities.  shared.counters, if
  * given, accumulate both launches.  forcing_mode 1 reads record_step back once (a small synchronous
  * copy on `stream`) to check F against the record grid.  Returns RS_OK or an error code. */
 int roadsurf_run_ensemble_device(const RsEnsembleBatch* batch, void* stream);
 
 /* The statistics kernel on its own, over any station-major member tensor member_out
  * [out_nvar][n_out][ld_members] (lane p * members + m): stats [RS_ENS_NFIXED + n_quantiles][out_nvar][n_out][ld],
- * prob [n_thresholds][n_out][ld] (either may be NULL).  Device pointers; asynchronous on `stream`. */
+ * prob [n_thresholds + n_events][n_out][ld] (either may be NULL); the events read the planes they name over the
+ * n_out slots.  Device pointers; asynchronous on `stream`. */
 int roadsurf_ensemble_stats(const double* member_out, int out_nvar, int n_out, int ld_members, int npoints,
                             int members, const RsEnsembleStatsSpec* spec, double* stats, double* prob, int ld,
                             void* stream);
@@ -731,11 +758,11 @@ int roadsurf_ensemble_stats(const double* member_out, int out_nvar, int n_out, i
  * and `latest_obs_index` (per station, as passed to that call; NULL = no observation anywhere, targets
  * -9999.9); shared->local is expected to hold what that call derived for the stations.
  * Coupled stations must share one window (RS_ERR_UNSUPPORTED otherwise).  Outputs: stats
- * [RS_ENS_NFIXED + n_quantiles][RS_O_NVAR][n_out_m][P], prob [n_thresholds][n_out_m][P] and, when not NULL,
+ * [RS_ENS_NFIXED + n_quantiles][RS_O_NVAR][n_out_m][P], prob [n_thresholds + n_events][n_out_m][P] and, when not NULL,
  * member_out [RS_O_NVAR][n_out_m][P * M] and member_status [P * M], with n_out_m the output slots of the
  * steps [F, sim_len].  Stations are processed in chunks that fit device memory and the option
  * "max_points_per_device_batch" (counted in member lanes).  Synchronous; roadsurf_last_batch_stats reports
- * the phases (kernel_ms: prefix, fork, members and statistics). */
+ * the phases (kernel_ms: prefix, fork, members, statistics and events). */
 int roadsurf_run_ensemble_host_soa(const RsHostBatch* shared, const double* member_records, int members,
                                    int fork_step, const int* latest_obs_index, const RsEnsembleStatsSpec* spec, double* stats, double* prob,
                                    double* member_out, int* member_status, const InputSettings* settings,

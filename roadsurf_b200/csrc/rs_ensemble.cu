@@ -1,7 +1,13 @@
 // rs_ensemble.cu -- the kernels of an ensemble run (roadsurf_run_ensemble_device): the prefix's copy of the
-// station statics, the fork of the station state into the member lanes, and the ensemble statistics.
+// station statics, the fork of the station state into the member lanes, the ensemble statistics and the event
+// probabilities.
 // Member lanes are station-major: lane = p * members + m.
 #include <cuda_runtime.h>
+
+#include <algorithm>
+#include <climits>
+#include <cstddef>
+#include <cstring>
 
 #include "rs_ensemble.cuh"
 #include "rs_kernel.cuh"
@@ -125,13 +131,24 @@ __global__ void rs_ens_fork_kernel(const RsForkArgs f)
 
 constexpr int kStatsBlock = 64;
 
+// The statistics kernel's part of RsEnsembleStatsSpec (everything before the events): its parameter keeps the
+// layout it had before the events were appended to the spec.
+struct StatsKernelSpec
+{
+  int n_quantiles;
+  int n_thresholds;
+  double quantiles[RS_ENS_MAX_QUANTILES];
+  RsEnsembleThreshold thresholds[RS_ENS_MAX_THRESHOLDS];
+};
+static_assert(offsetof(RsEnsembleStatsSpec, n_events) == sizeof(StatsKernelSpec), "spec prefix");
+
 __device__ __forceinline__ bool valid_value(double x) { return x == x && x > -9000.0; }
 
 // One thread per (station, output slot, plane); the valid member values go to this thread's column of shared
 // memory (y[k * kStatsBlock]), in member order, and are sorted there for the quantiles.
 __global__ void __launch_bounds__(kStatsBlock) rs_ens_stats_kernel(const double* __restrict__ mout, int out_nvar, int n_slots,
                                                                    int mo_slots, int ldm, int npoints, int members,
-                                                                   const RsEnsembleStatsSpec spec, double* __restrict__ stats,
+                                                                   const StatsKernelSpec spec, double* __restrict__ stats,
                                                                    double* __restrict__ prob, int st_slots, int ld)
 {
   extern __shared__ double ens_smem[];
@@ -225,6 +242,80 @@ __global__ void __launch_bounds__(kStatsBlock) rs_ens_stats_kernel(const double*
     o[(RS_ENS_NFIXED + j) * plane] = (tt == 0.0 || i == n - 1) ? yi : yi + tt * (y[(i + 1) * kStatsBlock] - yi);
   }
 }
+
+constexpr int kEventsBlock = 64;
+// Threads the event launch aims for before it splits the slots into tiles (about one resident wave on the B200).
+constexpr long long kEventsTargetThreads = 1LL << 17;
+
+// Event probabilities (RsEnsembleEvent).  A block is 64 stations of one event and one tile of output slots
+// [s0, s1); the event index varies fastest over the blocks, so that the events of a station block run side by
+// side and share the member values through L2.  Each thread scans the slots backward from the end of the tile's
+// last window, min(s1 + window - 1, S), down to s0, and loops over the members at each slot, reading every member
+// value of a referenced plane once per event and tile.  Per member it keeps, in its column of shared memory
+// (st[m * kEventsBlock]), the first slot >= s with an invalid value (x) and the first with a valid hit (y); the
+// window W(s) = [s, wend] is then valid when x > wend and hits when also y <= wend.
+__global__ void __launch_bounds__(kEventsBlock) rs_ens_events_kernel(const double* __restrict__ mout, int n_slots, int mo_slots,
+                                                                     int ldm, int npoints, int members, int n_events, int tile,
+                                                                     const RsEnsembleStatsSpec spec, double* __restrict__ prob,
+                                                                     int st_slots, int ld)
+{
+  extern __shared__ int2 ev_smem[];
+  const int station_blocks = (npoints + kEventsBlock - 1) / kEventsBlock;
+  const int e = static_cast<int>(blockIdx.x % n_events);
+  const int rest = static_cast<int>(blockIdx.x / n_events);
+  const int p = (rest % station_blocks) * kEventsBlock + threadIdx.x;
+  const int s0 = (rest / station_blocks) * tile;
+  if (p >= npoints) return;
+  const RsEnsembleEvent& ev = spec.events[e];
+  const int nc = ev.n_conditions, w = ev.window;
+  const double* src[RS_ENS_MAX_CONDITIONS];
+  int op[RS_ENS_MAX_CONDITIONS];
+  double val[RS_ENS_MAX_CONDITIONS];
+#pragma unroll
+  for (int c = 0; c < RS_ENS_MAX_CONDITIONS; ++c)
+  {
+    const RsEnsembleThreshold th = ev.conditions[c < nc ? c : 0];
+    src[c] = mout + static_cast<size_t>(th.plane) * mo_slots * ldm + static_cast<size_t>(p) * members;
+    op[c] = th.op;
+    val[c] = th.value;
+  }
+  const int s1 = tile >= n_slots - s0 ? n_slots : s0 + tile;
+  const int s_end = w - 1 >= n_slots - s1 ? n_slots : s1 + w - 1;  // the last window of the tile ends at s_end - 1
+  int2* st = ev_smem + threadIdx.x;
+  for (int m = 0; m < members; ++m) st[m * kEventsBlock] = make_int2(INT_MAX, INT_MAX);
+  const size_t out_base = (static_cast<size_t>(spec.n_thresholds) + e) * st_slots;
+  for (int s = s_end - 1; s >= s0; --s)
+  {
+    const size_t off = static_cast<size_t>(s) * ldm;
+    const int wend = w - 1 >= n_slots - 1 - s ? n_slots - 1 : s + w - 1;
+    int n = 0, count = 0;
+#pragma unroll 4
+    for (int m = 0; m < members; ++m)
+    {
+      bool ok = true, hit = true;
+#pragma unroll
+      for (int c = 0; c < RS_ENS_MAX_CONDITIONS; ++c)
+        if (c < nc)
+        {
+          const double x = __ldg(src[c] + off + m);
+          const double v = val[c];
+          ok &= valid_value(x);
+          hit &= op[c] == RS_ENS_LT ? x < v : op[c] == RS_ENS_LE ? x <= v : op[c] == RS_ENS_GT ? x > v : x >= v;
+        }
+      int2 t = st[m * kEventsBlock];
+      if (!ok)
+        t.x = s;
+      else if (hit)
+        t.y = s;
+      st[m * kEventsBlock] = t;
+      const bool valid = t.x > wend;
+      n += valid ? 1 : 0;
+      count += (valid && t.y <= wend) ? 1 : 0;
+    }
+    if (s < s1)
+      prob[(out_base + s) * ld + p] = n == 0 ? -9999.0 : static_cast<double>(count) / static_cast<double>(n);
+  }
+}
 }  // namespace
 
 int rs_launch_ens_prefix_local(const double* local, int ld, int npoints, const double* member_relax, int ldm,
@@ -251,7 +342,34 @@ int rs_launch_ens_stats(const double* member_out, int out_nvar, int n_slots, int
   cudaError_t e = cudaFuncSetAttribute(rs_ens_stats_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
   if (e != cudaSuccess) return static_cast<int>(e);
   const long long blocks = (total + kStatsBlock - 1) / kStatsBlock;
+  StatsKernelSpec ks;
+  std::memcpy(&ks, spec, sizeof ks);
   rs_ens_stats_kernel<<<static_cast<unsigned>(blocks), kStatsBlock, smem, static_cast<cudaStream_t>(stream)>>>(
-      member_out, out_nvar, n_slots, mo_slots, ldm, npoints, members, *spec, stats, prob, st_slots, ld);
+      member_out, out_nvar, n_slots, mo_slots, ldm, npoints, members, ks, stats, prob, st_slots, ld);
+  return static_cast<int>(cudaGetLastError());
+}
+
+int rs_launch_ens_events(const double* member_out, int n_slots, int mo_slots, int ldm, int npoints, int members,
+                         const RsEnsembleStatsSpec* spec, double* prob, int st_slots, int ld, void* stream)
+{
+  const int E = spec->n_events;
+  if (E == 0 || npoints == 0 || n_slots == 0) return 0;
+  // One tile of all slots per thread where P * n_events threads fill the GPU; else tiles of at least 32 slots and
+  // four look-aheads (window - 1), so that a tile's look-ahead re-reads at most a quarter of it.
+  long long tile = n_slots;
+  const long long want_tiles = (kEventsTargetThreads + static_cast<long long>(npoints) * E - 1) / (static_cast<long long>(npoints) * E);
+  if (want_tiles > 1)
+  {
+    long long wmax = 1;
+    for (int j = 0; j < E; ++j) wmax = std::max<long long>(wmax, spec->events[j].window);
+    tile = std::min<long long>(n_slots, std::max({(n_slots + want_tiles - 1) / want_tiles, 4 * (wmax - 1), 32LL}));
+  }
+  const long long tiles = (n_slots + tile - 1) / tile;
+  const long long blocks = static_cast<long long>(E) * ((npoints + kEventsBlock - 1) / kEventsBlock) * tiles;
+  const int smem = static_cast<int>(sizeof(int2)) * kEventsBlock * members;
+  cudaError_t e = cudaFuncSetAttribute(rs_ens_events_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+  if (e != cudaSuccess) return static_cast<int>(e);
+  rs_ens_events_kernel<<<static_cast<unsigned>(blocks), kEventsBlock, smem, static_cast<cudaStream_t>(stream)>>>(
+      member_out, n_slots, mo_slots, ldm, npoints, members, E, static_cast<int>(tile), *spec, prob, st_slots, ld);
   return static_cast<int>(cudaGetLastError());
 }

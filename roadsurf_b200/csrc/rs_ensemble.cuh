@@ -41,3 +41,7 @@ int rs_launch_ens_fork(const RsForkArgs* f, void* stream);
 int rs_launch_ens_stats(const double* member_out, int out_nvar, int n_slots, int mo_slots, int ldm, int npoints,
                         int members, const RsEnsembleStatsSpec* spec, double* stats, double* prob, int st_slots, int ld,
                         void* stream);
+// Event probabilities of the first n_slots output slots into prob planes [n_thresholds, n_thresholds + n_events)
+// of [..][st_slots][ld]; slots >= n_slots are not written.
+int rs_launch_ens_events(const double* member_out, int n_slots, int mo_slots, int ldm, int npoints, int members,
+                         const RsEnsembleStatsSpec* spec, double* prob, int st_slots, int ld, void* stream);

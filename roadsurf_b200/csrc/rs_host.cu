@@ -1522,7 +1522,7 @@ void roadsurf_session_close(void* session)
 
 const char* roadsurf_last_error(void) { return g_err.c_str(); }
 
-const char* roadsurf_version(void) { return "roadsurf_b200 0.1 (RoadSurf 1.6.1 per-point loop, sm_100a)"; }
+const char* roadsurf_version(void) { return "roadsurf_b200 0.2 (RoadSurf 1.6.1 per-point loop, sm_100a)"; }
 
 int roadsurf_device_count(void)
 {
@@ -2235,6 +2235,39 @@ int check_stats_spec(const RsEnsembleStatsSpec& s, int out_nvar)
     if (s.thresholds[j].plane < 0 || s.thresholds[j].plane >= out_nvar || s.thresholds[j].op < RS_ENS_LT ||
         s.thresholds[j].op > RS_ENS_GE)
       return fail(RS_ERR_BAD_ARGUMENT, "threshold plane outside the output planes or unknown comparison");
+  if (s.n_events < 0 || s.n_events > RS_ENS_MAX_EVENTS) return fail(RS_ERR_BAD_ARGUMENT, "at most 8 events");
+  for (int j = 0; j < s.n_events; ++j)
+  {
+    const RsEnsembleEvent& ev = s.events[j];
+    if (ev.n_conditions < 1 || ev.n_conditions > RS_ENS_MAX_CONDITIONS)
+      return fail(RS_ERR_BAD_ARGUMENT, "an event has 1 to 4 conditions");
+    if (ev.window < 1) return fail(RS_ERR_BAD_ARGUMENT, "an event window is at least 1 output slot");
+    for (int c = 0; c < ev.n_conditions; ++c)
+      if (ev.conditions[c].plane < 0 || ev.conditions[c].plane >= out_nvar || ev.conditions[c].op < RS_ENS_LT ||
+          ev.conditions[c].op > RS_ENS_GE)
+        return fail(RS_ERR_BAD_ARGUMENT, "event condition plane outside the output planes or unknown comparison");
+  }
+  return RS_OK;
+}
+
+// The statistics kernel (when stats, or prob with thresholds, is given), then the events kernel (when prob is given
+// and the spec has events), on `stream`.  The spec has been checked.
+int launch_stats_and_events(const double* member_out, int out_nvar, int n_slots, int mo_slots, int ldm, int npoints,
+                            int members, const RsEnsembleStatsSpec* spec, double* stats, double* prob, int st_slots, int ld,
+                            void* stream)
+{
+  if (stats || (prob && spec->n_thresholds > 0))
+  {
+    CU(static_cast<cudaError_t>(rs_launch_ens_stats(member_out, out_nvar, n_slots, mo_slots, ldm, npoints, members, spec,
+                                                    stats, prob, st_slots, ld, stream)));
+    ++g_launches_total;
+  }
+  if (prob && spec->n_events > 0)
+  {
+    CU(static_cast<cudaError_t>(
+        rs_launch_ens_events(member_out, n_slots, mo_slots, ldm, npoints, members, spec, prob, st_slots, ld, stream)));
+    ++g_launches_total;
+  }
   return RS_OK;
 }
 
@@ -2277,12 +2310,8 @@ int roadsurf_ensemble_stats(const double* member_out, int out_nvar, int n_out, i
     const int rc = check_stats_spec(*spec, out_nvar);
     if (rc != RS_OK) return rc;
   }
-  if (!stats && !prob) return RS_OK;
-  CU(static_cast<cudaError_t>(
-      rs_launch_ens_stats(member_out, out_nvar, n_out, n_out, ld_members, npoints, members, spec, stats, prob, n_out, ld,
-                          stream)));
-  ++g_launches_total;
-  return RS_OK;
+  return launch_stats_and_events(member_out, out_nvar, n_out, n_out, ld_members, npoints, members, spec, stats, prob, n_out,
+                                 ld, stream);
 }
 
 }  // extern "C"
@@ -2426,15 +2455,10 @@ int run_ensemble(const RsEnsembleBatch* e, void* stream, const int* host_record_
     const int rc = roadsurf_run_device(&mb, stream);
     if (rc != RS_OK) return rc;
   }
-  // (4) the statistics
-  if (e->stats || e->prob)
-  {
-    // the member slots [m0, m1) of member_out [out_nvar][n_out_members][ld_members]; slots beyond are not read
-    CU(static_cast<cudaError_t>(rs_launch_ens_stats(e->member_out, out_nvar, m1 - m0, e->n_out_members, e->ld_members, P, M,
-                                                    &e->spec, e->stats, e->prob, e->n_out_members, s.ld, stream)));
-    ++g_launches_total;
-  }
-  return RS_OK;
+  // (4) the statistics and events over the member slots [m0, m1) of member_out [out_nvar][n_out_members][ld_members];
+  // slots beyond are not read
+  return launch_stats_and_events(e->member_out, out_nvar, m1 - m0, e->n_out_members, e->ld_members, P, M, &e->spec,
+                                 e->stats, e->prob, e->n_out_members, s.ld, stream);
 }
 }  // namespace
 
@@ -2540,10 +2564,10 @@ int roadsurf_run_ensemble_host_soa(const RsHostBatch* b, const double* member_re
   slot_range(1, F - 1, 0, b->out_stride, &pre0, &pre1);
   slot_range(F, sim_len, 0, b->out_stride, &m0, &m1);
   const int n_pre = std::max(1, pre1 - pre0), n_m = m1 - m0;
-  const int nq = spec->n_quantiles, nt = spec->n_thresholds;
+  const int nq = spec->n_quantiles, np_planes = spec->n_thresholds + spec->n_events;  // prob: thresholds, then events
   const size_t frows = static_cast<size_t>(nrec) * nvar, frows_m = static_cast<size_t>(nrec_m + 1) * nvar;
   const size_t NS = RS_STATE_NPLANES(nl), SC = RS_SCRATCH_NPLANES(nl);
-  const size_t srows = static_cast<size_t>(RS_ENS_NFIXED + nq) * RS_O_NVAR * n_m, prows = static_cast<size_t>(nt) * n_m;
+  const size_t srows = static_cast<size_t>(RS_ENS_NFIXED + nq) * RS_O_NVAR * n_m, prows = static_cast<size_t>(np_planes) * n_m;
   const size_t per_station =
       sizeof(double) * (frows + RS_L_NLOCAL + (hor ? 360 : 0) + RS_O_NVAR * n_pre + NS + (cpl ? SC : 0) + 1 + srows + prows) +
       sizeof(double) * M * (frows_m + RS_L_NLOCAL + (hor ? 360 : 0) + NS + (cpl ? SC : 0) + 1 + 3 + RS_O_NVAR * n_m);
@@ -2580,7 +2604,7 @@ int roadsurf_run_ensemble_host_soa(const RsHostBatch* b, const double* member_re
       (hor && (rc = dbuf(408, D * 360 * ldmc, &d_mh))) || (rc = dbuf(409, D * NS * ldmc, &d_ms)) ||
       (cpl && (rc = dbuf(410, D * SC * ldmc, &d_msc))) || (rc = dbuf(411, D * RS_O_NVAR * n_m * ldmc, &d_mo)) ||
       (relax && (rc = dbuf(412, D * 3 * ldmc, &d_relax))) || (rc = dbuf(413, D * srows * ldc, &d_stats)) ||
-      (nt && (rc = dbuf(414, D * prows * ldc, &d_prob))) || (rc = dbuf(415, D * 4 * sim_len, &d_solar)) ||
+      (np_planes && (rc = dbuf(414, D * prows * ldc, &d_prob))) || (rc = dbuf(415, D * 4 * sim_len, &d_solar)) ||
       (rc = dbuf(416, sizeof(int) * ldc, &d_status)) || (rc = dbuf(417, sizeof(int) * ldmc, &d_mstatus)) ||
       (rc = dbuf(418, sizeof(int) * 6 * sim_len, &d_tf)) || (rc = dbuf(419, sizeof(int) * nrec, &d_rs)) ||
       (rc = dbuf(420, sizeof(unsigned long long) * RS_CNT_N, &d_counters)))
@@ -2645,7 +2669,7 @@ int roadsurf_run_ensemble_host_soa(const RsHostBatch* b, const double* member_re
     e.n_out_members = std::max(1, n_m);
     e.spec = *spec;
     e.stats = stats ? d_stats : nullptr;
-    e.prob = (prob && nt) ? d_prob : nullptr;
+    e.prob = (prob && np_planes) ? d_prob : nullptr;
     rc = run_ensemble(&e, st, b->record_step);
     if (rc != RS_OK) return rc;
     CU(cudaEventRecord(ev[2], st));
@@ -2654,7 +2678,7 @@ int roadsurf_run_ensemble_host_soa(const RsHostBatch* b, const double* member_re
                            cudaMemcpyDeviceToHost, st));
     if (stats && n_m > 0)
       CU(cudaMemcpy2DAsync(stats + col, D * np, d_stats, D * ld, D * n, srows, cudaMemcpyDeviceToHost, st));
-    if (prob && nt && n_m > 0) CU(cudaMemcpy2DAsync(prob + col, D * np, d_prob, D * ld, D * n, prows, cudaMemcpyDeviceToHost, st));
+    if (prob && np_planes && n_m > 0) CU(cudaMemcpy2DAsync(prob + col, D * np, d_prob, D * ld, D * n, prows, cudaMemcpyDeviceToHost, st));
     if (member_out && n_m > 0)
       CU(cudaMemcpy2DAsync(member_out + colm, D * npm, d_mo, D * ldm, D * nm, static_cast<size_t>(RS_O_NVAR) * n_m,
                            cudaMemcpyDeviceToHost, st));

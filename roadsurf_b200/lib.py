@@ -44,6 +44,7 @@ EXPORTS = ("runsimulation", "roadsurf_last_error", "roadsurf_device_count", "roa
 (PRIM_EXP, PRIM_EXP_SMEM, PRIM_LOG, PRIM_LOG_SMEM, PRIM_EXP_FLAT, PRIM_EXP_FLAT_SMEM, PRIM_PSIH_UNSTABLE,
  PRIM_PSIH_UNSTABLE_SMEM, PRIM_FRCP, PRIM_FDIV, PRIM_DIV_CONST, PRIM_N) = range(12)
 ENS_MAX_MEMBERS, ENS_MAX_QUANTILES, ENS_MAX_THRESHOLDS = 128, 8, 8
+ENS_MAX_EVENTS, ENS_MAX_CONDITIONS = 8, 4
 ENS_NVALID, ENS_MEAN, ENS_STD, ENS_MIN, ENS_MAX, ENS_NFIXED = range(6)
 ENS_LT, ENS_LE, ENS_GT, ENS_GE = range(4)
 ENS_OPS = {"<": ENS_LT, "<=": ENS_LE, ">": ENS_GT, ">=": ENS_GE}
@@ -95,9 +96,18 @@ class RsEnsembleThreshold(C.Structure):
     _fields_ = [("plane", C.c_int), ("op", C.c_int), ("value", C.c_double)]
 
 
+class RsEnsembleEvent(C.Structure):
+    _fields_ = [("n_conditions", C.c_int), ("window", C.c_int), ("conditions", RsEnsembleThreshold * 4)]
+
+
 class RsEnsembleStatsSpec(C.Structure):
     _fields_ = [("n_quantiles", C.c_int), ("n_thresholds", C.c_int), ("quantiles", C.c_double * 8),
-                ("thresholds", RsEnsembleThreshold * 8)]
+                ("thresholds", RsEnsembleThreshold * 8), ("n_events", C.c_int), ("events", RsEnsembleEvent * 8)]
+
+    @property
+    def n_prob(self):
+        """Planes of the probability tensor: the thresholds, then the events."""
+        return self.n_thresholds + self.n_events
 
 
 class RsEnsembleBatch(C.Structure):
@@ -109,17 +119,25 @@ class RsEnsembleBatch(C.Structure):
                 ("prob", C.c_void_p)]
 
 
-def stats_spec(quantiles=(), thresholds=()):
-    """RsEnsembleStatsSpec from quantiles [q, ...] and thresholds [(plane, op, value), ...], op one of
-    "<", "<=", ">", ">=" (or an ENS_* code)."""
-    quantiles, thresholds = list(quantiles), list(thresholds)
+def stats_spec(quantiles=(), thresholds=(), events=()):
+    """RsEnsembleStatsSpec from quantiles [q, ...], thresholds [(plane, op, value), ...], op one of
+    "<", "<=", ">", ">=" (or an ENS_* code), and events [(conditions, window), ...] whose conditions are
+    [(plane, op, value), ...] in the threshold form, combined with AND.  Event j is probability plane
+    n_thresholds + j."""
+    quantiles, thresholds, events = list(quantiles), list(thresholds), list(events)
     if len(quantiles) > ENS_MAX_QUANTILES or len(thresholds) > ENS_MAX_THRESHOLDS:
         raise ValueError("at most 8 quantiles and 8 thresholds")
-    sp = RsEnsembleStatsSpec(n_quantiles=len(quantiles), n_thresholds=len(thresholds))
+    if len(events) > ENS_MAX_EVENTS or any(not 1 <= len(conds) <= ENS_MAX_CONDITIONS for conds, _ in events):
+        raise ValueError("at most 8 events of 1 to 4 conditions")
+    sp = RsEnsembleStatsSpec(n_quantiles=len(quantiles), n_thresholds=len(thresholds), n_events=len(events))
     for j, q in enumerate(quantiles):
         sp.quantiles[j] = float(q)
     for j, (plane, op, value) in enumerate(thresholds):
         sp.thresholds[j] = RsEnsembleThreshold(int(plane), ENS_OPS.get(op, op), float(value))
+    for j, (conds, window) in enumerate(events):
+        sp.events[j].n_conditions, sp.events[j].window = len(conds), int(window)
+        for c, (plane, op, value) in enumerate(conds):
+            sp.events[j].conditions[c] = RsEnsembleThreshold(int(plane), ENS_OPS.get(op, op), float(value))
     return sp
 
 
@@ -609,19 +627,19 @@ def _ptr(x):
 def ensemble_stats(member_out, npoints, members, spec, stream=None):
     """roadsurf_ensemble_stats on a torch CUDA tensor member_out [out_nvar, n_out, ld_members] (lane
     p * members + m).  Returns (stats [5 + n_quantiles, out_nvar, n_out, npoints],
-    prob [n_thresholds, n_out, npoints]) as CUDA tensors (synchronised)."""
+    prob [n_thresholds + n_events, n_out, npoints]) as CUDA tensors (synchronised)."""
     import torch
     out_nvar, n_out, ldm = member_out.shape
     ld = max(32, (npoints + 31) // 32 * 32)
     f64 = dict(dtype=torch.float64, device=member_out.device)
     stats = torch.full((ENS_NFIXED + spec.n_quantiles, out_nvar, n_out, ld), 12345.0, **f64)
-    prob = torch.full((max(1, spec.n_thresholds), n_out, ld), 12345.0, **f64)
+    prob = torch.full((max(1, spec.n_prob), n_out, ld), 12345.0, **f64)
     st = stream if stream is not None else torch.cuda.current_stream()
     _check(load().roadsurf_ensemble_stats(member_out.data_ptr(), out_nvar, n_out, ldm, int(npoints), int(members),
                                           C.byref(spec), stats.data_ptr(), prob.data_ptr(), ld,
                                           C.c_void_p(st.cuda_stream)))
     torch.cuda.synchronize()
-    return stats[..., :npoints], prob[:spec.n_thresholds, :, :npoints]
+    return stats[..., :npoints], prob[:spec.n_prob, :, :npoints]
 
 
 def fork_record(record_step, fork_step):
@@ -670,7 +688,7 @@ class EnsembleBatch:
         self.spec = stats_spec if stats_spec is not None else RsEnsembleStatsSpec()
         ld = shared.ld
         self.stats_t = torch.empty((ENS_NFIXED + self.spec.n_quantiles, shared.out_nvar, self.n_out_members, ld), **f64)
-        self.prob_t = torch.empty((max(1, self.spec.n_thresholds), self.n_out_members, ld), **f64)
+        self.prob_t = torch.empty((max(1, self.spec.n_prob), self.n_out_members, ld), **f64)
 
     def load_member_records(self, member_recs):
         """Coarse records of every member (synth.Records with the full record axis, one per member, equal
@@ -722,7 +740,7 @@ class EnsembleBatch:
                                member_out=_ptr(self.member_out), n_out_members=self.n_out_members,
                                member_order=_ptr(self.member_order), spec=self.spec,
                                stats=_ptr(self.stats_t) if stats else None,
-                               prob=_ptr(self.prob_t) if (stats and self.spec.n_thresholds) else None)
+                               prob=_ptr(self.prob_t) if (stats and self.spec.n_prob) else None)
 
     def run(self, stream=None, stats=True):
         """Asynchronous: prefix, fork, members, statistics on `stream` (default: the current stream)."""
@@ -738,11 +756,11 @@ class EnsembleBatch:
         return {name: np.ascontiguousarray(o[v].T.reshape(P, M, -1)) for v, name in enumerate(names)}
 
     def stats(self):
-        """(stats [5 + n_quantiles, out_nvar, n_slots, P], prob [n_thresholds, n_slots, P]) numpy: the slots of the
-        steps [F, sim_len]."""
+        """(stats [5 + n_quantiles, out_nvar, n_slots, P], prob [n_thresholds + n_events, n_slots, P]) numpy: the slots
+        of the steps [F, sim_len]."""
         P, n = self.shared.npoints, self.n_slots
         return (self.stats_t.cpu().numpy()[:, :, :n, :P],
-                self.prob_t.cpu().numpy()[:self.spec.n_thresholds, :n, :P])
+                self.prob_t.cpu().numpy()[:self.spec.n_prob, :n, :P])
 
 
 def run_ensemble_host_soa(settings, params, forcing, record_step, time_fields, local, member_records, members,
@@ -751,7 +769,7 @@ def run_ensemble_host_soa(settings, params, forcing, record_step, time_fields, l
     """roadsurf_run_ensemble_host_soa on host arrays: forcing [n_records, nvar, P], record_step [n_records],
     local [L_NLOCAL, P], member_records [n_records - r_f - 1, nvar, P * members], latest_obs_index [P] int32 (the
     relaxation rule of read_input_derive_records; None = no observations).  Returns a dict with
-    stats [5 + nq, 6, n_out_m, P], prob [nt, n_out_m, P] and, when asked for, member_out [6, n_out_m, P * M]
+    stats [5 + nq, 6, n_out_m, P], prob [nt + n_events, n_out_m, P] and, when asked for, member_out [6, n_out_m, P * M]
     and member_status [P * M]."""
     n_records, nvar, npoints = forcing.shape
     sim_len = time_fields.shape[1]
@@ -759,7 +777,7 @@ def run_ensemble_host_soa(settings, params, forcing, record_step, time_fields, l
     slot0 = (k0 + out_stride - 1) // out_stride
     n_m = (sim_len + out_stride - 1) // out_stride - slot0
     res = dict(stats=np.zeros((ENS_NFIXED + spec.n_quantiles, O_NVAR, n_m, npoints)),
-               prob=np.zeros((spec.n_thresholds, n_m, npoints)))
+               prob=np.zeros((spec.n_prob, n_m, npoints)))
     if member_out:
         res["member_out"] = np.zeros((O_NVAR, n_m, npoints * members))
     if member_status:

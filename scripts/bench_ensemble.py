@@ -38,7 +38,7 @@ def card():
         return f"unknown ({e})"
 
 
-def build(shape, P, M, seed=2024):
+def build(shape, P, M, seed=2024, member_records=True):
     cfg = SHAPES[shape]
     ah, hours = cfg["analysis_hours"], cfg["hours"]
     start = synth.FORECAST_START - dt.timedelta(hours=ah)
@@ -48,7 +48,7 @@ def build(shape, P, M, seed=2024):
     fs = ah * 120
     F = fs + 2
     r_f = lib.fork_record(base.record_step, F)
-    mrecs = synth.member_records(base, M, r_f, seed, start)
+    mrecs = synth.member_records(base, M, r_f, seed, start) if member_records else None
     sim_len = 1 + (ah + hours) * 120
     settings = synth.abi.default_settings(sim_len, 1, 1)
     params = synth.abi.default_parameters()
