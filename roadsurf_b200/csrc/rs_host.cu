@@ -7,6 +7,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <array>
 #include <atomic>
 #include <chrono>
 #include <cmath>
@@ -28,6 +29,28 @@
 
 namespace
 {
+// Slots of the pooled work space (pooled / pooled_pinned below), grouped by entry.  An entry holds its device's
+// g_device_mu while it uses its buffers, so the entries of one device never run at the same time: a slot only
+// needs to be unique within one entry and its second buffer set.  Device and pinned buffers are separate pools.
+enum PoolSlot : int
+{
+  // run_shard (roadsurf_run_batch, runsimulation): the second buffer set adds RB_SET2 (except RB_TIME_FIELDS, RB_SOLAR)
+  RB_FORCING = 200, RB_OUT = 201, RB_LOCAL = 202, RB_HOR = 203, RB_STATUS = 204, RB_SCRATCH = 205, RB_STAGE = 206,
+  RB_STAGE2 = 207, RB_COUNTERS = 208, RB_TIME_FIELDS = 209, RB_SOLAR = 210, RB_STATE = 211, RB_NVIS = 212,
+  RB_SET2 = 50,
+  RB_H_STAGE = 0, RB_H_STAGE2 = 1, RB_H_LOCAL = 2, RB_H_HOR = 3, RB_H_STATUS = 4,  // pinned
+  // run_host_soa_shard (roadsurf_run_host_soa): the buffers of stream s add s * HS_STREAM
+  HS_FORCING = 0, HS_OUT = 1, HS_LOCAL = 2, HS_HOR = 3, HS_SCRATCH = 4, HS_STATUS = 5, HS_STATE = 6, HS_ORDER = 7,
+  HS_STREAM = 10,
+  HS_TIME_FIELDS = 100, HS_RECORD_STEP = 101, HS_COUNTERS = 102, HS_SOLAR = 103,
+  // roadsurf_run_ensemble_host_soa (EH_M_*: member lanes)
+  EH_FORCING = 400, EH_LOCAL = 401, EH_HOR = 402, EH_OUT = 403, EH_STATE = 404, EH_SCRATCH = 405, EH_M_FORCING = 406,
+  EH_M_LOCAL = 407, EH_M_HOR = 408, EH_M_STATE = 409, EH_M_SCRATCH = 410, EH_M_OUT = 411, EH_RELAX = 412,
+  EH_STATS = 413, EH_PROB = 414, EH_SOLAR = 415, EH_STATUS = 416, EH_M_STATUS = 417, EH_TIME_FIELDS = 418,
+  EH_RECORD_STEP = 419, EH_COUNTERS = 420,
+  EH_H_RELAX = 400,  // pinned
+};
+
 thread_local std::string g_err;
 thread_local RsBatchStats g_stats;
 thread_local RsLaunchInfo g_launch;
@@ -96,11 +119,15 @@ int launch_model(const RsArgs& a, const RsArgsCold& ac, const RsModel& m, int we
 {
   const int passes = opt_compaction_passes();
   *launches = 0;
+  auto run = [&](const RsArgs& ak, const RsArgsCold& ck, int staged) {
+    return static_cast<cudaError_t>(rs_launch_run(&ak, &ck, m.nlayers, staged, m.use_coupling, m.use_relaxation,
+                                                  m.depth_mode != 0, stream, &li->grid, &li->block,
+                                                  &li->regs_per_thread, &li->smem_bytes));
+  };
   if (!(m.use_coupling && wend > 0 && passes > 0 && ac.state && a.scratch && !(opt_staging() && a.forcing_mode == 0) &&
         a.forcing_step0 == 1 && a.step_begin <= 1 && wend + 1 < a.step_end))
   {
-    CU(static_cast<cudaError_t>(rs_launch_run(&a, &ac, m.nlayers, opt_staging(), m.use_coupling, m.use_relaxation, m.depth_mode != 0, stream, &li->grid, &li->block,
-                                              &li->regs_per_thread, &li->smem_bytes)));
+    CU(run(a, ac, opt_staging()));
     *launches = 1;
     return RS_OK;
   }
@@ -112,8 +139,7 @@ int launch_model(const RsArgs& a, const RsArgsCold& ac, const RsModel& m, int we
   a1.step_end = wend;
   c1.mode = RS_MODE_SPLIT;
   c1.window_end = wend;
-  CU(static_cast<cudaError_t>(rs_launch_run(&a1, &c1, m.nlayers, 0, m.use_coupling, m.use_relaxation, m.depth_mode != 0, stream, &li->grid, &li->block,
-                                            &li->regs_per_thread, &li->smem_bytes)));
+  CU(run(a1, c1, 0));
   RsArgs a2 = a;
   RsArgsCold c2 = c1;
   a2.step_begin = wend + 1;
@@ -124,8 +150,7 @@ int launch_model(const RsArgs& a, const RsArgsCold& ac, const RsModel& m, int we
   for (int k = 0; k < passes; ++k)
   {
     CU(static_cast<cudaError_t>(rs_launch_partition(flags, a.ld, a.npoints, 0, index, n_index, stream)));
-    CU(static_cast<cudaError_t>(rs_launch_run(&a2, &c2, m.nlayers, 0, m.use_coupling, m.use_relaxation, m.depth_mode != 0, stream, &li->grid, &li->block,
-                                              &li->regs_per_thread, &li->smem_bytes)));
+    CU(run(a2, c2, 0));
   }
   CU(static_cast<cudaError_t>(rs_launch_partition(flags, a.ld, a.npoints, 1, index, n_index, stream)));
   RsArgs a3 = a;
@@ -133,8 +158,7 @@ int launch_model(const RsArgs& a, const RsArgsCold& ac, const RsModel& m, int we
   a3.step_begin = wend + 1;
   c3.index = index;
   c3.n_index = n_index;
-  CU(static_cast<cudaError_t>(rs_launch_run(&a3, &c3, m.nlayers, 0, m.use_coupling, m.use_relaxation, m.depth_mode != 0, stream, &li->grid, &li->block,
-                                            &li->regs_per_thread, &li->smem_bytes)));
+  CU(run(a3, c3, 0));
   *launches = 2 * passes + 3;
   return RS_OK;
 }
@@ -145,27 +169,41 @@ double now_ms()
   return duration<double, std::milli>(steady_clock::now().time_since_epoch()).count();
 }
 
+// Makes `m` the model of device `dev`, the current device, by the ordering rule above.
+int upload_model(int dev, const RsModel& m)
+{
+  std::lock_guard<std::mutex> lk(g_model_mu);
+  DeviceModel& dm = g_models[dev];
+  if (dm.valid && std::memcmp(&dm.m, &m, sizeof m) == 0) return RS_OK;
+  // kernels of the asynchronous entry may still be reading the old model: wait for them
+  for (auto& kv : dm.last_launch) CU(cudaEventSynchronize(kv.second));
+  CU(static_cast<cudaError_t>(rs_upload_model(&m)));
+  dm.m = m;
+  dm.valid = true;
+  return RS_OK;
+}
+
 int set_model_on_current_device(const InputSettings* settings, const InputParameters* params, RsModel* out)
 {
   RsModel m;
   char err[256];
-  const int rc = rs_build_model(settings, params, &m, err, sizeof err);
+  int rc = rs_build_model(settings, params, &m, err, sizeof err);
   if (rc != RS_OK) return fail(rc, err);
   int dev = 0;
   CU(cudaGetDevice(&dev));
-  {
-    std::lock_guard<std::mutex> lk(g_model_mu);
-    DeviceModel& dm = g_models[dev];
-    if (!dm.valid || std::memcmp(&dm.m, &m, sizeof m) != 0)
-    {
-      // kernels of the asynchronous entry may still be reading the old model: wait for them
-      for (auto& kv : dm.last_launch) CU(cudaEventSynchronize(kv.second));
-      CU(static_cast<cudaError_t>(rs_upload_model(&m)));
-      dm.m = m;
-      dm.valid = true;
-    }
-  }
-  if (out) *out = m;
+  rc = upload_model(dev, m);
+  if (rc == RS_OK && out) *out = m;
+  return rc;
+}
+
+// The model roadsurf_set_model put on device `dev`.
+int current_model(int dev, RsModel* out)
+{
+  std::lock_guard<std::mutex> lk(g_model_mu);
+  auto it = g_models.find(dev);
+  if (it == g_models.end() || !it->second.valid)
+    return fail(RS_ERR_BAD_ARGUMENT, "roadsurf_set_model was not called on this device");
+  *out = it->second.m;
   return RS_OK;
 }
 
@@ -219,9 +257,134 @@ long long window_key(const RsModel& m, const LocalParameters& lp)
   return lp.couplingIndexI;
 }
 
-struct Shard
+// ---- the reference's point structs <-> the kernel's planes ------------------------------------------
+// A point's time axis in the order of the kernel's time-field planes.
+std::array<const int*, 6> time_fields(const InputPointers& ip)
+{
+  return {ip.c_year, ip.c_month, ip.c_day, ip.c_hour, ip.c_minute, ip.c_second};
+}
+
+bool same_time_axis(const InputPointers& a, const InputPointers& b, int sim_len)
+{
+  const auto fa = time_fields(a), fb = time_fields(b);
+  for (int k = 0; k < 6; ++k)
+    if (fa[k] != fb[k] && std::memcmp(fa[k], fb[k], sizeof(int) * sim_len)) return false;
+  return true;
+}
+
+// Whether the kernel applies the sky-view correction to a point (RS_L_SKY_VIEW).
+bool sky_view_point(double sky_view) { return sky_view < 1.0 && sky_view > -0.01f; }
+
+// Forcing plane v (RS_F_*) of a point, steps 0 .. n-1, to dst[t * stride]; the precipitation phase is an int
+// array in the reference and a double plane in the kernel.
+void forcing_row(const InputPointers& ip, int v, int n, double* dst, size_t stride)
+{
+  const double* src[RS_F_NVAR_DEPTH] = {ip.c_tair, ip.c_tdew, ip.c_VZ,     ip.c_Rhz,      ip.c_prec, ip.c_SW,
+                                        ip.c_LW,   ip.c_SW_dir, ip.c_LW_net, ip.c_TSurfObs, nullptr,   ip.c_Depth};
+  if (v == RS_F_PHASE)
+    for (int t = 0; t < n; ++t) dst[t * stride] = static_cast<double>(ip.c_PrecPhase[t]);
+  else if (stride == 1)
+    std::memcpy(dst, src[v], sizeof(double) * n);
+  else
+    for (int t = 0; t < n; ++t) dst[t * stride] = src[v][t];
+}
+
+// A point's output arrays in the order of the kernel's output planes (RS_O_*).
+std::array<double*, RS_O_NVAR> output_planes(const OutputPointers& op)
+{
+  return {op.c_TsurfOut, op.c_SnowOut, op.c_WaterOut, op.c_IceOut, op.c_DepositOut, op.c_Ice2Out};
+}
+
+// A point's values of the statics planes RS_L_* to dst[k * stride]; lp == nullptr gives those of a padding slot.
+void local_row(const LocalParameters* lp, double* dst, size_t stride)
+{
+  double row[RS_L_NLOCAL] = {};
+  row[RS_L_SKY_VIEW] = 1.0;
+  if (lp)
+  {
+    row[RS_L_TAIR_RELAX] = lp->tair_relax;
+    row[RS_L_VZ_RELAX] = lp->VZ_relax;
+    row[RS_L_RH_RELAX] = lp->RH_relax;
+    row[RS_L_COUPLING_TSURF] = lp->couplingTsurf;
+    row[RS_L_LAT] = lp->lat;
+    row[RS_L_LON] = lp->lon;
+    row[RS_L_SKY_VIEW] = lp->sky_view;
+    row[RS_L_COUPLING_INDEX] = lp->couplingIndexI;
+    row[RS_L_INIT_LEN] = lp->InitLenI;
+    row[RS_L_ACTIVE] = 1.0;
+  }
+  for (int k = 0; k < RS_L_NLOCAL; ++k) dst[k * stride] = row[k];
+}
+
+// The coupling window end shared by the active coupled points of SoA statics [RS_L_NLOCAL][np]: 0 when no
+// point is coupled, -1 when their windows differ.
+int common_window_end(const double* local, size_t np)
+{
+  int w = 0;
+  for (size_t p = 0; p < np; ++p)
+  {
+    const double ts = local[RS_L_COUPLING_TSURF * np + p], ix = local[RS_L_COUPLING_INDEX * np + p];
+    if (local[RS_L_ACTIVE * np + p] == 0.0 || ts < -100 || ix < 1) continue;
+    if (w == 0)
+      w = static_cast<int>(ix);
+    else if (w != static_cast<int>(ix))
+      return -1;
+  }
+  return w;
+}
+
+// Output slots of the steps [first, last] (1-based) as [slot_begin, slot_end); empty when none.
+void slot_range(int first, int last, int out_start, int out_stride, int* s0, int* s1)
+{
+  *s0 = *s1 = 0;
+  if (last - 1 < out_start || last < first) return;
+  const int k0 = first - 1 - out_start;
+  *s0 = k0 > 0 ? (k0 + out_stride - 1) / out_stride : 0;
+  *s1 = (last - 1 - out_start) / out_stride + 1;
+  if (*s1 < *s0) *s1 = *s0;
+}
+
+// Adds the device time between the events ev[0..3] (input copies, kernels, output copies) to s.
+void add_stage_times(RsBatchStats& s, const cudaEvent_t ev[4])
+{
+  float ms = 0.f;
+  cudaEventElapsedTime(&ms, ev[0], ev[1]);
+  s.h2d_ms += ms;
+  cudaEventElapsedTime(&ms, ev[1], ev[2]);
+  s.kernel_ms += ms;
+  cudaEventElapsedTime(&ms, ev[2], ev[3]);
+  s.d2h_ms += ms;
+}
+
+// Points [first, first + count) of a batch, run on `device`.
+struct ShardRange
 {
   int first = 0, count = 0, device = 0;
+};
+
+// The split of npoints over the GPUs: ngpus <= 0 or above the device count means every device, and there are
+// never more shards than points.  A single shard runs on the caller's device, *current.
+int split_shards(int npoints, int ngpus, int* current, std::vector<ShardRange>* shards)
+{
+  const int ndev = roadsurf_device_count();
+  if (ndev < 1) return fail(RS_ERR_NO_DEVICE, "no CUDA device visible (this library has no CPU path)");
+  if (ngpus <= 0 || ngpus > ndev) ngpus = ndev;
+  if (ngpus > npoints) ngpus = npoints;
+  *current = 0;
+  cudaGetDevice(current);
+  shards->resize(ngpus);
+  for (int g = 0; g < ngpus; ++g)
+  {
+    ShardRange& s = (*shards)[g];
+    s.first = static_cast<int>(static_cast<long long>(npoints) * g / ngpus);
+    s.count = static_cast<int>(static_cast<long long>(npoints) * (g + 1) / ngpus) - s.first;
+    s.device = (ngpus == 1) ? *current : g;
+  }
+  return RS_OK;
+}
+
+struct Shard : ShardRange
+{
   int rc = RS_OK;
   std::string err;
   RsBatchStats stats{};
@@ -237,69 +400,43 @@ struct PoolEntry
   size_t cap = 0;
 };
 std::mutex g_pool_mu;
-std::map<std::pair<int, int>, PoolEntry> g_pool;
-
-cudaError_t pool_get(int device, int slot, size_t bytes, void** out)
-{
-  std::lock_guard<std::mutex> lk(g_pool_mu);
-  PoolEntry& e = g_pool[{device, slot}];
-  if (e.cap < bytes)
-  {
-    if (e.p) cudaFree(e.p);
-    e.p = nullptr;
-    e.cap = 0;
-    cudaError_t rc = cudaMalloc(&e.p, bytes);
-    if (rc != cudaSuccess) return rc;
-    e.cap = bytes;
-  }
-  *out = e.p;
-  return cudaSuccess;
-}
-
-std::map<std::pair<int, int>, PoolEntry> g_pinned_pool;
+std::map<std::pair<int, int>, PoolEntry> g_pool, g_pinned_pool;
 
 // The pooled buffers of a device are used by one call at a time: concurrent callers (the reference
 // calls runsimulation from N host threads) are serialised per device, as the GPU would do anyway.
 std::mutex g_device_mu[64];
 
-cudaError_t pinned_get(int device, int slot, size_t bytes, void** out)
+// The buffer of (device, slot), grown to `count` elements of T (and at least 8 bytes); in pinned host memory
+// when `pinned`.  Use pooled / pooled_pinned.
+template <class T>
+cudaError_t pool_get(bool pinned, int device, int slot, size_t count, T** out)
 {
+  size_t bytes = sizeof(T) * count;
+  if (bytes == 0) bytes = 8;
   std::lock_guard<std::mutex> lk(g_pool_mu);
-  PoolEntry& e = g_pinned_pool[{device, slot}];
+  PoolEntry& e = (pinned ? g_pinned_pool : g_pool)[{device, slot}];
   if (e.cap < bytes)
   {
-    if (e.p) cudaFreeHost(e.p);
+    if (e.p) pinned ? cudaFreeHost(e.p) : cudaFree(e.p);
     e.p = nullptr;
     e.cap = 0;
-    cudaError_t rc = cudaMallocHost(&e.p, bytes);
+    cudaError_t rc = pinned ? cudaMallocHost(&e.p, bytes) : cudaMalloc(&e.p, bytes);
     if (rc != cudaSuccess) return rc;
     e.cap = bytes;
   }
-  *out = e.p;
+  *out = static_cast<T*>(e.p);
   return cudaSuccess;
 }
-
-// Non-owning views with the DeviceMem / PinnedMem interface, backed by the pools above.
-struct PooledDevice
+template <class T>
+cudaError_t pooled(int device, int slot, size_t count, T** out)
 {
-  void* p = nullptr;
-  cudaError_t alloc(int device, int slot, size_t bytes) { return pool_get(device, slot, bytes ? bytes : 8, &p); }
-  template <class T>
-  T* as() const
-  {
-    return static_cast<T*>(p);
-  }
-};
-struct PooledPinned
+  return pool_get(false, device, slot, count, out);
+}
+template <class T>
+cudaError_t pooled_pinned(int device, int slot, size_t count, T** out)
 {
-  void* p = nullptr;
-  cudaError_t alloc(int device, int slot, size_t bytes) { return pinned_get(device, slot, bytes ? bytes : 8, &p); }
-  template <class T>
-  T* as() const
-  {
-    return static_cast<T*>(p);
-  }
-};
+  return pool_get(true, device, slot, count, out);
+}
 
 // Run points [first, first+count) of the batch on `device`.
 int run_shard(Shard& sh, OutputPointers* const* out, const InputPointers* const* in,
@@ -340,13 +477,7 @@ int run_shard(Shard& sh, OutputPointers* const* out, const InputPointers* const*
     bool placed = false;
     for (auto& g : groups)
     {
-      const InputPointers* r = g.rep;
-      const bool same_ptr = r->c_year == ip->c_year && r->c_month == ip->c_month && r->c_day == ip->c_day &&
-                            r->c_hour == ip->c_hour && r->c_minute == ip->c_minute && r->c_second == ip->c_second;
-      const size_t nb = sizeof(int) * sim_len;
-      if (same_ptr || (!std::memcmp(r->c_year, ip->c_year, nb) && !std::memcmp(r->c_month, ip->c_month, nb) &&
-                       !std::memcmp(r->c_day, ip->c_day, nb) && !std::memcmp(r->c_hour, ip->c_hour, nb) &&
-                       !std::memcmp(r->c_minute, ip->c_minute, nb) && !std::memcmp(r->c_second, ip->c_second, nb)))
+      if (same_time_axis(*g.rep, *ip, sim_len))
       {
         g.points.push_back(p);
         placed = true;
@@ -367,10 +498,8 @@ int run_shard(Shard& sh, OutputPointers* const* out, const InputPointers* const*
     // inside a window, points with sky-view radiation go last: the solar geometry and the horizon
     // lookup are skipped by warps without such a point (7 % on a grid with 30 % of them scattered)
     for (auto& kv : by_window)
-      std::stable_partition(kv.second.begin(), kv.second.end(), [&](int p) {
-        const double sv = local[p]->sky_view;
-        return !(sv < 1.0 && sv > -0.01f);
-      });
+      std::stable_partition(kv.second.begin(), kv.second.end(),
+                            [&](int p) { return !sky_view_point(local[p]->sky_view); });
     std::vector<int> slots;  // point index or -1 (padding)
     std::vector<int> loose;
     if (by_window.count(-1)) loose = by_window[-1];
@@ -407,8 +536,7 @@ int run_shard(Shard& sh, OutputPointers* const* out, const InputPointers* const*
     std::atomic<bool> any_depth_a(false), any_sky_a(false);
     parallel_for(static_cast<int>(g.points.size()), host_threads(), [&](int k) {
       const int p = g.points[k];
-      const LocalParameters& lp = *local[p];
-      if (lp.sky_view < 1.0 && lp.sky_view > -0.01f) any_sky_a = true;
+      if (sky_view_point(local[p]->sky_view)) any_sky_a = true;
       if (!any_depth_a.load(std::memory_order_relaxed))  // depth(1), depth(SimLen) are read even with tsurfOutputDepth
       {
         const double* d = in[p]->c_Depth;
@@ -442,19 +570,18 @@ int run_shard(Shard& sh, OutputPointers* const* out, const InputPointers* const*
     const size_t stage_budget = 192ull << 20;
     int chunk = static_cast<int>(std::max<size_t>(32, stage_budget / (sizeof(double) * sim_len * nvar) / 32 * 32));
 
-    PooledDevice d_tf;
-    CU(d_tf.alloc(sh.device, 209, sizeof(int) * 6 * sim_len));
+    int* d_tf = nullptr;
+    CU(pooled(sh.device, RB_TIME_FIELDS, 6 * static_cast<size_t>(sim_len), &d_tf));
     {
-      const int* src[6] = {g.rep->c_year, g.rep->c_month, g.rep->c_day, g.rep->c_hour, g.rep->c_minute,
-                           g.rep->c_second};
+      const auto src = time_fields(*g.rep);
       for (int k = 0; k < 6; ++k)
-        CU(cudaMemcpyAsync(d_tf.as<int>() + static_cast<size_t>(k) * sim_len, src[k], sizeof(int) * sim_len,
+        CU(cudaMemcpyAsync(d_tf + static_cast<size_t>(k) * sim_len, src[k], sizeof(int) * sim_len,
                            cudaMemcpyHostToDevice, stream));
       sh.stats.h2d_bytes += sizeof(int) * 6 * sim_len;
     }
-    PooledDevice d_solar;
-    CU(d_solar.alloc(sh.device, 210, sizeof(double) * 4 * sim_len));
-    CU(static_cast<cudaError_t>(rs_launch_solar(d_tf.as<int>(), sim_len, d_solar.as<double>(), stream)));
+    double* d_solar = nullptr;
+    CU(pooled(sh.device, RB_SOLAR, 4 * static_cast<size_t>(sim_len), &d_solar));
+    CU(static_cast<cudaError_t>(rs_launch_solar(d_tf, sim_len, d_solar, stream)));
     ++sh.stats.kernel_launches;
 
     // ---- software pipeline over the device batches: while a helper thread copies batch b back and
@@ -462,11 +589,13 @@ int run_shard(Shard& sh, OutputPointers* const* out, const InputPointers* const*
     // and uploads batch b+1 into the other buffer set.  Each set has its own stream.
     struct Ctx
     {
-      PooledDevice d_forcing, d_out, d_local, d_hor, d_status, d_scratch, d_stage, d_stage2, d_counters, d_state;
-      PooledPinned h_stage, h_stage2, h_local, h_hor, h_status;
+      double *d_forcing = nullptr, *d_out = nullptr, *d_local = nullptr, *d_hor = nullptr, *d_scratch = nullptr,
+             *d_state = nullptr, *d_stage[2] = {}, *h_stage[2] = {}, *h_local = nullptr, *h_hor = nullptr;
+      int *d_status = nullptr, *h_status = nullptr;
+      unsigned long long* d_counters = nullptr;
       cudaStream_t st = nullptr;
-      cudaEvent_t ev_free[2] = {nullptr, nullptr};                       // staging buffer reuse
-      cudaEvent_t ev_in0 = nullptr, ev_in1 = nullptr, ev_k1 = nullptr, ev_o1 = nullptr;
+      cudaEvent_t ev_free[2] = {nullptr, nullptr};  // staging buffer reuse
+      cudaEvent_t ev[4] = {};                       // input stage begins, ends; kernels end; output stage ends
       size_t s0 = 0;
       int ld = 0, chunk = 0;
       RsBatchStats out_stats{};   // what the helper thread measured
@@ -483,7 +612,9 @@ int run_shard(Shard& sh, OutputPointers* const* out, const InputPointers* const*
         for (int k = 0; k < 2; ++k)
         {
           if (c[k].drain.joinable()) c[k].drain.join();
-          for (cudaEvent_t e : {c[k].ev_free[0], c[k].ev_free[1], c[k].ev_in0, c[k].ev_in1, c[k].ev_k1, c[k].ev_o1})
+          for (cudaEvent_t e : c[k].ev_free)
+            if (e) cudaEventDestroy(e);
+          for (cudaEvent_t e : c[k].ev)
             if (e) cudaEventDestroy(e);
           if (c[k].st) cudaStreamDestroy(c[k].st);
         }
@@ -496,28 +627,27 @@ int run_shard(Shard& sh, OutputPointers* const* out, const InputPointers* const*
     for (int k = 0; k < (nbatches > 1 ? 2 : 1); ++k)
     {
       Ctx& c = ctx[k];
-      const int o = 50 * k;  // pool slots of the second buffer set
+      const int o = RB_SET2 * k;
       CU(cudaStreamCreateWithFlags(&c.st, cudaStreamNonBlocking));
-      for (cudaEvent_t* e : {&c.ev_free[0], &c.ev_free[1]}) CU(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
-      for (cudaEvent_t* e : {&c.ev_in0, &c.ev_in1, &c.ev_k1, &c.ev_o1}) CU(cudaEventCreate(e));
+      for (cudaEvent_t& e : c.ev_free) CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+      for (cudaEvent_t& e : c.ev) CU(cudaEventCreate(&e));
       c.chunk = static_cast<int>(std::min<size_t>(chunk, max_ld));
-      CU(c.d_forcing.alloc(dv, 200 + o, sizeof(double) * sim_len * nvar * max_ld));
-      CU(c.d_out.alloc(dv, 201 + o, sizeof(double) * RS_O_NVAR * sim_len * max_ld));
-      CU(c.d_local.alloc(dv, 202 + o, sizeof(double) * RS_L_NLOCAL * max_ld));
-      if (any_sky) CU(c.d_hor.alloc(dv, 203 + o, sizeof(double) * 360 * max_ld));
-      CU(c.d_status.alloc(dv, 204 + o, sizeof(int) * max_ld));
-      if (model.use_coupling) CU(c.d_scratch.alloc(dv, 205 + o, sizeof(double) * RS_SCRATCH_NPLANES(nl) * max_ld));
-      if (wend > 0) CU(c.d_state.alloc(dv, 211 + o, sizeof(double) * RS_STATE_NPLANES(nl) * max_ld));
-      const size_t stage_bytes =
-          sizeof(double) * static_cast<size_t>(c.chunk) * sim_len * std::max(nvar, static_cast<int>(RS_O_NVAR));
-      CU(c.d_stage.alloc(dv, 206 + o, stage_bytes));
-      CU(c.d_stage2.alloc(dv, 207 + o, stage_bytes));
-      CU(c.d_counters.alloc(dv, 208 + o, sizeof(unsigned long long) * RS_CNT_N));
-      CU(c.h_stage.alloc(dv, 0 + o, stage_bytes));
-      CU(c.h_stage2.alloc(dv, 1 + o, stage_bytes));
-      CU(c.h_local.alloc(dv, 2 + o, sizeof(double) * RS_L_NLOCAL * max_ld));
-      if (any_sky) CU(c.h_hor.alloc(dv, 3 + o, sizeof(double) * 360 * max_ld));
-      CU(c.h_status.alloc(dv, 4 + o, sizeof(int) * max_ld));
+      CU(pooled(dv, RB_FORCING + o, static_cast<size_t>(sim_len) * nvar * max_ld, &c.d_forcing));
+      CU(pooled(dv, RB_OUT + o, static_cast<size_t>(RS_O_NVAR) * sim_len * max_ld, &c.d_out));
+      CU(pooled(dv, RB_LOCAL + o, RS_L_NLOCAL * max_ld, &c.d_local));
+      if (any_sky) CU(pooled(dv, RB_HOR + o, 360 * max_ld, &c.d_hor));
+      CU(pooled(dv, RB_STATUS + o, max_ld, &c.d_status));
+      if (model.use_coupling) CU(pooled(dv, RB_SCRATCH + o, RS_SCRATCH_NPLANES(nl) * max_ld, &c.d_scratch));
+      if (wend > 0) CU(pooled(dv, RB_STATE + o, RS_STATE_NPLANES(nl) * max_ld, &c.d_state));
+      const size_t stage_n = static_cast<size_t>(c.chunk) * sim_len * std::max(nvar, static_cast<int>(RS_O_NVAR));
+      CU(pooled(dv, RB_STAGE + o, stage_n, &c.d_stage[0]));
+      CU(pooled(dv, RB_STAGE2 + o, stage_n, &c.d_stage[1]));
+      CU(pooled(dv, RB_COUNTERS + o, RS_CNT_N, &c.d_counters));
+      CU(pooled_pinned(dv, RB_H_STAGE + o, stage_n, &c.h_stage[0]));
+      CU(pooled_pinned(dv, RB_H_STAGE2 + o, stage_n, &c.h_stage[1]));
+      CU(pooled_pinned(dv, RB_H_LOCAL + o, RS_L_NLOCAL * max_ld, &c.h_local));
+      if (any_sky) CU(pooled_pinned(dv, RB_H_HOR + o, 360 * max_ld, &c.h_hor));
+      CU(pooled_pinned(dv, RB_H_STATUS + o, max_ld, &c.h_status));
     }
     // the time axis and the solar table were queued on `stream`: every batch stream reads them
     CU(cudaStreamSynchronize(stream));
@@ -530,32 +660,17 @@ int run_shard(Shard& sh, OutputPointers* const* out, const InputPointers* const*
       const int ld = c.ld;
       const size_t s0 = c.s0;
       cudaStream_t st = c.st;
-      double* h_st[2] = {c.h_stage.as<double>(), c.h_stage2.as<double>()};
-      double* d_st[2] = {c.d_stage.as<double>(), c.d_stage2.as<double>()};
-      CU(cudaMemsetAsync(c.d_counters.p, 0, sizeof(unsigned long long) * RS_CNT_N, st));
+      CU(cudaMemsetAsync(c.d_counters, 0, sizeof(unsigned long long) * RS_CNT_N, st));
       double t0 = now_ms();
       {
-        double* L = c.h_local.as<double>();
         for (int q = 0; q < ld; ++q)
         {
           const int p = slots[s0 + q];
-          LocalParameters lp;
-          std::memset(&lp, 0, sizeof lp);
-          if (p >= 0) lp = *local[p];
-          L[RS_L_TAIR_RELAX * (size_t)ld + q] = lp.tair_relax;
-          L[RS_L_VZ_RELAX * (size_t)ld + q] = lp.VZ_relax;
-          L[RS_L_RH_RELAX * (size_t)ld + q] = lp.RH_relax;
-          L[RS_L_COUPLING_TSURF * (size_t)ld + q] = lp.couplingTsurf;
-          L[RS_L_LAT * (size_t)ld + q] = lp.lat;
-          L[RS_L_LON * (size_t)ld + q] = lp.lon;
-          L[RS_L_SKY_VIEW * (size_t)ld + q] = (p >= 0) ? lp.sky_view : 1.0;
-          L[RS_L_COUPLING_INDEX * (size_t)ld + q] = lp.couplingIndexI;
-          L[RS_L_INIT_LEN * (size_t)ld + q] = lp.InitLenI;
-          L[RS_L_ACTIVE * (size_t)ld + q] = (p >= 0) ? 1.0 : 0.0;
+          local_row(p >= 0 ? local[p] : nullptr, c.h_local + q, ld);
         }
         if (any_sky)
         {
-          double* H = c.h_hor.as<double>();
+          double* H = c.h_hor;
           for (int q = 0; q < ld; ++q)
           {
             const int p = slots[s0 + q];
@@ -565,12 +680,12 @@ int run_shard(Shard& sh, OutputPointers* const* out, const InputPointers* const*
         }
       }
       sh.stats.pack_ms += now_ms() - t0;
-      CU(cudaEventRecord(c.ev_in0, st));
-      CU(cudaMemcpyAsync(c.d_local.p, c.h_local.p, sizeof(double) * RS_L_NLOCAL * ld, cudaMemcpyHostToDevice, st));
+      CU(cudaEventRecord(c.ev[0], st));
+      CU(cudaMemcpyAsync(c.d_local, c.h_local, sizeof(double) * RS_L_NLOCAL * ld, cudaMemcpyHostToDevice, st));
       sh.stats.h2d_bytes += sizeof(double) * RS_L_NLOCAL * ld;
       if (any_sky)
       {
-        CU(cudaMemcpyAsync(c.d_hor.p, c.h_hor.p, sizeof(double) * 360 * ld, cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(c.d_hor, c.h_hor, sizeof(double) * 360 * ld, cudaMemcpyHostToDevice, st));
         sh.stats.h2d_bytes += sizeof(double) * 360 * ld;
       }
       int cidx = 0;
@@ -580,7 +695,7 @@ int run_shard(Shard& sh, OutputPointers* const* out, const InputPointers* const*
         const int bsel = cidx & 1;
         if (cidx >= 2) CU(cudaEventSynchronize(c.ev_free[bsel]));
         t0 = now_ms();
-        double* S = h_st[bsel];
+        double* S = c.h_stage[bsel];
         const size_t plane = static_cast<size_t>(npc) * sim_len;
         parallel_for(npc, nthreads, [&](int q) {
           const int p = slots[s0 + q0 + q];
@@ -590,29 +705,18 @@ int run_shard(Shard& sh, OutputPointers* const* out, const InputPointers* const*
             for (int v = 0; v < nvar; ++v) std::memset(S + v * plane + row, 0, sizeof(double) * sim_len);
             return;
           }
-          const InputPointers* ip = in[p];
-          const double* src[RS_F_NVAR_DEPTH] = {ip->c_tair, ip->c_tdew, ip->c_VZ,     ip->c_Rhz,
-                                                ip->c_prec, ip->c_SW,   ip->c_LW,     ip->c_SW_dir,
-                                                ip->c_LW_net, ip->c_TSurfObs, nullptr, ip->c_Depth};
-          for (int v = 0; v < nvar; ++v)
-          {
-            double* dst = S + v * plane + row;
-            if (v == RS_F_PHASE)
-              for (int t = 0; t < sim_len; ++t) dst[t] = static_cast<double>(ip->c_PrecPhase[t]);
-            else
-              std::memcpy(dst, src[v], sizeof(double) * sim_len);
-          }
+          for (int v = 0; v < nvar; ++v) forcing_row(*in[p], v, sim_len, S + v * plane + row, 1);
         });
         sh.stats.pack_ms += now_ms() - t0;
         const size_t bytes = sizeof(double) * plane * nvar;
-        CU(cudaMemcpyAsync(d_st[bsel], S, bytes, cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(c.d_stage[bsel], S, bytes, cudaMemcpyHostToDevice, st));
         CU(static_cast<cudaError_t>(
-            rs_launch_pack_forcing(d_st[bsel], npc, q0, sim_len, nvar, c.d_forcing.as<double>(), ld, st)));
+            rs_launch_pack_forcing(c.d_stage[bsel], npc, q0, sim_len, nvar, c.d_forcing, ld, st)));
         CU(cudaEventRecord(c.ev_free[bsel], st));
         ++sh.stats.kernel_launches;
         sh.stats.h2d_bytes += bytes;
       }
-      CU(cudaEventRecord(c.ev_in1, st));
+      CU(cudaEventRecord(c.ev[1], st));
 
       // ---- the step kernel(s), queued behind the input stage
       RsArgs a;
@@ -629,27 +733,27 @@ int run_shard(Shard& sh, OutputPointers* const* out, const InputPointers* const*
       a.step_end = sim_len;
       a.forcing_step0 = 1;
       a.out_slot0 = 0;
-      a.forcing = c.d_forcing.as<double>();
-      a.tf = d_tf.as<int>();
-      a.local = c.d_local.as<double>();
-      a.horizons = any_sky ? c.d_hor.as<double>() : nullptr;
-      a.solar = d_solar.as<double>();
-      a.out = c.d_out.as<double>();
-      a.status = c.d_status.as<int>();
-      a.scratch = model.use_coupling ? c.d_scratch.as<double>() : nullptr;
+      a.forcing = c.d_forcing;
+      a.tf = d_tf;
+      a.local = c.d_local;
+      a.horizons = any_sky ? c.d_hor : nullptr;
+      a.solar = d_solar;
+      a.out = c.d_out;
+      a.status = c.d_status;
+      a.scratch = model.use_coupling ? c.d_scratch : nullptr;
       RsArgsCold ac;
       std::memset(&ac, 0, sizeof ac);
-      ac.counters = c.d_counters.as<unsigned long long>();
+      ac.counters = c.d_counters;
       ac.out_start = 0;
       ac.out_nvar = RS_O_NVAR;
-      ac.state = wend > 0 ? c.d_state.as<double>() : nullptr;
+      ac.state = wend > 0 ? c.d_state : nullptr;
       {
         int n = 0;
         const int rc = launch_model(a, ac, model, wend, st, &sh.launch, &n);
         if (rc != RS_OK) return rc;
         sh.stats.kernel_launches += n;
       }
-      CU(cudaEventRecord(c.ev_k1, st));
+      CU(cudaEventRecord(c.ev[2], st));
       sh.launch.nlayers = nl;
       sh.launch.forcing_mode = 0;
       return RS_OK;
@@ -662,17 +766,13 @@ int run_shard(Shard& sh, OutputPointers* const* out, const InputPointers* const*
       const int ld = c.ld;
       const size_t s0 = c.s0;
       cudaStream_t st = c.st;
-      double* h_st[2] = {c.h_stage.as<double>(), c.h_stage2.as<double>()};
-      double* d_st[2] = {c.d_stage.as<double>(), c.d_stage2.as<double>()};
       RsBatchStats& os = c.out_stats;
       auto scatter = [&](int q0, int npc, const double* S) {
         const size_t plane = static_cast<size_t>(npc) * sim_len;
         parallel_for(npc, nthreads, [&](int q) {
           const int p = slots[s0 + q0 + q];
           if (p < 0) return;
-          OutputPointers* op = out[p];
-          double* dst[RS_O_NVAR] = {op->c_TsurfOut, op->c_SnowOut, op->c_WaterOut,
-                                    op->c_IceOut,   op->c_DepositOut, op->c_Ice2Out};
+          const auto dst = output_planes(*out[p]);
           for (int v = 0; v < RS_O_NVAR; ++v)
             std::memcpy(dst[v], S + v * plane + static_cast<size_t>(q) * sim_len, sizeof(double) * sim_len);
         });
@@ -683,9 +783,9 @@ int run_shard(Shard& sh, OutputPointers* const* out, const InputPointers* const*
         const int npc = std::min(c.chunk, ld - q0);
         const int bsel = cidx & 1;
         const size_t bytes = sizeof(double) * static_cast<size_t>(npc) * sim_len * RS_O_NVAR;
-        CU(static_cast<cudaError_t>(rs_launch_unpack_out(c.d_out.as<double>(), ld, sim_len, q0, npc, d_st[bsel], st)));
+        CU(static_cast<cudaError_t>(rs_launch_unpack_out(c.d_out, ld, sim_len, q0, npc, c.d_stage[bsel], st)));
         ++os.kernel_launches;
-        CU(cudaMemcpyAsync(h_st[bsel], d_st[bsel], bytes, cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(c.h_stage[bsel], c.d_stage[bsel], bytes, cudaMemcpyDeviceToHost, st));
         CU(cudaEventRecord(c.ev_free[bsel], st));
         os.d2h_bytes += bytes;
         if (prev_q0 >= 0)
@@ -693,38 +793,38 @@ int run_shard(Shard& sh, OutputPointers* const* out, const InputPointers* const*
           // buffer of the previous chunk: its copy was enqueued before this one
           CU(cudaEventSynchronize(c.ev_free[bsel ^ 1]));
           const double t0 = now_ms();
-          scatter(prev_q0, prev_npc, h_st[bsel ^ 1]);
+          scatter(prev_q0, prev_npc, c.h_stage[bsel ^ 1]);
           os.unpack_ms += now_ms() - t0;
         }
         prev_q0 = q0;
         prev_npc = npc;
       }
-      CU(cudaEventRecord(c.ev_o1, st));
+      CU(cudaEventRecord(c.ev[3], st));
       if (prev_q0 >= 0)
       {
         CU(cudaEventSynchronize(c.ev_free[(cidx - 1) & 1]));
         const double t0 = now_ms();
-        scatter(prev_q0, prev_npc, h_st[(cidx - 1) & 1]);
+        scatter(prev_q0, prev_npc, c.h_stage[(cidx - 1) & 1]);
         os.unpack_ms += now_ms() - t0;
       }
       if (g_opt_write_back.load())
       {
         // the reference's caller-visible input mutations (see rs_mutation_kernel), chunk by chunk through the
         // first staging buffer; VZ(1) is clamped on the host (src/Initialization.f90:121-123)
-        PooledDevice d_nvis;
-        CU(d_nvis.alloc(dv, 212 + (&c == &ctx[1] ? 50 : 0), sizeof(int) * ld));
+        int* d_nvis = nullptr;
+        CU(pooled(dv, RB_NVIS + (&c == &ctx[1] ? RB_SET2 : 0), ld, &d_nvis));
         for (int q0 = 0; q0 < ld; q0 += c.chunk)
         {
           const int npc = std::min(c.chunk, ld - q0);
           const size_t plane = static_cast<size_t>(npc) * sim_len;
-          CU(static_cast<cudaError_t>(rs_launch_mutation(c.d_forcing.as<double>(), nvar, ld, sim_len, c.d_local.as<double>(),
-                                                         any_sky ? c.d_hor.as<double>() : nullptr, d_solar.as<double>(),
-                                                         c.d_out.as<double>(), d_nvis.as<int>(), q0, npc, d_st[0], st)));
+          CU(static_cast<cudaError_t>(rs_launch_mutation(c.d_forcing, nvar, ld, sim_len, c.d_local,
+                                                         any_sky ? c.d_hor : nullptr, d_solar,
+                                                         c.d_out, d_nvis, q0, npc, c.d_stage[0], st)));
           os.kernel_launches += q0 == 0 ? 2 : 1;
-          CU(cudaMemcpyAsync(h_st[0], d_st[0], sizeof(double) * 3 * plane, cudaMemcpyDeviceToHost, st));
+          CU(cudaMemcpyAsync(c.h_stage[0], c.d_stage[0], sizeof(double) * 3 * plane, cudaMemcpyDeviceToHost, st));
           CU(cudaStreamSynchronize(st));
           os.d2h_bytes += sizeof(double) * 3 * plane;
-          const double* S = h_st[0];
+          const double* S = c.h_stage[0];
           parallel_for(npc, nthreads, [&](int q) {
             const int p = slots[s0 + q0 + q];
             if (p < 0) return;
@@ -736,24 +836,18 @@ int run_shard(Shard& sh, OutputPointers* const* out, const InputPointers* const*
           });
         }
       }
-      CU(cudaMemcpyAsync(c.h_status.p, c.d_status.p, sizeof(int) * ld, cudaMemcpyDeviceToHost, st));
+      CU(cudaMemcpyAsync(c.h_status, c.d_status, sizeof(int) * ld, cudaMemcpyDeviceToHost, st));
       unsigned long long cnt[RS_CNT_N];
-      CU(cudaMemcpyAsync(cnt, c.d_counters.p, sizeof cnt, cudaMemcpyDeviceToHost, st));
+      CU(cudaMemcpyAsync(cnt, c.d_counters, sizeof cnt, cudaMemcpyDeviceToHost, st));
       CU(cudaStreamSynchronize(st));
-      float ms = 0.f;
-      cudaEventElapsedTime(&ms, c.ev_in0, c.ev_in1);
-      os.h2d_ms += ms;  // device-side time of the input stage (copies + transposes, overlapped with packing)
-      cudaEventElapsedTime(&ms, c.ev_in1, c.ev_k1);
-      os.kernel_ms += ms;
-      cudaEventElapsedTime(&ms, c.ev_k1, c.ev_o1);
-      os.d2h_ms += ms;
+      add_stage_times(os, c.ev);  // h2d: device-side time of the input stage (copies + transposes, overlapped with packing)
       os.d2h_bytes += sizeof(int) * ld;
       os.executed_steps += static_cast<int64_t>(cnt[RS_CNT_EXECUTED_STEPS]);
       if (status)
         for (int q = 0; q < ld; ++q)
         {
           const int p = slots[s0 + q];
-          if (p >= 0) status[p] = c.h_status.as<int>()[q];
+          if (p >= 0) status[p] = c.h_status[q];
         }
       return RS_OK;
     };
@@ -833,9 +927,9 @@ struct StaticsChunk
   int* order = nullptr;   // [ld]
   int ld = 0;
 };
-struct StaticsShard
+struct StaticsShard : ShardRange
 {
-  int device = 0, first = 0, count = 0, chunk = 0;
+  int chunk = 0;
   std::vector<StaticsChunk> chunks;
 };
 struct RsStatics
@@ -912,58 +1006,31 @@ int run_host_soa_shard(Shard& sh, const RsHostBatch* b, const InputSettings* set
   cudaEvent_t(*ev)[4] = ss->ev;
 
   // per-stream device buffers
-  double *d_forcing[NSTREAM], *d_out[NSTREAM], *d_local[NSTREAM], *d_hor[NSTREAM], *d_scratch[NSTREAM],
-      *d_state[NSTREAM];
   const int wend = (model.use_coupling && opt_compaction_passes() > 0) ? b->coupling_window_end : 0;
-  int* d_status[NSTREAM];
-  int* d_order[NSTREAM];
-  unsigned long long* d_counters = nullptr;
-  int *d_tf = nullptr, *d_rs = nullptr;
-  void* tmp = nullptr;
+  double *d_forcing[NSTREAM], *d_out[NSTREAM], *d_local[NSTREAM], *d_hor[NSTREAM] = {}, *d_scratch[NSTREAM] = {},
+         *d_state[NSTREAM] = {};
+  int *d_status[NSTREAM], *d_order[NSTREAM] = {};
+  const size_t cols = chunk;
   for (int s = 0; s < NSTREAM; ++s)
   {
-    CU(pool_get(sh.device, 10 * s + 0, sizeof(double) * frows * chunk, &tmp));
-    d_forcing[s] = static_cast<double*>(tmp);
-    CU(pool_get(sh.device, 10 * s + 1, sizeof(double) * orows * chunk, &tmp));
-    d_out[s] = static_cast<double*>(tmp);
-    CU(pool_get(sh.device, 10 * s + 2, sizeof(double) * RS_L_NLOCAL * chunk, &tmp));
-    d_local[s] = static_cast<double*>(tmp);
-    d_hor[s] = nullptr;
-    if (hor && !resident)
-    {
-      CU(pool_get(sh.device, 10 * s + 3, sizeof(double) * 360 * chunk, &tmp));
-      d_hor[s] = static_cast<double*>(tmp);
-    }
-    d_scratch[s] = nullptr;
-    if (model.use_coupling)
-    {
-      CU(pool_get(sh.device, 10 * s + 4, sizeof(double) * RS_SCRATCH_NPLANES(nl) * chunk, &tmp));
-      d_scratch[s] = static_cast<double*>(tmp);
-    }
-    CU(pool_get(sh.device, 10 * s + 5, sizeof(int) * chunk, &tmp));
-    d_status[s] = static_cast<int*>(tmp);
-    d_state[s] = nullptr;
-    if (wend > 0)
-    {
-      CU(pool_get(sh.device, 10 * s + 6, sizeof(double) * RS_STATE_NPLANES(nl) * chunk, &tmp));
-      d_state[s] = static_cast<double*>(tmp);
-    }
-    d_order[s] = nullptr;
+    const int o = HS_STREAM * s;
+    CU(pooled(sh.device, HS_FORCING + o, frows * cols, &d_forcing[s]));
+    CU(pooled(sh.device, HS_OUT + o, orows * cols, &d_out[s]));
+    CU(pooled(sh.device, HS_LOCAL + o, RS_L_NLOCAL * cols, &d_local[s]));
+    if (hor && !resident) CU(pooled(sh.device, HS_HOR + o, 360 * cols, &d_hor[s]));
+    if (model.use_coupling) CU(pooled(sh.device, HS_SCRATCH + o, RS_SCRATCH_NPLANES(nl) * cols, &d_scratch[s]));
+    CU(pooled(sh.device, HS_STATUS + o, cols, &d_status[s]));
+    if (wend > 0) CU(pooled(sh.device, HS_STATE + o, RS_STATE_NPLANES(nl) * cols, &d_state[s]));
     if (hor && !resident && b->forcing_mode == 1)  // sky-view points gathered at one end of the chunk (see roadsurf_order_points)
-    {
-      CU(pool_get(sh.device, 10 * s + 7, sizeof(int) * chunk, &tmp));
-      d_order[s] = static_cast<int*>(tmp);
-    }
+      CU(pooled(sh.device, HS_ORDER + o, cols, &d_order[s]));
   }
-  CU(pool_get(sh.device, 100, sizeof(int) * 6 * b->sim_len, &tmp));
-  d_tf = static_cast<int*>(tmp);
-  CU(pool_get(sh.device, 101, sizeof(int) * std::max(1, b->n_records), &tmp));
-  d_rs = static_cast<int*>(tmp);
-  CU(pool_get(sh.device, 102, sizeof(unsigned long long) * RS_CNT_N, &tmp));
-  d_counters = static_cast<unsigned long long*>(tmp);
+  int *d_tf = nullptr, *d_rs = nullptr;
+  unsigned long long* d_counters = nullptr;
   double* d_solar = nullptr;
-  CU(pool_get(sh.device, 103, sizeof(double) * 4 * b->sim_len, &tmp));
-  d_solar = static_cast<double*>(tmp);
+  CU(pooled(sh.device, HS_TIME_FIELDS, 6 * static_cast<size_t>(b->sim_len), &d_tf));
+  CU(pooled(sh.device, HS_RECORD_STEP, std::max(1, b->n_records), &d_rs));
+  CU(pooled(sh.device, HS_COUNTERS, RS_CNT_N, &d_counters));
+  CU(pooled(sh.device, HS_SOLAR, 4 * static_cast<size_t>(b->sim_len), &d_solar));
   CU(cudaMemcpyAsync(d_tf, b->time_fields, sizeof(int) * 6 * b->sim_len, cudaMemcpyHostToDevice, streams[0]));
   if (b->forcing_mode == 1)
     CU(cudaMemcpyAsync(d_rs, b->record_step, sizeof(int) * b->n_records, cudaMemcpyHostToDevice, streams[0]));
@@ -985,13 +1052,7 @@ int run_host_soa_shard(Shard& sh, const RsHostBatch* b, const InputSettings* set
     {
       // buffers of this stream are free once its previous chunk's D2H has finished
       CU(cudaStreamSynchronize(st));
-      float ms = 0.f;
-      cudaEventElapsedTime(&ms, ev[s][0], ev[s][1]);
-      sh.stats.h2d_ms += ms;
-      cudaEventElapsedTime(&ms, ev[s][1], ev[s][2]);
-      sh.stats.kernel_ms += ms;
-      cudaEventElapsedTime(&ms, ev[s][2], ev[s][3]);
-      sh.stats.d2h_ms += ms;
+      add_stage_times(sh.stats, ev[s]);
     }
     const size_t wbytes = sizeof(double) * npc;
     CU(cudaEventRecord(ev[s][0], st));
@@ -1065,13 +1126,7 @@ int run_host_soa_shard(Shard& sh, const RsHostBatch* b, const InputSettings* set
   for (int s = 0; s < NSTREAM && s < nchunks; ++s)
   {
     CU(cudaStreamSynchronize(streams[s]));
-    float ms = 0.f;
-    cudaEventElapsedTime(&ms, ev[s][0], ev[s][1]);
-    sh.stats.h2d_ms += ms;
-    cudaEventElapsedTime(&ms, ev[s][1], ev[s][2]);
-    sh.stats.kernel_ms += ms;
-    cudaEventElapsedTime(&ms, ev[s][2], ev[s][3]);
-    sh.stats.d2h_ms += ms;
+    add_stage_times(sh.stats, ev[s]);
   }
   unsigned long long cnt[RS_CNT_N];
   CU(cudaMemcpy(cnt, d_counters, sizeof cnt, cudaMemcpyDeviceToHost));
@@ -1083,21 +1138,15 @@ int run_host_soa_shard(Shard& sh, const RsHostBatch* b, const InputSettings* set
 int run_sharded(int npoints, int ngpus, const std::function<int(Shard&)>& fn)
 {
   const double wall0 = now_ms();
-  const int ndev = roadsurf_device_count();
-  if (ndev < 1) return fail(RS_ERR_NO_DEVICE, "no CUDA device visible (this library has no CPU path)");
-  if (ngpus <= 0 || ngpus > ndev) ngpus = ndev;
-  if (ngpus > npoints) ngpus = npoints;
   int current = 0;
-  cudaGetDevice(&current);
-  std::vector<Shard> shards(ngpus);
-  for (int g = 0; g < ngpus; ++g)
+  std::vector<ShardRange> ranges;
   {
-    const long long a = static_cast<long long>(npoints) * g / ngpus;
-    const long long b = static_cast<long long>(npoints) * (g + 1) / ngpus;
-    shards[g].first = static_cast<int>(a);
-    shards[g].count = static_cast<int>(b - a);
-    shards[g].device = (ngpus == 1) ? current : g;
+    const int rc = split_shards(npoints, ngpus, &current, &ranges);
+    if (rc != RS_OK) return rc;
   }
+  ngpus = static_cast<int>(ranges.size());
+  std::vector<Shard> shards(ngpus);
+  for (int g = 0; g < ngpus; ++g) static_cast<ShardRange&>(shards[g]) = ranges[g];
   auto work = [&](int g) {
     Shard& sh = shards[g];
     sh.rc = fn(sh);
@@ -1176,24 +1225,19 @@ int roadsurf_prepare_statics(const RsHostBatch* b, int ngpus, void** handle)
 {
   g_err.clear();
   if (!b || !handle || b->npoints < 1 || !b->local) return fail(RS_ERR_BAD_ARGUMENT, "bad arguments");
-  const int ndev = roadsurf_device_count();
-  if (ndev < 1) return fail(RS_ERR_NO_DEVICE, "no CUDA device visible (this library has no CPU path)");
-  if (ngpus <= 0 || ngpus > ndev) ngpus = ndev;
-  if (ngpus > b->npoints) ngpus = b->npoints;
   int current = 0;
-  cudaGetDevice(&current);
+  std::vector<ShardRange> ranges;
+  int rc = split_shards(b->npoints, ngpus, &current, &ranges);
+  if (rc != RS_OK) return rc;
   RsStatics* h = new RsStatics;
   h->npoints = b->npoints;
-  h->ngpus = ngpus;
+  h->ngpus = static_cast<int>(ranges.size());
   h->has_horizons = b->horizons != nullptr;
   const size_t np_all = static_cast<size_t>(b->npoints);
-  int rc = RS_OK;
-  for (int g = 0; g < ngpus && rc == RS_OK; ++g)
+  for (size_t g = 0; g < ranges.size() && rc == RS_OK; ++g)
   {
     StaticsShard s;
-    s.first = static_cast<int>(static_cast<long long>(b->npoints) * g / ngpus);
-    s.count = static_cast<int>(static_cast<long long>(b->npoints) * (g + 1) / ngpus) - s.first;
-    s.device = (ngpus == 1) ? current : g;
+    static_cast<ShardRange&>(s) = ranges[g];
     s.chunk = host_soa_chunk(s.count);
     auto body = [&]() -> int {
       CU(cudaSetDevice(s.device));
@@ -1310,14 +1354,10 @@ int roadsurf_session_open(int npoints, OutputPointers* const* out, const InputPo
     const InputPointers* ip = in[p];
     if (ip->inputLen < sim_len || out[p]->outputLen < sim_len)
       return fail(RS_ERR_BAD_ARGUMENT, "inputLen/outputLen shorter than SimLen");
-    const size_t nb = sizeof(int) * sim_len;
-    const InputPointers* r = in[0];
-    if (p > 0 && (std::memcmp(r->c_year, ip->c_year, nb) || std::memcmp(r->c_month, ip->c_month, nb) ||
-                  std::memcmp(r->c_day, ip->c_day, nb) || std::memcmp(r->c_hour, ip->c_hour, nb) ||
-                  std::memcmp(r->c_minute, ip->c_minute, nb) || std::memcmp(r->c_second, ip->c_second, nb)))
+    if (p > 0 && !same_time_axis(*in[0], *ip, sim_len))
       return fail(RS_ERR_UNSUPPORTED, "the points of a session must share one time axis");
     const LocalParameters& lp = *local[p];
-    if (lp.sky_view < 1.0 && lp.sky_view > -0.01f) any_sky = true;
+    if (sky_view_point(lp.sky_view)) any_sky = true;
     for (int t = 0; t < sim_len && !any_depth; ++t) any_depth = ip->c_Depth[t] >= 0.0;
     const long long w = window_key(s->model, lp);
     if (w > 0)
@@ -1335,28 +1375,15 @@ int roadsurf_session_open(int npoints, OutputPointers* const* out, const InputPo
   std::vector<double> hf(static_cast<size_t>(sim_len) * nvar * ld, 0.0), hl(RS_L_NLOCAL * ld, 0.0);
   std::vector<double> hh(any_sky ? 360 * ld : 0, 0.0);
   s->outs.resize(npoints);
-  for (size_t q = 0; q < ld; ++q) hl[RS_L_SKY_VIEW * ld + q] = 1.0;
+  for (size_t q = 0; q < ld; ++q) local_row(q < static_cast<size_t>(npoints) ? local[q] : nullptr, &hl[q], ld);
   for (int p = 0; p < npoints; ++p)
   {
     const InputPointers* ip = in[p];
-    const double* src[RS_F_NVAR_DEPTH] = {ip->c_tair, ip->c_tdew, ip->c_VZ,     ip->c_Rhz,      ip->c_prec, ip->c_SW,
-                                          ip->c_LW,   ip->c_SW_dir, ip->c_LW_net, ip->c_TSurfObs, nullptr,    ip->c_Depth};
-    for (int t = 0; t < sim_len; ++t)
-      for (int v = 0; v < nvar; ++v)
-        hf[(static_cast<size_t>(t) * nvar + v) * ld + p] =
-            (v == RS_F_PHASE) ? static_cast<double>(ip->c_PrecPhase[t]) : src[v][t];
-    const LocalParameters& lp = *local[p];
-    const double row[RS_L_NLOCAL] = {lp.tair_relax, lp.VZ_relax, lp.RH_relax, lp.couplingTsurf, lp.lat, lp.lon,
-                                     lp.sky_view, static_cast<double>(lp.couplingIndexI),
-                                     static_cast<double>(lp.InitLenI), 1.0};
-    for (int k = 0; k < RS_L_NLOCAL; ++k) hl[k * ld + p] = row[k];
+    for (int v = 0; v < nvar; ++v) forcing_row(*ip, v, sim_len, &hf[static_cast<size_t>(v) * ld + p], nvar * ld);
     if (any_sky)
       for (int k = 0; k < 360; ++k) hh[static_cast<size_t>(k) * ld + p] = ip->c_local_horizons ? ip->c_local_horizons[k] : 0.0;
     s->outs[p] = *out[p];
-    double* o[RS_O_NVAR] = {out[p]->c_TsurfOut, out[p]->c_SnowOut,    out[p]->c_WaterOut,
-                            out[p]->c_IceOut,   out[p]->c_DepositOut, out[p]->c_Ice2Out};
-    for (int v = 0; v < RS_O_NVAR; ++v)
-      for (int t = 0; t < sim_len; ++t) o[v][t] = -9999.0;
+    for (double* o : output_planes(*out[p])) std::fill(o, o + sim_len, -9999.0);
   }
   CU(cudaStreamCreateWithFlags(&s->stream, cudaStreamNonBlocking));
   CU(cudaMalloc(&s->d_forcing, sizeof(double) * hf.size()));
@@ -1372,7 +1399,7 @@ int roadsurf_session_open(int npoints, OutputPointers* const* out, const InputPo
   CU(cudaMemcpyAsync(s->d_forcing, hf.data(), sizeof(double) * hf.size(), cudaMemcpyHostToDevice, s->stream));
   CU(cudaMemcpyAsync(s->d_local, hl.data(), sizeof(double) * hl.size(), cudaMemcpyHostToDevice, s->stream));
   if (any_sky) CU(cudaMemcpyAsync(s->d_hor, hh.data(), sizeof(double) * hh.size(), cudaMemcpyHostToDevice, s->stream));
-  const int* tf[6] = {in[0]->c_year, in[0]->c_month, in[0]->c_day, in[0]->c_hour, in[0]->c_minute, in[0]->c_second};
+  const auto tf = time_fields(*in[0]);
   for (int k = 0; k < 6; ++k)
     CU(cudaMemcpyAsync(s->d_tf + static_cast<size_t>(k) * sim_len, tf[k], sizeof(int) * sim_len, cudaMemcpyHostToDevice,
                        s->stream));
@@ -1415,18 +1442,10 @@ int roadsurf_step(void* session, int i)
   if (s->wend > 0 && begin <= s->wend + 1 && target >= s->wstart) target = std::max(target, std::min(s->wend + 1, s->sim_len));
   {
     std::lock_guard<std::mutex> device_lock(g_device_mu[s->device & 63]);
-    RsModel m;
     // (another caller may have replaced the device's model since the session was opened)
     {
-      std::lock_guard<std::mutex> lk(g_model_mu);
-      DeviceModel& dm = g_models[s->device];
-      if (!dm.valid || std::memcmp(&dm.m, &s->model, sizeof m) != 0)
-      {
-        for (auto& kv : dm.last_launch) CU(cudaEventSynchronize(kv.second));
-        CU(static_cast<cudaError_t>(rs_upload_model(&s->model)));
-        dm.m = s->model;
-        dm.valid = true;
-      }
+      const int rc = upload_model(s->device, s->model);
+      if (rc != RS_OK) return rc;
     }
     RsArgs a;
     std::memset(&a, 0, sizeof a);
@@ -1490,8 +1509,7 @@ int roadsurf_session_fetch(void* session, int i, int* status)
                     cudaMemcpyDeviceToHost));
     for (int p = 0; p < s->npoints; ++p)
     {
-      OutputPointers& op = s->outs[p];
-      double* dst[RS_O_NVAR] = {op.c_TsurfOut, op.c_SnowOut, op.c_WaterOut, op.c_IceOut, op.c_DepositOut, op.c_Ice2Out};
+      const auto dst = output_planes(s->outs[p]);
       for (int v = 0; v < RS_O_NVAR; ++v)
         for (int t = 0; t < n; ++t) dst[v][t0 + t] = h[(static_cast<size_t>(v) * n + t) * s->ld + p];
     }
@@ -1549,13 +1567,10 @@ int roadsurf_run_device(const RsDeviceBatch* b, void* stream)
   CU(cudaGetDevice(&dev));
   RsModel m;
   {
-    std::lock_guard<std::mutex> lk(g_model_mu);
-    auto it = g_models.find(dev);
-    if (it == g_models.end() || !it->second.valid)
-      return fail(RS_ERR_BAD_ARGUMENT, "roadsurf_set_model was not called on this device");
-    m = it->second.m;
+    const int rc = current_model(dev, &m);
+    if (rc != RS_OK) return rc;
   }
-  if (b->ld < 32 || b->ld % 32 != 0 || b->npoints < 0 || b->npoints > b->ld)
+  if (b->ld < 32|| b->ld % 32 != 0 || b->npoints < 0 || b->npoints > b->ld)
     return fail(RS_ERR_BAD_ARGUMENT, "ld must be a positive multiple of 32 and >= npoints");
   const int step_begin = b->step_begin > 0 ? b->step_begin : 1;
   const int step_end = b->step_end > 0 ? b->step_end : b->sim_len;
@@ -1567,12 +1582,10 @@ int roadsurf_run_device(const RsDeviceBatch* b, void* stream)
   if (b->out_start < 0 || b->out_start >= b->sim_len) return fail(RS_ERR_BAD_ARGUMENT, "out_start outside [0, sim_len)");
   if (b->out_nvar != 0 && b->out_nvar != RS_O_NVAR && b->out_nvar != RS_O_NVAR_EXT)
     return fail(RS_ERR_BAD_ARGUMENT, "out_nvar must be 0, RS_O_NVAR or RS_O_NVAR_EXT");
-  if (step_end - 1 >= b->out_start)
   {
-    const int k0 = step_begin - 1 - b->out_start;
-    const int first_slot = k0 > 0 ? (k0 + b->out_stride - 1) / b->out_stride : 0;
-    const int last_slot = (step_end - 1 - b->out_start) / b->out_stride;
-    if (last_slot >= first_slot && (first_slot < b->out_slot0 || last_slot - b->out_slot0 >= b->n_out))
+    int s0, s1;
+    slot_range(step_begin, step_end, b->out_start, b->out_stride, &s0, &s1);
+    if (s1 > s0 && (s0 < b->out_slot0 || s1 - b->out_slot0 > b->n_out))
       return fail(RS_ERR_BAD_ARGUMENT, "out tensor does not cover the output slots of [step_begin, step_end]");
   }
   if (step_begin > 1 && !b->state) return fail(RS_ERR_BAD_ARGUMENT, "step_begin > 1 needs batch->state from the previous chunk");
@@ -1684,15 +1697,12 @@ int roadsurf_expand_records(const RsDeviceBatch* b, int rule, int step_begin, in
     return fail(RS_ERR_BAD_ARGUMENT, "bad arguments");
   int dev = 0;
   CU(cudaGetDevice(&dev));
-  double DT;
+  RsModel m;
   {
-    std::lock_guard<std::mutex> lk(g_model_mu);
-    auto it = g_models.find(dev);
-    if (it == g_models.end() || !it->second.valid)
-      return fail(RS_ERR_BAD_ARGUMENT, "roadsurf_set_model was not called on this device");
-    DT = it->second.m.DT;
+    const int rc = current_model(dev, &m);
+    if (rc != RS_OK) return rc;
   }
-  CU(static_cast<cudaError_t>(rs_launch_expand(b->forcing, b->record_step, b->n_records, b->nvar, b->ld, b->npoints, rule, DT,
+  CU(static_cast<cudaError_t>(rs_launch_expand(b->forcing, b->record_step, b->n_records, b->nvar, b->ld, b->npoints, rule, m.DT,
                                                 step_begin, step_end, dst, stream)));
   ++g_launches_total;
   return RS_OK;
@@ -2012,19 +2022,8 @@ int roadsurf_read_input_derive_records(const RsHostBatch* b, const InputSettings
   });
   if (window_end)
   {
-    int w = 0;
-    bool differs = false;
-    if (settings->use_coupling == 1)
-      for (size_t p = 0; p < np; ++p)
-      {
-        const double ts = local[RS_L_COUPLING_TSURF * np + p], ix = local[RS_L_COUPLING_INDEX * np + p];
-        if (local[RS_L_ACTIVE * np + p] == 0.0 || ts < -100 || ix < 1) continue;
-        if (w == 0)
-          w = static_cast<int>(ix);
-        else if (w != static_cast<int>(ix))
-          differs = true;
-      }
-    *window_end = differs ? 0 : w;
+    const int w = settings->use_coupling == 1 ? common_window_end(local, np) : 0;
+    *window_end = w < 0 ? 0 : w;  // windows that differ: no common window
   }
   return RS_OK;
 }
@@ -2083,11 +2082,9 @@ void mark_not_computed(OutputPointers* outPointers, const InputSettings* inSetti
   // The reference signature has no error channel: leave the outputs at -9999.0, which is how the
   // reference marks "not computed" (src/Initialization.f90:397-412).
   if (!outPointers || !inSettings) return;
-  double* o[RS_O_NVAR] = {outPointers->c_TsurfOut, outPointers->c_SnowOut,    outPointers->c_WaterOut,
-                          outPointers->c_IceOut,   outPointers->c_DepositOut, outPointers->c_Ice2Out};
-  for (int v = 0; v < RS_O_NVAR; ++v)
-    if (o[v])
-      for (int t = 0; t < inSettings->SimLen && t < outPointers->outputLen; ++t) o[v][t] = -9999.0;
+  for (double* o : output_planes(*outPointers))
+    if (o)
+      for (int t = 0; t < inSettings->SimLen && t < outPointers->outputLen; ++t) o[t] = -9999.0;
 }
 }  // namespace
 
@@ -2213,17 +2210,6 @@ extern "C" void runsimulation(OutputPointers* outPointers, const InputPointers* 
 // ---- ensemble runs (include/roadsurf_b200.h, part 3) -------------------------------------------------
 namespace
 {
-// Output slots of the steps [first, last] (1-based) as [slot_begin, slot_end); empty when none.
-void slot_range(int first, int last, int out_start, int out_stride, int* s0, int* s1)
-{
-  *s0 = *s1 = 0;
-  if (last - 1 < out_start || last < first) return;
-  const int k0 = first - 1 - out_start;
-  *s0 = k0 > 0 ? (k0 + out_stride - 1) / out_stride : 0;
-  *s1 = (last - 1 - out_start) / out_stride + 1;
-  if (*s1 < *s0) *s1 = *s0;
-}
-
 int check_stats_spec(const RsEnsembleStatsSpec& s, int out_nvar)
 {
   if (s.n_quantiles < 0 || s.n_quantiles > RS_ENS_MAX_QUANTILES || s.n_thresholds < 0 ||
@@ -2354,11 +2340,8 @@ int run_ensemble(const RsEnsembleBatch* e, void* stream, const int* host_record_
   CU(cudaGetDevice(&dev));
   RsModel m;
   {
-    std::lock_guard<std::mutex> lk(g_model_mu);
-    auto it = g_models.find(dev);
-    if (it == g_models.end() || !it->second.valid)
-      return fail(RS_ERR_BAD_ARGUMENT, "roadsurf_set_model was not called on this device");
-    m = it->second.m;
+    const int rc = current_model(dev, &m);
+    if (rc != RS_OK) return rc;
   }
   const int nl = m.nlayers;
   if (m.use_coupling && (!s.scratch || !e->member_scratch))
@@ -2498,16 +2481,8 @@ int roadsurf_run_ensemble_host_soa(const RsHostBatch* b, const double* member_re
   // one coupling window, and before the fork
   if (settings->use_coupling == 1)
   {
-    int w = 0;
-    for (size_t p = 0; p < np; ++p)
-    {
-      const double ts = b->local[RS_L_COUPLING_TSURF * np + p], ix = b->local[RS_L_COUPLING_INDEX * np + p];
-      if (b->local[RS_L_ACTIVE * np + p] == 0.0 || ts < -100 || ix < 1) continue;
-      if (w == 0)
-        w = static_cast<int>(ix);
-      else if (w != static_cast<int>(ix))
-        return fail(RS_ERR_UNSUPPORTED, "ensembles need one coupling window for all coupled stations");
-    }
+    const int w = common_window_end(b->local, np);
+    if (w < 0) return fail(RS_ERR_UNSUPPORTED, "ensembles need one coupling window for all coupled stations");
     if (w > 0 && F < w + 2)
       return fail(RS_ERR_BAD_ARGUMENT, "the coupling window [start, end + 1] must lie before the fork (F >= couplingIndexI + 2)");
   }
@@ -2526,9 +2501,7 @@ int roadsurf_run_ensemble_host_soa(const RsHostBatch* b, const double* member_re
   const double setup0 = now_ms();
   if (relax)
   {
-    void* hp = nullptr;
-    CU(pinned_get(dev, 400, sizeof(double) * 3 * npm, &hp));
-    relax_h = static_cast<double*>(hp);
+    CU(pooled_pinned(dev, EH_H_RELAX, 3 * npm, &relax_h));
     const int* rs = b->record_step;
     const double DT = settings->DTSecs;
     parallel_for(P, host_threads(), [&](int pi) {
@@ -2586,29 +2559,33 @@ int roadsurf_run_ensemble_host_soa(const RsHostBatch* b, const double* member_re
   }
   cudaStream_t st = ss->st[0];
   cudaEvent_t* ev = ss->ev[0];
-  void* tmp = nullptr;
-  auto dbuf = [&](int slot, size_t bytes, double** out) -> int {
-    CU(pool_get(dev, slot, bytes ? bytes : 8, &tmp));
-    *out = static_cast<double*>(tmp);
-    return RS_OK;
-  };
   double *d_forcing, *d_local, *d_hor = nullptr, *d_out, *d_state, *d_scratch = nullptr, *d_mf, *d_ml, *d_mh = nullptr,
-         *d_ms, *d_msc = nullptr, *d_mo, *d_relax = nullptr, *d_stats = nullptr, *d_prob = nullptr, *d_solar, *d_status,
-         *d_mstatus, *d_tf, *d_rs, *d_counters;
-  int rc = RS_OK;
+         *d_ms, *d_msc = nullptr, *d_mo, *d_relax = nullptr, *d_stats = nullptr, *d_prob = nullptr, *d_solar;
+  int *d_status, *d_mstatus, *d_tf, *d_rs;
+  unsigned long long* d_counters;
+  const size_t lc = ldc, lm = ldmc;
+  CU(pooled(dev, EH_FORCING, frows * lc, &d_forcing));
+  CU(pooled(dev, EH_LOCAL, RS_L_NLOCAL * lc, &d_local));
+  if (hor) CU(pooled(dev, EH_HOR, 360 * lc, &d_hor));
+  CU(pooled(dev, EH_OUT, RS_O_NVAR * n_pre * lc, &d_out));
+  CU(pooled(dev, EH_STATE, NS * lc, &d_state));
+  if (cpl) CU(pooled(dev, EH_SCRATCH, SC * lc, &d_scratch));
+  CU(pooled(dev, EH_M_FORCING, frows_m * lm, &d_mf));
+  CU(pooled(dev, EH_M_LOCAL, RS_L_NLOCAL * lm, &d_ml));
+  if (hor) CU(pooled(dev, EH_M_HOR, 360 * lm, &d_mh));
+  CU(pooled(dev, EH_M_STATE, NS * lm, &d_ms));
+  if (cpl) CU(pooled(dev, EH_M_SCRATCH, SC * lm, &d_msc));
+  CU(pooled(dev, EH_M_OUT, RS_O_NVAR * n_m * lm, &d_mo));
+  if (relax) CU(pooled(dev, EH_RELAX, 3 * lm, &d_relax));
+  CU(pooled(dev, EH_STATS, srows * lc, &d_stats));
+  if (np_planes) CU(pooled(dev, EH_PROB, prows * lc, &d_prob));
+  CU(pooled(dev, EH_SOLAR, 4 * static_cast<size_t>(sim_len), &d_solar));
+  CU(pooled(dev, EH_STATUS, lc, &d_status));
+  CU(pooled(dev, EH_M_STATUS, lm, &d_mstatus));
+  CU(pooled(dev, EH_TIME_FIELDS, 6 * static_cast<size_t>(sim_len), &d_tf));
+  CU(pooled(dev, EH_RECORD_STEP, nrec, &d_rs));
+  CU(pooled(dev, EH_COUNTERS, RS_CNT_N, &d_counters));
   const size_t D = sizeof(double);
-  if ((rc = dbuf(400, D * frows * ldc, &d_forcing)) || (rc = dbuf(401, D * RS_L_NLOCAL * ldc, &d_local)) ||
-      (hor && (rc = dbuf(402, D * 360 * ldc, &d_hor))) || (rc = dbuf(403, D * RS_O_NVAR * n_pre * ldc, &d_out)) ||
-      (rc = dbuf(404, D * NS * ldc, &d_state)) || (cpl && (rc = dbuf(405, D * SC * ldc, &d_scratch))) ||
-      (rc = dbuf(406, D * frows_m * ldmc, &d_mf)) || (rc = dbuf(407, D * RS_L_NLOCAL * ldmc, &d_ml)) ||
-      (hor && (rc = dbuf(408, D * 360 * ldmc, &d_mh))) || (rc = dbuf(409, D * NS * ldmc, &d_ms)) ||
-      (cpl && (rc = dbuf(410, D * SC * ldmc, &d_msc))) || (rc = dbuf(411, D * RS_O_NVAR * n_m * ldmc, &d_mo)) ||
-      (relax && (rc = dbuf(412, D * 3 * ldmc, &d_relax))) || (rc = dbuf(413, D * srows * ldc, &d_stats)) ||
-      (np_planes && (rc = dbuf(414, D * prows * ldc, &d_prob))) || (rc = dbuf(415, D * 4 * sim_len, &d_solar)) ||
-      (rc = dbuf(416, sizeof(int) * ldc, &d_status)) || (rc = dbuf(417, sizeof(int) * ldmc, &d_mstatus)) ||
-      (rc = dbuf(418, sizeof(int) * 6 * sim_len, &d_tf)) || (rc = dbuf(419, sizeof(int) * nrec, &d_rs)) ||
-      (rc = dbuf(420, sizeof(unsigned long long) * RS_CNT_N, &d_counters)))
-    return rc;
   CU(cudaMemcpyAsync(d_tf, b->time_fields, sizeof(int) * 6 * sim_len, cudaMemcpyHostToDevice, st));
   CU(cudaMemcpyAsync(d_rs, b->record_step, sizeof(int) * nrec, cudaMemcpyHostToDevice, st));
   CU(cudaMemsetAsync(d_counters, 0, sizeof(unsigned long long) * RS_CNT_N, st));
@@ -2641,17 +2618,17 @@ int roadsurf_run_ensemble_host_soa(const RsHostBatch* b, const double* member_re
     s.n_records = nrec;
     s.nvar = nvar;
     s.forcing = d_forcing;
-    s.record_step = reinterpret_cast<const int*>(d_rs);
-    s.time_fields = reinterpret_cast<const int*>(d_tf);
+    s.record_step = d_rs;
+    s.time_fields = d_tf;
     s.local = d_local;
     s.horizons = hor ? d_hor : nullptr;
     s.out = d_out;
     s.out_stride = b->out_stride;
     s.n_out = n_pre;
-    s.status = reinterpret_cast<int*>(d_status);
+    s.status = d_status;
     s.state = d_state;
     s.scratch = d_scratch;
-    s.counters = reinterpret_cast<unsigned long long*>(d_counters);
+    s.counters = d_counters;
     s.solar = d_solar;
     s.out_nvar = RS_O_NVAR;
     s.coupling_window_end = (cpl && opt_compaction_passes() > 0) ? b->coupling_window_end : 0;
@@ -2664,14 +2641,16 @@ int roadsurf_run_ensemble_host_soa(const RsHostBatch* b, const double* member_re
     e.member_horizons = d_mh;
     e.member_state = d_ms;
     e.member_scratch = d_msc;
-    e.member_status = reinterpret_cast<int*>(d_mstatus);
+    e.member_status = d_mstatus;
     e.member_out = d_mo;
     e.n_out_members = std::max(1, n_m);
     e.spec = *spec;
     e.stats = stats ? d_stats : nullptr;
     e.prob = (prob && np_planes) ? d_prob : nullptr;
-    rc = run_ensemble(&e, st, b->record_step);
-    if (rc != RS_OK) return rc;
+    {
+      const int rc = run_ensemble(&e, st, b->record_step);
+      if (rc != RS_OK) return rc;
+    }
     CU(cudaEventRecord(ev[2], st));
     if (b->out && pre1 > pre0)
       CU(cudaMemcpy2DAsync(b->out + col, D * np, d_out, D * ld, D * n, static_cast<size_t>(RS_O_NVAR) * (pre1 - pre0),
@@ -2688,13 +2667,7 @@ int roadsurf_run_ensemble_host_soa(const RsHostBatch* b, const double* member_re
                               (member_out ? nm * RS_O_NVAR * n_m : 0)) + (member_status ? sizeof(int) * nm : 0);
     CU(cudaEventRecord(ev[3], st));
     CU(cudaStreamSynchronize(st));
-    float ms = 0.f;
-    cudaEventElapsedTime(&ms, ev[0], ev[1]);
-    g_stats.h2d_ms += ms;
-    cudaEventElapsedTime(&ms, ev[1], ev[2]);
-    g_stats.kernel_ms += ms;
-    cudaEventElapsedTime(&ms, ev[2], ev[3]);
-    g_stats.d2h_ms += ms;
+    add_stage_times(g_stats, ev);
     ++g_stats.groups;
   }
   unsigned long long cnt[RS_CNT_N];
