@@ -31,11 +31,11 @@ def needs_build():
     return any(os.path.getmtime(d) > t for d in deps)
 
 
-def build_library(force=False, verbose=False, extra_flags=()):
+def build_library(force=False, verbose=False):
     """Compile every CUDA source of the package into roadsurf_b200/libroadsurf_b200.so."""
     if not force and not needs_build():
         return LIB
-    cmd = [nvcc_path()] + NVCC_FLAGS + list(extra_flags) + os.environ.get("ROADSURF_B200_NVCC_EXTRA", "").split()
+    cmd = [nvcc_path()] + NVCC_FLAGS + os.environ.get("ROADSURF_B200_NVCC_EXTRA", "").split()
     if verbose:
         cmd += ["-Xptxas", "-v"]
     cmd += ["-o", LIB] + [os.path.join(CSRC, s) for s in SOURCES]

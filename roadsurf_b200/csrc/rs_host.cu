@@ -120,9 +120,9 @@ int launch_model(const RsArgs& a, const RsArgsCold& ac, const RsModel& m, int we
   const int passes = opt_compaction_passes();
   *launches = 0;
   auto run = [&](const RsArgs& ak, const RsArgsCold& ck, int staged) {
-    return static_cast<cudaError_t>(rs_launch_run(&ak, &ck, m.nlayers, staged, m.use_coupling, m.use_relaxation,
-                                                  m.depth_mode != 0, stream, &li->grid, &li->block,
-                                                  &li->regs_per_thread, &li->smem_bytes));
+    return static_cast<cudaError_t>(rs_launch_run(&ak, &ck, m.nlayers, staged, m.use_coupling, m.depth_mode != 0,
+                                                  stream, &li->grid, &li->block, &li->regs_per_thread,
+                                                  &li->smem_bytes));
   };
   if (!(m.use_coupling && wend > 0 && passes > 0 && ac.state && a.scratch && !(opt_staging() && a.forcing_mode == 0) &&
         a.forcing_step0 == 1 && a.step_begin <= 1 && wend + 1 < a.step_end))

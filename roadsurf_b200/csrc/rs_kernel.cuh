@@ -95,8 +95,8 @@ int rs_launch_partition(const double* flags_plane, int ld, int npoints, int sort
 // the kernel variant compiled with exactly the features the run needs.
 void rs_set_spread_small(int on);      // one point per warp for batches of at most 4 points per SM (default on)
 void rs_set_latency_body(int mode);  // -1 auto (small grids), 0 never, 1 every 128-thread launch
-int rs_launch_run(const RsArgs* a, const RsArgsCold* cold, int nlayers, int staged, int coupling, int relaxation, int depth,
-                  void* stream, int* grid, int* block, int* regs, int* smem);
+int rs_launch_run(const RsArgs* a, const RsArgsCold* cold, int nlayers, int staged, int coupling, int depth, void* stream,
+                  int* grid, int* block, int* regs, int* smem);
 int rs_launch_transpose_to_soa(const double* src, long long src_ld, int npoints, int n, double* dst,
                                int ld, void* stream);
 int rs_launch_transpose_from_soa(const double* src, int ld, int npoints, int n, double* dst,
