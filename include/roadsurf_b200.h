@@ -297,8 +297,12 @@ typedef struct RsDeviceBatch
   int n_records;        /* forcing_mode 0: == sim_len.  1: number of coarse records */
   int nvar;             /* RS_F_NVAR or RS_F_NVAR_DEPTH */
   const double* forcing;      /* [n_records][nvar][ld] */
-  const int* record_step;     /* forcing_mode 1: 0-based model step index of every record
-                                 (strictly increasing, record_step[0] <= 0); else NULL */
+  const int* record_step;     /* forcing_mode 1 / 2: 0-based model step index of every record,
+                                 strictly increasing; forcing_mode 1 also needs record_step[0] <= 0
+                                 (example1's rule is implemented for grids that start at or before
+                                 step 0).  A precondition here: this is device memory and the
+                                 asynchronous entry does not read it back to check it.  The host
+                                 entries check their copy (RS_ERR_BAD_ARGUMENT); else NULL */
   const int* time_fields;     /* [6][sim_len]: year, month, day, hour, minute, second */
   const double* local;        /* [RS_L_NLOCAL][ld] */
   const double* horizons;     /* [360][ld] local horizon angles, or NULL (all zero) */
@@ -396,7 +400,8 @@ typedef struct RsHostBatch
   int nvar;                   /* RS_F_NVAR or RS_F_NVAR_DEPTH */
   int out_stride;
   const double* forcing;      /* [n_records][nvar][npoints] */
-  const int* record_step;     /* [n_records] (forcing_mode 1) */
+  const int* record_step;     /* [n_records] (forcing_mode 1): strictly increasing, record_step[0] <= 0;
+                                 RS_ERR_BAD_ARGUMENT otherwise, before any device work */
   const int* time_fields;     /* [6][sim_len] */
   const double* local;        /* [RS_L_NLOCAL][npoints] */
   const double* horizons;     /* [360][npoints] or NULL */
@@ -434,7 +439,8 @@ void roadsurf_release_statics(void* handle);
  * `local` [RS_L_NLOCAL][npoints]; lat / lon / sky view are the caller's.  TSurfObs records are NOT
  * modified: the kernel blanks the coupling window itself.  *window_end (may be NULL) receives the
  * common couplingIndexI of the coupled points, or 0 if they differ or there are none (the value to
- * put into coupling_window_end).  Pure host code. */
+ * put into coupling_window_end).  A record grid that is not strictly increasing or starts after step 0
+ * is RS_ERR_BAD_ARGUMENT.  Pure host code. */
 int roadsurf_read_input_derive_records(const RsHostBatch* batch, const InputSettings* settings, int forecast_step,
                                        const int* latest_obs_index, double* local, int* window_end);
 
@@ -738,7 +744,8 @@ typedef struct RsEnsembleBatch
  * launch of the step kernel, (4) the statistics (when stats or prob is given) and, when prob is given and
  * spec.n_events > 0, the event probabilities.  shared.counters, if
  * given, accumulate both launches.  forcing_mode 1 reads record_step back once (a small synchronous
- * copy on `stream`) to check F against the record grid.  Returns RS_OK or an error code. */
+ * copy on `stream`) to check the record grid (strictly increasing, record_step[0] <= 0) and F against
+ * it.  Returns RS_OK or an error code. */
 int roadsurf_run_ensemble_device(const RsEnsembleBatch* batch, void* stream);
 
 /* The statistics kernel on its own, over any station-major member tensor member_out

@@ -1182,6 +1182,19 @@ int run_sharded(int npoints, int ngpus, const std::function<int(Shard&)>& fn)
     if (sh.rc != RS_OK) return fail(sh.rc, sh.err);
   return RS_OK;
 }
+// The record grid example1's rule is implemented for (forcing_mode 1): record_step strictly increasing, the
+// first record at or before step 0.  The kernel and record_value_at extrapolate the first interval back to
+// step 0 where JsonSource leaves the steps before its first record missing, and equal record steps divide
+// by a zero span.  Host entries call this before any device work; roadsurf_run_device, whose record_step
+// is device memory, keeps it as a precondition.
+int check_record_grid(const int* rs, int nrec)
+{
+  if (rs[0] > 0) return fail(RS_ERR_BAD_ARGUMENT, "record_step[0] must be <= 0 (the first record at or before step 0)");
+  for (int k = 1; k < nrec; ++k)
+    if (rs[k] <= rs[k - 1]) return fail(RS_ERR_BAD_ARGUMENT, "record_step must be strictly increasing");
+  return RS_OK;
+}
+
 // The value JsonSource's interpolation gives at vector index t (the kernel's fetch_coarse rule) from coarse
 // records at record_step rs[0 .. nrec): rec(k) is record k's value of the variable.  Used by
 // roadsurf_read_input_derive_records and, on each member's records, by roadsurf_run_ensemble_host_soa.
@@ -1215,6 +1228,11 @@ int roadsurf_run_host_soa(const RsHostBatch* b, const InputSettings* settings, c
                                     "the device entry: roadsurf_run_device / roadsurf_expand_records)");
   if (b->forcing_mode == 0 ? b->n_records != b->sim_len : (b->n_records < 2 || !b->record_step))
     return fail(RS_ERR_BAD_ARGUMENT, "bad n_records / record_step for the forcing mode");
+  if (b->forcing_mode == 1)
+  {
+    const int rc = check_record_grid(b->record_step, b->n_records);
+    if (rc != RS_OK) return rc;
+  }
   if (b->npoints > 0 && (!b->forcing || !b->time_fields || !b->local || !b->out))
     return fail(RS_ERR_BAD_ARGUMENT, "null host pointer in batch");
   if (b->npoints == 0) return roadsurf_device_count() < 1 ? fail(RS_ERR_NO_DEVICE, "no CUDA device visible") : RS_OK;
@@ -1944,6 +1962,10 @@ int roadsurf_read_input_derive_records(const RsHostBatch* b, const InputSettings
   if (!b || !settings || !local || !b->forcing || !b->record_step || b->forcing_mode != 1 || b->n_records < 2 ||
       b->npoints < 0 || (b->nvar != RS_F_NVAR && b->nvar != RS_F_NVAR_DEPTH))
     return fail(RS_ERR_BAD_ARGUMENT, "needs a coarse-record host batch");
+  {
+    const int rc = check_record_grid(b->record_step, b->n_records);
+    if (rc != RS_OK) return rc;
+  }
   const int sim_len = settings->SimLen, nrec = b->n_records;
   const size_t np = static_cast<size_t>(b->npoints), nvar = static_cast<size_t>(b->nvar);
   const double DT = settings->DTSecs;
@@ -2360,7 +2382,8 @@ int run_ensemble(const RsEnsembleBatch* e, void* stream, const int* host_record_
       CU(cudaStreamSynchronize(st));
       host_record_step = rs.data();
     }
-    const int rc = check_fork(1, s.sim_len, F, M, host_record_step, s.n_records, &r_f);
+    int rc = check_record_grid(host_record_step, s.n_records);
+    if (rc == RS_OK) rc = check_fork(1, s.sim_len, F, M, host_record_step, s.n_records, &r_f);
     if (rc != RS_OK) return rc;
   }
   const bool relax = m.use_relaxation != 0;
@@ -2469,7 +2492,8 @@ int roadsurf_run_ensemble_host_soa(const RsHostBatch* b, const double* member_re
   const int P = b->npoints, M = members, F = fork_step, nvar = b->nvar, nrec = b->n_records;
   int r_f = -1;
   {
-    const int rc = check_fork(1, b->sim_len, F, M, b->record_step, nrec, &r_f);
+    int rc = check_record_grid(b->record_step, nrec);
+    if (rc == RS_OK) rc = check_fork(1, b->sim_len, F, M, b->record_step, nrec, &r_f);
     if (rc != RS_OK) return rc;
   }
   {

@@ -191,3 +191,45 @@ def test_every_run_time_option_is_documented_in_the_header():
     import pytest
     with pytest.raises(Exception):
         lib.set_option("no_such_option", 1)
+
+
+def test_record_grids_are_checked_before_any_device_work():
+    """forcing_mode 1 needs record_step strictly increasing with record_step[0] <= 0: the kernel and the host
+    derivation extrapolate the first interval back to step 0 where example1's JsonSource leaves those steps
+    missing, and two equal steps divide by a zero span.  Every entry that holds record_step in host memory
+    rejects another grid with RS_ERR_BAD_ARGUMENT before it looks for a device (these run on the CPU box)."""
+    import ctypes as C
+    import numpy as np
+    import pytest
+    from roadsurf_b200 import synth
+    arrays, settings, params, rec = synth.make_case(3, 2, seed=1)
+    nrec, sim_len = rec.nrec, arrays.sim_len
+    forcing = np.zeros((nrec, 11, 3))
+    local = np.zeros((lib.L_NLOCAL, 3))
+    out = np.zeros((lib.O_NVAR, sim_len, 3))
+    good = rec.record_step.astype(np.int32)
+    bad_grids = {
+        "after step 0": good + 1,
+        "repeated step": np.where(np.arange(nrec) == 2, good[1], good).astype(np.int32),
+        "decreasing": good[::-1].copy(),
+        "two records, equal": np.array([0, 0], dtype=np.int32),
+    }
+    handle = lib.load()
+    for name, rs in bad_grids.items():
+        n = len(rs)
+        f = np.ascontiguousarray(forcing[:n])
+        hb = lib.RsHostBatch(npoints=3, sim_len=sim_len, forcing_mode=1, n_records=n, nvar=11, out_stride=1,
+                             forcing=f.ctypes.data, record_step=rs.ctypes.data, time_fields=arrays.time.ctypes.data,
+                             local=local.ctypes.data, out=out.ctypes.data)
+        assert handle.roadsurf_run_host_soa(C.byref(hb), C.byref(settings), C.byref(params), 1) == -2, name
+        assert b"record_step" in handle.roadsurf_last_error(), name
+        with pytest.raises(lib.RoadSurfError, match="record_step"):
+            lib.read_input_derive_records(f, rs, settings, 0, local)
+        if n > 2:
+            members = np.zeros((n - 2, 11, 3 * 2))
+            with pytest.raises(lib.RoadSurfError, match="record_step"):
+                lib.run_ensemble_host_soa(settings, params, f, rs, arrays.time, local, members, 2, 122, lib.stats_spec())
+    # the grid the entries are built for passes the check (the derivation is pure host code)
+    assert lib.read_input_derive_records(np.ascontiguousarray(forcing), good, settings, 0, local) == 0
+    for first in (0, -1, -500):
+        lib.read_input_derive_records(np.ascontiguousarray(forcing), (good + first).astype(np.int32), settings, 0, local)

@@ -8,7 +8,7 @@ import numpy as np
 import pytest
 
 from roadsurf_b200 import example1
-from test_host_logic import _interpolate_like_json_source
+from record_refs import interpolate_like_json_source
 
 
 def _oracle_runner(oracle):
@@ -35,7 +35,7 @@ def test_interpolation_general_time_grids():
     for start, n in ((0, 400), (-900, 300), (1800, 350)):
         simtime = [start + 30 * i for i in range(n)]
         got = example1.interpolate(rawtime, raw, simtime)
-        want = _interpolate_like_json_source(raw, rawtime, simtime)
+        want = interpolate_like_json_source(raw, rawtime, simtime)
         assert np.array_equal(got, want), start
     ph = example1.interpolate(rawtime, np.array([1, 2, 3, -9999, 1.0]), [0, 30, 3600, 3630, 5400, 5430], next_record=True)
     assert list(ph) == [1, 2, 2, 3, 3, -9999]
