@@ -163,6 +163,82 @@ int launch_model(const RsArgs& a, const RsArgsCold& ac, const RsModel& m, int we
   return RS_OK;
 }
 
+// The batch with its documented defaults filled in: step_begin 0 -> 1, step_end 0 -> sim_len, forcing_step0 0 -> 1,
+// and out_nvar RS_O_NVAR unless it is RS_O_NVAR_EXT.
+RsDeviceBatch with_defaults(RsDeviceBatch b)
+{
+  if (b.step_begin <= 0) b.step_begin = 1;
+  if (b.step_end <= 0) b.step_end = b.sim_len;
+  if (b.forcing_step0 <= 0) b.forcing_step0 = 1;
+  if (b.out_nvar != RS_O_NVAR_EXT) b.out_nvar = RS_O_NVAR;
+  return b;
+}
+
+// A checked batch as step-kernel launches on `stream`: the one place the kernel's arguments are built.  forcing_mode
+// 2 runs an expansion pass and a full-resolution model run per chunk of expand_steps; the other modes are one model
+// run, with lane compaction when b.coupling_window_end is set.  b.solar must already hold the solar table.
+// *launches receives the number of kernels queued.
+int launch_batch(const RsDeviceBatch& batch, const RsModel& m, cudaStream_t stream, RsLaunchInfo* li, int* launches)
+{
+  const RsDeviceBatch b = with_defaults(batch);
+  RsArgs a;
+  std::memset(&a, 0, sizeof a);
+  a.npoints = b.npoints;
+  a.ld = b.ld;
+  a.sim_len = b.sim_len;
+  a.n_records = b.n_records;
+  a.nvar = b.nvar;
+  a.out_stride = b.out_stride;
+  a.n_out = b.n_out;
+  a.forcing_mode = b.forcing_mode;
+  a.step_begin = b.step_begin;
+  a.step_end = b.step_end;
+  a.forcing_step0 = b.forcing_step0;
+  a.out_slot0 = b.out_slot0;
+  a.forcing = b.forcing;
+  a.record_step = b.record_step;
+  a.tf = b.time_fields;
+  a.local = b.local;
+  a.horizons = b.horizons;
+  a.solar = b.solar;
+  a.out = b.out;
+  a.status = b.status;
+  a.scratch = b.scratch;
+  RsArgsCold ac;
+  std::memset(&ac, 0, sizeof ac);
+  ac.state = b.state;
+  ac.counters = b.counters;
+  ac.out_start = b.out_start;
+  ac.out_nvar = b.out_nvar;
+  if (b.order && !(opt_staging() && b.forcing_mode == 0))  // (the staged ring needs consecutive points per warp)
+  {
+    ac.index = b.order;  // thread t runs point order[t]
+    ac.n_fixed = b.ld;
+  }
+  li->nlayers = m.nlayers;
+  li->forcing_mode = b.forcing_mode;
+  *launches = 0;
+  if (b.forcing_mode != 2) return launch_model(a, ac, m, b.coupling_window_end, stream, li, launches);
+  for (int cb = b.step_begin; cb <= b.step_end; cb += b.expand_steps)
+  {
+    const int ce = std::min(b.step_end, cb + b.expand_steps - 1);
+    CU(static_cast<cudaError_t>(rs_launch_expand(b.forcing, b.record_step, b.n_records, b.nvar, b.ld, b.npoints, 2,
+                                                 m.DT, cb, ce, b.expand_workspace, stream)));
+    RsArgs ak = a;
+    ak.forcing_mode = 0;
+    ak.forcing = b.expand_workspace;
+    ak.n_records = ce - cb + 1;
+    ak.forcing_step0 = cb;
+    ak.step_begin = cb;
+    ak.step_end = ce;
+    int n = 0;
+    const int rc = launch_model(ak, ac, m, 0, stream, li, &n);
+    if (rc != RS_OK) return rc;
+    *launches += 1 + n;
+  }
+  return RS_OK;
+}
+
 double now_ms()
 {
   using namespace std::chrono;
@@ -719,43 +795,32 @@ int run_shard(Shard& sh, OutputPointers* const* out, const InputPointers* const*
       CU(cudaEventRecord(c.ev[1], st));
 
       // ---- the step kernel(s), queued behind the input stage
-      RsArgs a;
-      std::memset(&a, 0, sizeof a);
-      a.npoints = ld;
-      a.ld = ld;
-      a.sim_len = sim_len;
-      a.n_records = sim_len;
-      a.nvar = nvar;
-      a.out_stride = 1;
-      a.n_out = sim_len;
-      a.forcing_mode = 0;
-      a.step_begin = 1;
-      a.step_end = sim_len;
-      a.forcing_step0 = 1;
-      a.out_slot0 = 0;
-      a.forcing = c.d_forcing;
-      a.tf = d_tf;
-      a.local = c.d_local;
-      a.horizons = any_sky ? c.d_hor : nullptr;
-      a.solar = d_solar;
-      a.out = c.d_out;
-      a.status = c.d_status;
-      a.scratch = model.use_coupling ? c.d_scratch : nullptr;
-      RsArgsCold ac;
-      std::memset(&ac, 0, sizeof ac);
-      ac.counters = c.d_counters;
-      ac.out_start = 0;
-      ac.out_nvar = RS_O_NVAR;
-      ac.state = wend > 0 ? c.d_state : nullptr;
+      RsDeviceBatch db{};
+      db.npoints = ld;
+      db.ld = ld;
+      db.sim_len = sim_len;
+      db.n_records = sim_len;
+      db.nvar = nvar;
+      db.forcing = c.d_forcing;
+      db.time_fields = d_tf;
+      db.local = c.d_local;
+      db.horizons = any_sky ? c.d_hor : nullptr;
+      db.out = c.d_out;
+      db.out_stride = 1;
+      db.n_out = sim_len;
+      db.status = c.d_status;
+      db.state = wend > 0 ? c.d_state : nullptr;
+      db.scratch = model.use_coupling ? c.d_scratch : nullptr;
+      db.counters = c.d_counters;
+      db.solar = d_solar;
+      db.coupling_window_end = wend;
       {
         int n = 0;
-        const int rc = launch_model(a, ac, model, wend, st, &sh.launch, &n);
+        const int rc = launch_batch(db, model, st, &sh.launch, &n);
         if (rc != RS_OK) return rc;
         sh.stats.kernel_launches += n;
       }
       CU(cudaEventRecord(c.ev[2], st));
-      sh.launch.nlayers = nl;
-      sh.launch.forcing_mode = 0;
       return RS_OK;
     };
 
@@ -1065,56 +1130,42 @@ int run_host_soa_shard(Shard& sh, const RsHostBatch* b, const InputSettings* set
                            cudaMemcpyHostToDevice, st));
     sh.stats.h2d_bytes += wbytes * (frows + RS_L_NLOCAL + ((hor && !resident) ? 360 : 0));
     CU(cudaEventRecord(ev[s][1], st));
-    RsArgs a;
-    std::memset(&a, 0, sizeof a);
-    a.npoints = npc;
-    a.ld = ld;
-    a.sim_len = b->sim_len;
-    a.n_records = b->n_records;
-    a.nvar = b->nvar;
-    a.out_stride = b->out_stride;
-    a.n_out = n_out;
-    a.forcing_mode = b->forcing_mode;
-    a.step_begin = 1;
-    a.step_end = b->sim_len;
-    a.forcing_step0 = 1;
-    a.out_slot0 = 0;
-    a.forcing = d_forcing[s];
-    a.record_step = d_rs;
-    a.tf = d_tf;
-    a.local = d_local[s];
-    a.horizons = resident ? resident->chunks[c].hor : d_hor[s];
-    a.solar = d_solar;
-    a.out = d_out[s];
-    a.status = d_status[s];
-    a.scratch = d_scratch[s];
-    RsArgsCold ac;
-    std::memset(&ac, 0, sizeof ac);
-    ac.counters = d_counters;
-    ac.out_start = 0;
-    ac.out_nvar = RS_O_NVAR;
-    ac.state = d_state[s];
+    RsDeviceBatch db{};
+    db.npoints = npc;
+    db.ld = ld;
+    db.sim_len = b->sim_len;
+    db.forcing_mode = b->forcing_mode;
+    db.n_records = b->n_records;
+    db.nvar = b->nvar;
+    db.forcing = d_forcing[s];
+    db.record_step = d_rs;
+    db.time_fields = d_tf;
+    db.local = d_local[s];
+    db.horizons = resident ? resident->chunks[c].hor : d_hor[s];
+    db.out = d_out[s];
+    db.out_stride = b->out_stride;
+    db.n_out = n_out;
+    db.status = d_status[s];
+    db.state = d_state[s];
+    db.scratch = d_scratch[s];
+    db.counters = d_counters;
+    db.solar = d_solar;
+    db.coupling_window_end = wend;
     if (resident && b->forcing_mode == 1 && resident->chunks[c].order)
-    {
-      ac.index = resident->chunks[c].order;  // built once by roadsurf_prepare_statics
-      ac.n_fixed = ld;
-    }
+      db.order = resident->chunks[c].order;  // built once by roadsurf_prepare_statics
     else if (d_order[s])
     {
       CU(static_cast<cudaError_t>(rs_launch_partition(d_local[s] + static_cast<size_t>(RS_L_SKY_VIEW) * ld, ld, npc, 2,
                                                       d_order[s], nullptr, st)));
       ++sh.stats.kernel_launches;
-      ac.index = d_order[s];
-      ac.n_fixed = ld;
+      db.order = d_order[s];
     }
     {
       int n = 0;
-      const int rc = launch_model(a, ac, model, wend, st, &sh.launch, &n);
+      const int rc = launch_batch(db, model, st, &sh.launch, &n);
       if (rc != RS_OK) return rc;
       sh.stats.kernel_launches += n;
     }
-    sh.launch.nlayers = nl;
-    sh.launch.forcing_mode = b->forcing_mode;
     CU(cudaEventRecord(ev[s][2], st));
     CU(cudaMemcpy2DAsync(b->out + col0, sizeof(double) * np_all, d_out[s], sizeof(double) * ld, wbytes, orows,
                          cudaMemcpyDeviceToHost, st));
@@ -1326,12 +1377,9 @@ namespace
 struct RsSession
 {
   unsigned magic = 0x52535345u;  // "RSSE"
-  int device = 0, npoints = 0, ld = 0, sim_len = 0, nl = 0, nvar = 0;
+  int device = 0;
   RsModel model;
-  double *d_forcing = nullptr, *d_local = nullptr, *d_hor = nullptr, *d_out = nullptr, *d_state = nullptr,
-         *d_scratch = nullptr, *d_solar = nullptr;
-  int *d_tf = nullptr, *d_status = nullptr;
-  unsigned long long* d_counters = nullptr;
+  RsDeviceBatch batch{};  // device buffers this session owns; roadsurf_step sets step_begin / step_end
   cudaStream_t stream = nullptr;
   std::vector<OutputPointers> outs;
   int done = 0, fetched = 0, chunk = 1;
@@ -1361,11 +1409,14 @@ int roadsurf_session_open(int npoints, OutputPointers* const* out, const InputPo
     if (rc != RS_OK) return rc;
   }
   const int sim_len = settings->SimLen, nl = s->model.nlayers;
-  s->npoints = npoints;
-  s->ld = (npoints + 31) / 32 * 32;
-  s->sim_len = sim_len;
-  s->nl = nl;
-  const size_t ld = s->ld;
+  RsDeviceBatch& b = s->batch;
+  b.npoints = npoints;
+  b.ld = (npoints + 31) / 32 * 32;
+  b.sim_len = sim_len;
+  b.n_records = sim_len;
+  b.out_stride = 1;
+  b.n_out = sim_len;
+  const size_t ld = b.ld;
   bool any_depth = false, any_sky = false;
   for (int p = 0; p < npoints; ++p)
   {
@@ -1388,7 +1439,7 @@ int roadsurf_session_open(int npoints, OutputPointers* const* out, const InputPo
       s->wstart = cstart;
     }
   }
-  const int nvar = s->nvar = any_depth ? RS_F_NVAR_DEPTH : RS_F_NVAR;
+  const int nvar = b.nvar = any_depth ? RS_F_NVAR_DEPTH : RS_F_NVAR;
   // ---- pack on the host: forcing [t][var][ld], statics, horizons; pre-fill the caller's outputs
   std::vector<double> hf(static_cast<size_t>(sim_len) * nvar * ld, 0.0), hl(RS_L_NLOCAL * ld, 0.0);
   std::vector<double> hh(any_sky ? 360 * ld : 0, 0.0);
@@ -1404,27 +1455,32 @@ int roadsurf_session_open(int npoints, OutputPointers* const* out, const InputPo
     for (double* o : output_planes(*out[p])) std::fill(o, o + sim_len, -9999.0);
   }
   CU(cudaStreamCreateWithFlags(&s->stream, cudaStreamNonBlocking));
-  CU(cudaMalloc(&s->d_forcing, sizeof(double) * hf.size()));
-  CU(cudaMalloc(&s->d_local, sizeof(double) * hl.size()));
-  if (any_sky) CU(cudaMalloc(&s->d_hor, sizeof(double) * hh.size()));
-  CU(cudaMalloc(&s->d_out, sizeof(double) * RS_O_NVAR * sim_len * ld));
-  CU(cudaMalloc(&s->d_state, sizeof(double) * RS_STATE_NPLANES(nl) * ld));
-  CU(cudaMalloc(&s->d_scratch, sizeof(double) * RS_SCRATCH_NPLANES(nl) * ld));
-  CU(cudaMalloc(&s->d_solar, sizeof(double) * 4 * sim_len));
-  CU(cudaMalloc(&s->d_tf, sizeof(int) * 6 * sim_len));
-  CU(cudaMalloc(&s->d_status, sizeof(int) * ld));
-  CU(cudaMalloc(&s->d_counters, sizeof(unsigned long long) * RS_CNT_N));
-  CU(cudaMemcpyAsync(s->d_forcing, hf.data(), sizeof(double) * hf.size(), cudaMemcpyHostToDevice, s->stream));
-  CU(cudaMemcpyAsync(s->d_local, hl.data(), sizeof(double) * hl.size(), cudaMemcpyHostToDevice, s->stream));
-  if (any_sky) CU(cudaMemcpyAsync(s->d_hor, hh.data(), sizeof(double) * hh.size(), cudaMemcpyHostToDevice, s->stream));
+  // (the batch declares the inputs const: the session fills the buffers it owns through const_cast)
+  CU(cudaMalloc(&b.forcing, sizeof(double) * hf.size()));
+  CU(cudaMalloc(&b.local, sizeof(double) * hl.size()));
+  if (any_sky) CU(cudaMalloc(&b.horizons, sizeof(double) * hh.size()));
+  CU(cudaMalloc(&b.out, sizeof(double) * RS_O_NVAR * sim_len * ld));
+  CU(cudaMalloc(&b.state, sizeof(double) * RS_STATE_NPLANES(nl) * ld));
+  CU(cudaMalloc(&b.scratch, sizeof(double) * RS_SCRATCH_NPLANES(nl) * ld));
+  CU(cudaMalloc(&b.solar, sizeof(double) * 4 * sim_len));
+  CU(cudaMalloc(&b.time_fields, sizeof(int) * 6 * sim_len));
+  CU(cudaMalloc(&b.status, sizeof(int) * ld));
+  CU(cudaMalloc(&b.counters, sizeof(unsigned long long) * RS_CNT_N));
+  CU(cudaMemcpyAsync(const_cast<double*>(b.forcing), hf.data(), sizeof(double) * hf.size(), cudaMemcpyHostToDevice,
+                     s->stream));
+  CU(cudaMemcpyAsync(const_cast<double*>(b.local), hl.data(), sizeof(double) * hl.size(), cudaMemcpyHostToDevice,
+                     s->stream));
+  if (any_sky)
+    CU(cudaMemcpyAsync(const_cast<double*>(b.horizons), hh.data(), sizeof(double) * hh.size(), cudaMemcpyHostToDevice,
+                       s->stream));
   const auto tf = time_fields(*in[0]);
   for (int k = 0; k < 6; ++k)
-    CU(cudaMemcpyAsync(s->d_tf + static_cast<size_t>(k) * sim_len, tf[k], sizeof(int) * sim_len, cudaMemcpyHostToDevice,
-                       s->stream));
-  CU(cudaMemsetAsync(s->d_status, 0, sizeof(int) * ld, s->stream));
-  CU(cudaMemsetAsync(s->d_counters, 0, sizeof(unsigned long long) * RS_CNT_N, s->stream));
-  CU(static_cast<cudaError_t>(rs_launch_fill(s->d_out, static_cast<long long>(RS_O_NVAR) * sim_len * ld, -9999.0, s->stream)));
-  CU(static_cast<cudaError_t>(rs_launch_solar(s->d_tf, sim_len, s->d_solar, s->stream)));
+    CU(cudaMemcpyAsync(const_cast<int*>(b.time_fields) + static_cast<size_t>(k) * sim_len, tf[k], sizeof(int) * sim_len,
+                       cudaMemcpyHostToDevice, s->stream));
+  CU(cudaMemsetAsync(b.status, 0, sizeof(int) * ld, s->stream));
+  CU(cudaMemsetAsync(b.counters, 0, sizeof(unsigned long long) * RS_CNT_N, s->stream));
+  CU(static_cast<cudaError_t>(rs_launch_fill(b.out, static_cast<long long>(RS_O_NVAR) * sim_len * ld, -9999.0, s->stream)));
+  CU(static_cast<cudaError_t>(rs_launch_solar(b.time_fields, sim_len, b.solar, s->stream)));
   g_launches_total += 2;
   CU(cudaStreamSynchronize(s->stream));  // the host staging vectors die with this frame
   *session = guard.release();
@@ -1449,15 +1505,16 @@ int roadsurf_step(void* session, int i)
 {
   RsSession* s = session_of(session);
   if (!s) return fail(RS_ERR_BAD_ARGUMENT, "not a session");
-  if (i < 1 || i > s->sim_len) return fail(RS_ERR_BAD_ARGUMENT, "step outside [1, SimLen]");
+  const int sim_len = s->batch.sim_len;
+  if (i < 1 || i > sim_len) return fail(RS_ERR_BAD_ARGUMENT, "step outside [1, SimLen]");
   if (i <= s->done) return RS_OK;
   int current = 0;
   CU(cudaGetDevice(&current));
   if (current != s->device) CU(cudaSetDevice(s->device));
   const int begin = s->done + 1;
-  int target = std::min(s->sim_len, std::max(i, s->done + s->chunk));
+  int target = std::min(sim_len, std::max(i, s->done + s->chunk));
   // a coupling window [start, end + 1] is indivisible: its rewinds happen inside the kernel
-  if (s->wend > 0 && begin <= s->wend + 1 && target >= s->wstart) target = std::max(target, std::min(s->wend + 1, s->sim_len));
+  if (s->wend > 0 && begin <= s->wend + 1 && target >= s->wstart) target = std::max(target, std::min(s->wend + 1, sim_len));
   {
     std::lock_guard<std::mutex> device_lock(g_device_mu[s->device & 63]);
     // (another caller may have replaced the device's model since the session was opened)
@@ -1465,39 +1522,14 @@ int roadsurf_step(void* session, int i)
       const int rc = upload_model(s->device, s->model);
       if (rc != RS_OK) return rc;
     }
-    RsArgs a;
-    std::memset(&a, 0, sizeof a);
-    a.npoints = s->npoints;
-    a.ld = s->ld;
-    a.sim_len = s->sim_len;
-    a.n_records = s->sim_len;
-    a.nvar = s->nvar;
-    a.out_stride = 1;
-    a.n_out = s->sim_len;
-    a.forcing_mode = 0;
-    a.step_begin = begin;
-    a.step_end = target;
-    a.forcing_step0 = 1;
-    a.forcing = s->d_forcing;
-    a.tf = s->d_tf;
-    a.local = s->d_local;
-    a.horizons = s->d_hor;
-    a.solar = s->d_solar;
-    a.out = s->d_out;
-    a.status = s->d_status;
-    a.scratch = s->d_scratch;
-    RsArgsCold ac;
-    std::memset(&ac, 0, sizeof ac);
-    ac.state = s->d_state;
-    ac.counters = s->d_counters;
-    ac.out_nvar = RS_O_NVAR;
+    s->batch.step_begin = begin;
+    s->batch.step_end = target;
     RsLaunchInfo li;
     std::memset(&li, 0, sizeof li);
     int n = 0;
-    const int rc = launch_model(a, ac, s->model, 0, s->stream, &li, &n);
+    const int rc = launch_batch(s->batch, s->model, s->stream, &li, &n);
     if (rc != RS_OK) return rc;
     g_launches_total += n;
-    li.nlayers = s->nl;
     li.launches_total = g_launches_total;
     g_launch = li;
     CU(cudaStreamSynchronize(s->stream));
@@ -1517,23 +1549,24 @@ int roadsurf_session_fetch(void* session, int i, int* status)
   if (current != s->device) CU(cudaSetDevice(s->device));
   // deliver every executed step not yet delivered; the steps of a coupling window were overwritten by the
   // kernel's re-runs before they became visible here
+  const RsDeviceBatch& b = s->batch;
   const int t0 = s->fetched, n = s->done - s->fetched;
   if (n > 0)
   {
-    std::vector<double> h(static_cast<size_t>(RS_O_NVAR) * n * s->ld);
+    std::vector<double> h(static_cast<size_t>(RS_O_NVAR) * n * b.ld);
     for (int v = 0; v < RS_O_NVAR; ++v)
-      CU(cudaMemcpy(h.data() + static_cast<size_t>(v) * n * s->ld,
-                    s->d_out + (static_cast<size_t>(v) * s->sim_len + t0) * s->ld, sizeof(double) * n * s->ld,
+      CU(cudaMemcpy(h.data() + static_cast<size_t>(v) * n * b.ld,
+                    b.out + (static_cast<size_t>(v) * b.sim_len + t0) * b.ld, sizeof(double) * n * b.ld,
                     cudaMemcpyDeviceToHost));
-    for (int p = 0; p < s->npoints; ++p)
+    for (int p = 0; p < b.npoints; ++p)
     {
       const auto dst = output_planes(s->outs[p]);
       for (int v = 0; v < RS_O_NVAR; ++v)
-        for (int t = 0; t < n; ++t) dst[v][t0 + t] = h[(static_cast<size_t>(v) * n + t) * s->ld + p];
+        for (int t = 0; t < n; ++t) dst[v][t0 + t] = h[(static_cast<size_t>(v) * n + t) * b.ld + p];
     }
     s->fetched = s->done;
   }
-  if (status) CU(cudaMemcpy(status, s->d_status, sizeof(int) * s->npoints, cudaMemcpyDeviceToHost));
+  if (status) CU(cudaMemcpy(status, b.status, sizeof(int) * b.npoints, cudaMemcpyDeviceToHost));
   if (current != s->device) cudaSetDevice(current);
   return RS_OK;
 }
@@ -1545,11 +1578,13 @@ void roadsurf_session_close(void* session)
   int current = 0;
   cudaGetDevice(&current);
   cudaSetDevice(s->device);
-  for (void* p : {static_cast<void*>(s->d_forcing), static_cast<void*>(s->d_local), static_cast<void*>(s->d_hor),
-                  static_cast<void*>(s->d_out), static_cast<void*>(s->d_state), static_cast<void*>(s->d_scratch),
-                  static_cast<void*>(s->d_solar), static_cast<void*>(s->d_tf), static_cast<void*>(s->d_status),
-                  static_cast<void*>(s->d_counters)})
-    if (p) cudaFree(p);
+  const RsDeviceBatch& b = s->batch;
+  for (const void* p : {static_cast<const void*>(b.forcing), static_cast<const void*>(b.local),
+                        static_cast<const void*>(b.horizons), static_cast<const void*>(b.out),
+                        static_cast<const void*>(b.state), static_cast<const void*>(b.scratch),
+                        static_cast<const void*>(b.solar), static_cast<const void*>(b.time_fields),
+                        static_cast<const void*>(b.status), static_cast<const void*>(b.counters)})
+    if (p) cudaFree(const_cast<void*>(p));
   if (s->stream) cudaStreamDestroy(s->stream);
   cudaSetDevice(current);
   s->magic = 0;
@@ -1590,9 +1625,8 @@ int roadsurf_run_device(const RsDeviceBatch* b, void* stream)
   }
   if (b->ld < 32|| b->ld % 32 != 0 || b->npoints < 0 || b->npoints > b->ld)
     return fail(RS_ERR_BAD_ARGUMENT, "ld must be a positive multiple of 32 and >= npoints");
-  const int step_begin = b->step_begin > 0 ? b->step_begin : 1;
-  const int step_end = b->step_end > 0 ? b->step_end : b->sim_len;
-  const int forcing_step0 = b->forcing_step0 > 0 ? b->forcing_step0 : 1;
+  const RsDeviceBatch d = with_defaults(*b);
+  const int step_begin = d.step_begin, step_end = d.step_end, forcing_step0 = d.forcing_step0;
   if (b->sim_len < 1 || b->out_stride < 1 || b->n_out < 1)
     return fail(RS_ERR_BAD_ARGUMENT, "bad sim_len / out_stride / n_out");
   if (step_begin > step_end || step_end > b->sim_len || forcing_step0 > step_begin || b->out_slot0 < 0)
@@ -1629,81 +1663,20 @@ int roadsurf_run_device(const RsDeviceBatch* b, void* stream)
   else
     return fail(RS_ERR_BAD_ARGUMENT, "forcing_mode must be 0, 1 or 2");
   if (m.use_coupling && !b->scratch) return fail(RS_ERR_BAD_ARGUMENT, "coupling needs batch->scratch");
-  RsArgs a;
-  std::memset(&a, 0, sizeof a);
-  a.npoints = b->npoints;
-  a.ld = b->ld;
-  a.sim_len = b->sim_len;
-  a.n_records = b->n_records;
-  a.nvar = b->nvar;
-  a.out_stride = b->out_stride;
-  a.n_out = b->n_out;
-  a.forcing_mode = b->forcing_mode;
-  a.step_begin = step_begin;
-  a.step_end = step_end;
-  a.forcing_step0 = forcing_step0;
-  a.out_slot0 = b->out_slot0;
-  a.forcing = b->forcing;
-  a.record_step = b->record_step;
-  a.tf = b->time_fields;
-  a.local = b->local;
-  a.horizons = b->horizons;
-  a.solar = b->solar;
-  a.out = b->out;
-  a.status = b->status;
-  a.scratch = b->scratch;
-  RsArgsCold ac;
-  std::memset(&ac, 0, sizeof ac);
-  ac.state = b->state;
-  ac.counters = b->counters;
-  ac.out_start = b->out_start;
-  ac.out_nvar = b->out_nvar == RS_O_NVAR_EXT ? RS_O_NVAR_EXT : RS_O_NVAR;
-  if (b->order && !(opt_staging() && b->forcing_mode == 0))  // (the staged ring needs consecutive points per warp)
-  {
-    ac.index = b->order;  // thread t runs point order[t]
-    ac.n_fixed = b->ld;
-  }
+  const cudaStream_t st = static_cast<cudaStream_t>(stream);
+  CU(static_cast<cudaError_t>(rs_launch_solar(b->time_fields, b->sim_len, b->solar, st)));
   RsLaunchInfo li;
   std::memset(&li, 0, sizeof li);
-  CU(static_cast<cudaError_t>(rs_launch_solar(b->time_fields, b->sim_len, b->solar, stream)));
-  ++g_launches_total;
-
-  if (b->forcing_mode == 2)
+  int n = 0;
   {
-    // expansion pass + full-resolution step kernel, chunk by chunk through the resumable path
-    for (int cb = step_begin; cb <= step_end; cb += b->expand_steps)
-    {
-      const int ce = std::min(step_end, cb + b->expand_steps - 1);
-      CU(static_cast<cudaError_t>(rs_launch_expand(b->forcing, b->record_step, b->n_records, b->nvar, b->ld, b->npoints, 2,
-                                                    m.DT, cb, ce, b->expand_workspace, stream)));
-      RsArgs ak = a;
-      ak.forcing_mode = 0;
-      ak.forcing = b->expand_workspace;
-      ak.n_records = ce - cb + 1;
-      ak.forcing_step0 = cb;
-      ak.step_begin = cb;
-      ak.step_end = ce;
-      int n = 0;
-      const int rc = launch_model(ak, ac, m, 0, stream, &li, &n);
-      if (rc != RS_OK) return rc;
-      g_launches_total += n + 1;
-    }
-    --g_launches_total;  // (the last one is counted below)
-  }
-  else
-  {
-    int n = 0;
-    const int rc = launch_model(a, ac, m, b->coupling_window_end, stream, &li, &n);
-    if (rc != RS_OK) return rc;
-    g_launches_total += n - 1;  // (the last one is counted below)
-  }
-  {
-    const int rc = note_async_launch(dev, static_cast<cudaStream_t>(stream));
+    const int rc = launch_batch(d, m, st, &li, &n);
     if (rc != RS_OK) return rc;
   }
-  li.nlayers = m.nlayers;
-  li.forcing_mode = b->forcing_mode;
-  li.launches_total = ++g_launches_total;
+  {
+    const int rc = note_async_launch(dev, st);
+    if (rc != RS_OK) return rc;
+  }
+  li.launches_total = g_launches_total += 1 + n;  // the solar table and the model run
   g_launch = li;
   return RS_OK;
 }

@@ -36,7 +36,7 @@ struct RsArgsCold
   unsigned long long* counters;  // [RS_CNT_N] or null
   int out_start;                 // 0-based step index of output slot 0
   int out_nvar;                  // RS_O_NVAR or RS_O_NVAR_EXT
-  // Lane compaction between coupling passes (see rs_launch_run_coupled): thread t handles point
+  // Lane compaction between coupling passes (see launch_model in rs_host.cu): thread t handles point
   // index[t] for t < *n_index (threads beyond are ghosts that write nothing); null = thread t is point t.
   const int* index;
   const int* n_index;            // device-side list length, or null: n_fixed entries
