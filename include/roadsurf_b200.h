@@ -704,6 +704,27 @@ typedef struct RsEnsembleStatsSpec
   RsEnsembleEvent events[RS_ENS_MAX_EVENTS];
 } RsEnsembleStatsSpec;
 
+/* Areas: groups of stations such as a maintenance route or a district, for the probability that an event of
+ * spec.events occurs anywhere in the group.  An area is a non-empty set of station indices; areas may overlap, and
+ * a station may belong to any number of them.  For area A, event e, member m and member slot s < S (the slots the
+ * station events cover):
+ *   - valid: member m is valid for A at s when it is valid for e at s (RsEnsembleEvent's station rule) at EVERY
+ *     station of A.  A station that did not run (RS_ST_NOT_RUN, all -9999) therefore makes every area that holds it
+ *     invalid for that member: leave such stations out of the areas;
+ *   - hit: the member is valid for A and hits e at s at one station of A or more (each station within its own window
+ *     W(s); different stations may hit at different slots of the window);
+ *   - result: area_prob[e][s][a] = (double)hits / (double)valid, -9999.0 where no member is valid.
+ * So an area of one station equals that station's event plane of `prob` bit for bit, and neither repeated stations
+ * nor their order change an area's result.  The arrays are HOST memory in every entry: the library checks every
+ * index and copies the arrays, and the caller may reuse them when the call returns. */
+typedef struct RsEnsembleAreas
+{
+  int n_areas;         /* >= 1 */
+  const int* offsets;  /* HOST [n_areas + 1]: offsets[0] == 0, strictly increasing (no empty area) */
+  const int* stations; /* HOST [offsets[n_areas]]: area a is stations[offsets[a] .. offsets[a + 1] - 1], each in
+                          [0, npoints) */
+} RsEnsembleAreas;
+
 /* A device-resident ensemble (DEVICE pointers on the current device). */
 typedef struct RsEnsembleBatch
 {
@@ -756,6 +777,19 @@ int roadsurf_ensemble_stats(const double* member_out, int out_nvar, int n_out, i
                             int members, const RsEnsembleStatsSpec* spec, double* stats, double* prob, int ld,
                             void* stream);
 
+/* Area event probabilities (RsEnsembleAreas) over a station-major member tensor member_out
+ * [out_nvar][n_out][ld_members] (lane p * members + m), as for roadsurf_ensemble_stats: area_prob DEVICE
+ * [n_events][n_out][n_areas].  spec->n_events >= 1; quantiles and thresholds are ignored.  The area arrays are
+ * host memory, checked and copied by the library (the caller may reuse them when the call returns); asynchronous on
+ * `stream` otherwise.  After roadsurf_run_ensemble_device, call it on the same stream with the batch's member_out,
+ * n_out = n_out_members (equal to the member slots of the run), ld_members, shared.npoints and members:
+ *   roadsurf_run_ensemble_device(&e, stream);
+ *   roadsurf_ensemble_area_events(e.member_out, e.shared.out_nvar, e.n_out_members, e.ld_members,
+ *                                 e.shared.npoints, e.members, &e.spec, &areas, d_area_prob, stream); */
+int roadsurf_ensemble_area_events(const double* member_out, int out_nvar, int n_out, int ld_members, int npoints,
+                                  int members, const RsEnsembleStatsSpec* spec, const RsEnsembleAreas* areas,
+                                  double* area_prob, void* stream);
+
 /* Host form on the current device, forcing_mode 1 only.  `shared` is the stations' host SoA batch
  * (as for roadsurf_run_host_soa, with the full record axis); its `out`, if not NULL, receives the
  * station outputs of the steps before F, [RS_O_NVAR][n_out_pre][P] with n_out_pre = ceil((F - 1) /
@@ -774,6 +808,19 @@ int roadsurf_run_ensemble_host_soa(const RsHostBatch* shared, const double* memb
                                    int fork_step, const int* latest_obs_index, const RsEnsembleStatsSpec* spec, double* stats, double* prob,
                                    double* member_out, int* member_status, const InputSettings* settings,
                                    const InputParameters* params);
+
+/* roadsurf_run_ensemble_host_soa plus area event probabilities: area_prob HOST [n_events][n_out_m][n_areas].  The
+ * areas are planned once per call and accumulated on the device after each station chunk, so an area may span
+ * chunks; one device-to-host copy of area_prob at the end (counted in d2h_bytes; the two area kernels in kernel_ms).
+ * prob may be NULL with areas given (no station events are computed then).  areas == NULL and area_prob == NULL is
+ * exactly roadsurf_run_ensemble_host_soa; one without the other is RS_ERR_BAD_ARGUMENT.  The area accumulators,
+ * 2 * n_areas * n_events * ceil(n_out_m / 64) * members * 8 bytes, stay on the device for the whole call:
+ * RS_ERR_CUDA where they do not fit. */
+int roadsurf_run_ensemble_host_soa_areas(const RsHostBatch* shared, const double* member_records, int members,
+                                         int fork_step, const int* latest_obs_index, const RsEnsembleStatsSpec* spec,
+                                         double* stats, double* prob, double* member_out, int* member_status,
+                                         const RsEnsembleAreas* areas, double* area_prob,
+                                         const InputSettings* settings, const InputParameters* params);
 
 #ifdef __cplusplus
 }

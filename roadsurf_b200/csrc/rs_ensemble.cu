@@ -1,6 +1,6 @@
 // rs_ensemble.cu -- the kernels of an ensemble run (roadsurf_run_ensemble_device): the prefix's copy of the
-// station statics, the fork of the station state into the member lanes, the ensemble statistics and the event
-// probabilities.
+// station statics, the fork of the station state into the member lanes, the ensemble statistics, the event
+// probabilities and the area event probabilities.
 // Member lanes are station-major: lane = p * members + m.
 #include <cuda_runtime.h>
 
@@ -316,6 +316,130 @@ __global__ void __launch_bounds__(kEventsBlock) rs_ens_events_kernel(const doubl
       prob[(out_base + s) * ld + p] = n == 0 ? -9999.0 : static_cast<double>(count) / static_cast<double>(n);
   }
 }
+
+// Area event probabilities (RsEnsembleAreas), step 1: the stations of one chunk into the accumulators.  A work item
+// is one (segment, event, tile of kRsAreaTile slots); the event index varies fastest, so that the events of a segment
+// run side by side and share its member values through L2.  A block holds blockDim.y items, each of 32 * ceil(M / 32)
+// threads, one per member.  Per station of the segment a thread scans the tile and its look-ahead backward once,
+// keeping the next invalid slot (nx) and the next hit slot (ny) of its member in registers, and sets bit s - s0 of
+// the station's masks where W(s) is valid, and valid with a hit.  The masks are ANDed (valid) and ORed (hit) over
+// the segment, then once into the accumulators [area][event][tile][member] with atomicAnd / atomicOr.  AND and OR
+// are exact whatever the order, so the result does not depend on chunks, segments, tiles or launch geometry.
+__global__ void __launch_bounds__(kRsAreaBlock) rs_ens_area_accumulate_kernel(
+    const double* __restrict__ mout, int n_slots, int mo_slots, int ldm, int members, int n_events, int tiles,
+    long long n_items, const RsEnsembleStatsSpec spec, const int* __restrict__ stations, int p0,
+    const int4* __restrict__ segments, unsigned long long* __restrict__ acc_valid, unsigned long long* __restrict__ acc_hit)
+{
+  const long long item = static_cast<long long>(blockIdx.x) * blockDim.y + threadIdx.y;
+  const int m = threadIdx.x;
+  if (item >= n_items || m >= members) return;
+  const int e = static_cast<int>(item % n_events);
+  const long long rest = item / n_events;
+  const int t = static_cast<int>(rest % tiles);
+  const int4 seg = __ldg(segments + rest / tiles);  // area, first and end index into `stations`
+  const RsEnsembleEvent& ev = spec.events[e];
+  const int nc = ev.n_conditions, w = ev.window;
+  const double* src[RS_ENS_MAX_CONDITIONS];
+  int op[RS_ENS_MAX_CONDITIONS];
+  double val[RS_ENS_MAX_CONDITIONS];
+#pragma unroll
+  for (int c = 0; c < RS_ENS_MAX_CONDITIONS; ++c)
+  {
+    const RsEnsembleThreshold th = ev.conditions[c < nc ? c : 0];
+    src[c] = mout + static_cast<size_t>(th.plane) * mo_slots * ldm + m;
+    op[c] = th.op;
+    val[c] = th.value;
+  }
+  const int s0 = t * kRsAreaTile;
+  const int s1 = kRsAreaTile >= n_slots - s0 ? n_slots : s0 + kRsAreaTile;
+  const int s_end = w - 1 >= n_slots - s1 ? n_slots : s1 + w - 1;  // the last window of the tile ends at s_end - 1
+  unsigned long long valid = ~0ULL, hit = 0;
+  for (int k = seg.y; k < seg.z; ++k)
+  {
+    const size_t lane = static_cast<size_t>(__ldg(stations + k) - p0) * members;
+    int nx = INT_MAX, ny = INT_MAX;
+    unsigned long long vm = 0, hm = 0;
+#pragma unroll 4
+    for (int s = s_end - 1; s >= s0; --s)
+    {
+      const size_t off = static_cast<size_t>(s) * ldm + lane;
+      bool ok = true, h = true;
+#pragma unroll
+      for (int c = 0; c < RS_ENS_MAX_CONDITIONS; ++c)
+        if (c < nc)
+        {
+          const double x = __ldg(src[c] + off);
+          const double v = val[c];
+          ok &= valid_value(x);
+          h &= op[c] == RS_ENS_LT ? x < v : op[c] == RS_ENS_LE ? x <= v : op[c] == RS_ENS_GT ? x > v : x >= v;
+        }
+      if (!ok)
+        nx = s;
+      else if (h)
+        ny = s;
+      if (s < s1)
+      {
+        const int wend = w - 1 >= n_slots - 1 - s ? n_slots - 1 : s + w - 1;
+        const unsigned long long bit = 1ULL << (s - s0);
+        if (nx > wend)
+        {
+          vm |= bit;
+          if (ny <= wend) hm |= bit;
+        }
+      }
+    }
+    valid &= vm;
+    hit |= hm;
+  }
+  const size_t a = ((static_cast<size_t>(seg.x) * n_events + e) * tiles + t) * members + m;
+  atomicAnd(acc_valid + a, valid);
+  atomicOr(acc_hit + a, hit);
+}
+
+// Step 2, once after the last chunk: one block per (area, event, tile), one thread per member.  Per slot of the tile,
+// a warp ballot and __popc count the members whose valid bit is set and those whose hit bit is set too; the warps'
+// counts are summed in shared memory and one thread per slot writes area_prob[e][s][a].
+__global__ void __launch_bounds__(kRsAreaBlock) rs_ens_area_finalize_kernel(
+    const unsigned long long* __restrict__ acc_valid, const unsigned long long* __restrict__ acc_hit, int n_areas,
+    int n_events, int tiles, int n_slots, int members, double* __restrict__ area_prob, int st_slots)
+{
+  __shared__ int counts[2][kRsAreaBlock / 32][kRsAreaTile];
+  const long long b = blockIdx.x;  // (a * n_events + e) * tiles + t
+  const int t = static_cast<int>(b % tiles), e = static_cast<int>((b / tiles) % n_events);
+  const int a = static_cast<int>(b / (static_cast<long long>(tiles) * n_events));
+  const int m = threadIdx.x, warp = m / 32, warps = blockDim.x / 32;
+  unsigned long long v = 0, h = 0;
+  if (m < members)
+  {
+    v = acc_valid[static_cast<size_t>(b) * members + m];
+    h = acc_hit[static_cast<size_t>(b) * members + m] & v;
+  }
+  for (int j = 0; j < kRsAreaTile; ++j)
+  {
+    const unsigned bv = __ballot_sync(0xffffffffu, (v >> j) & 1ULL), bh = __ballot_sync(0xffffffffu, (h >> j) & 1ULL);
+    if ((m & 31) == 0)
+    {
+      counts[0][warp][j] = __popc(bv);
+      counts[1][warp][j] = __popc(bh);
+    }
+  }
+  __syncthreads();
+  const int s0 = t * kRsAreaTile;
+  for (int j = m; j < kRsAreaTile && s0 + j < n_slots; j += blockDim.x)
+  {
+    int n = 0, count = 0;
+    for (int k = 0; k < warps; ++k)
+    {
+      n += counts[0][k][j];
+      count += counts[1][k][j];
+    }
+    area_prob[(static_cast<size_t>(e) * st_slots + s0 + j) * n_areas + a] =
+        n == 0 ? -9999.0 : static_cast<double>(count) / static_cast<double>(n);
+  }
+}
+
+// Items of one (member-)thread group per block: as many as fill kRsAreaBlock threads.
+inline int area_groups(int members) { return kRsAreaBlock / (32 * ((members + 31) / 32)); }
 }  // namespace
 
 int rs_launch_ens_prefix_local(const double* local, int ld, int npoints, const double* member_relax, int ldm,
@@ -371,5 +495,33 @@ int rs_launch_ens_events(const double* member_out, int n_slots, int mo_slots, in
   if (e != cudaSuccess) return static_cast<int>(e);
   rs_ens_events_kernel<<<static_cast<unsigned>(blocks), kEventsBlock, smem, static_cast<cudaStream_t>(stream)>>>(
       member_out, n_slots, mo_slots, ldm, npoints, members, E, static_cast<int>(tile), *spec, prob, st_slots, ld);
+  return static_cast<int>(cudaGetLastError());
+}
+
+int rs_launch_ens_area_accumulate(const double* member_out, int n_slots, int mo_slots, int ldm, int members,
+                                  const RsEnsembleStatsSpec* spec, const int* stations, int p0, const int* segments,
+                                  int n_segments, unsigned long long* acc_valid, unsigned long long* acc_hit, void* stream)
+{
+  const int E = spec->n_events, tiles = rs_area_tiles(n_slots);
+  if (E == 0 || n_segments == 0 || n_slots == 0) return 0;
+  const int groups = area_groups(members);
+  const long long items = static_cast<long long>(n_segments) * E * tiles;
+  const dim3 block(32 * ((members + 31) / 32), groups);
+  rs_ens_area_accumulate_kernel<<<static_cast<unsigned>((items + groups - 1) / groups), block, 0,
+                                  static_cast<cudaStream_t>(stream)>>>(
+      member_out, n_slots, mo_slots, ldm, members, E, tiles, items, *spec, stations, p0,
+      reinterpret_cast<const int4*>(segments), acc_valid, acc_hit);
+  return static_cast<int>(cudaGetLastError());
+}
+
+int rs_launch_ens_area_finalize(const unsigned long long* acc_valid, const unsigned long long* acc_hit, int n_areas,
+                                int n_events, int n_slots, int members, double* area_prob, int st_slots, void* stream)
+{
+  const int tiles = rs_area_tiles(n_slots);
+  if (n_events == 0 || n_areas == 0 || n_slots == 0) return 0;
+  const long long blocks = static_cast<long long>(n_areas) * n_events * tiles;
+  rs_ens_area_finalize_kernel<<<static_cast<unsigned>(blocks), 32 * ((members + 31) / 32), 0,
+                                static_cast<cudaStream_t>(stream)>>>(acc_valid, acc_hit, n_areas, n_events, tiles,
+                                                                     n_slots, members, area_prob, st_slots);
   return static_cast<int>(cudaGetLastError());
 }

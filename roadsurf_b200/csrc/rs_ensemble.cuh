@@ -45,3 +45,19 @@ int rs_launch_ens_stats(const double* member_out, int out_nvar, int n_slots, int
 // of [..][st_slots][ld]; slots >= n_slots are not written.
 int rs_launch_ens_events(const double* member_out, int n_slots, int mo_slots, int ldm, int npoints, int members,
                          const RsEnsembleStatsSpec* spec, double* prob, int st_slots, int ld, void* stream);
+
+// Area event probabilities (RsEnsembleAreas).  The accumulators acc_valid / acc_hit are
+// [n_areas][n_events][rs_area_tiles(n_slots)][members] slot masks (bit j of tile t = slot t * kRsAreaTile + j),
+// set to all ones / all zeros before the first chunk.
+constexpr int kRsAreaTile = 64;     // slots per accumulator word
+constexpr int kRsAreaBlock = 128;   // threads of an area kernel's block (at most 4 warps of members)
+inline int rs_area_tiles(int n_slots) { return (n_slots + kRsAreaTile - 1) / kRsAreaTile; }
+// Accumulates the stations [p0, p0 + npoints) of member_out [..][mo_slots][ldm] (station p at lanes
+// (p - p0) * members + m).  segments [n_segments][4] = {area, begin, end, 0}: the stations stations[begin .. end - 1]
+// (global indices, all in the chunk) of one area.  `segments` is 16-byte aligned.
+int rs_launch_ens_area_accumulate(const double* member_out, int n_slots, int mo_slots, int ldm, int members,
+                                  const RsEnsembleStatsSpec* spec, const int* stations, int p0, const int* segments,
+                                  int n_segments, unsigned long long* acc_valid, unsigned long long* acc_hit, void* stream);
+// area_prob [n_events][st_slots][n_areas] from the accumulators; slots >= n_slots are not written.
+int rs_launch_ens_area_finalize(const unsigned long long* acc_valid, const unsigned long long* acc_hit, int n_areas,
+                                int n_events, int n_slots, int members, double* area_prob, int st_slots, void* stream);

@@ -47,7 +47,7 @@ enum PoolSlot : int
   EH_FORCING = 400, EH_LOCAL = 401, EH_HOR = 402, EH_OUT = 403, EH_STATE = 404, EH_SCRATCH = 405, EH_M_FORCING = 406,
   EH_M_LOCAL = 407, EH_M_HOR = 408, EH_M_STATE = 409, EH_M_SCRATCH = 410, EH_M_OUT = 411, EH_RELAX = 412,
   EH_STATS = 413, EH_PROB = 414, EH_SOLAR = 415, EH_STATUS = 416, EH_M_STATUS = 417, EH_TIME_FIELDS = 418,
-  EH_RECORD_STEP = 419, EH_COUNTERS = 420,
+  EH_RECORD_STEP = 419, EH_COUNTERS = 420, EH_AREAS = 421, EH_AREA_PROB = 422,
   EH_H_RELAX = 400,  // pinned
 };
 
@@ -1593,7 +1593,7 @@ void roadsurf_session_close(void* session)
 
 const char* roadsurf_last_error(void) { return g_err.c_str(); }
 
-const char* roadsurf_version(void) { return "roadsurf_b200 0.2 (RoadSurf 1.6.1 per-point loop, sm_100a)"; }
+const char* roadsurf_version(void) { return "roadsurf_b200 0.3 (RoadSurf 1.6.1 per-point loop, sm_100a)"; }
 
 int roadsurf_device_count(void)
 {
@@ -2252,6 +2252,127 @@ int launch_stats_and_events(const double* member_out, int out_nvar, int n_slots,
   return RS_OK;
 }
 
+// ---- area event probabilities (RsEnsembleAreas) ----
+// Every index the area kernels use comes from here: the arrays are checked against npoints on the host.
+int check_areas(const RsEnsembleAreas* areas, int npoints, const RsEnsembleStatsSpec& spec)
+{
+  if (!areas || !areas->offsets || !areas->stations) return fail(RS_ERR_BAD_ARGUMENT, "null area pointer (areas, offsets or stations)");
+  if (areas->n_areas < 1) return fail(RS_ERR_BAD_ARGUMENT, "n_areas must be at least 1");
+  if (spec.n_events == 0) return fail(RS_ERR_BAD_ARGUMENT, "area probabilities need at least one event in the spec");
+  const int* o = areas->offsets;
+  if (o[0] != 0) return fail(RS_ERR_BAD_ARGUMENT, "area offsets[0] must be 0");
+  for (int a = 0; a < areas->n_areas; ++a)
+    if (o[a + 1] <= o[a]) return fail(RS_ERR_BAD_ARGUMENT, "area offsets must be strictly increasing (no empty area)");
+  for (int k = 0; k < o[areas->n_areas]; ++k)
+    if (areas->stations[k] < 0 || areas->stations[k] >= npoints)
+      return fail(RS_ERR_BAD_ARGUMENT, "area station index outside [0, npoints)");
+  return RS_OK;
+}
+
+// The library's copy of a checked area set: each area's stations sorted, without repeats, and the segments that the
+// accumulate kernel takes, {area, begin, end, 0}: a run of stations of one area, all in one station chunk.
+struct AreaPlan
+{
+  int n_areas = 0;
+  std::vector<int> stations;  // area after area
+  std::vector<int> first;     // [n_areas + 1]: area a is stations[first[a] .. first[a + 1] - 1]
+  std::vector<int> segments;  // [n][4], every chunk's in chunk order
+};
+
+AreaPlan plan_areas(const RsEnsembleAreas& a)
+{
+  AreaPlan pl;
+  pl.n_areas = a.n_areas;
+  pl.first.push_back(0);
+  for (int k = 0; k < a.n_areas; ++k)
+  {
+    const size_t b = pl.stations.size();
+    pl.stations.insert(pl.stations.end(), a.stations + a.offsets[k], a.stations + a.offsets[k + 1]);
+    std::sort(pl.stations.begin() + b, pl.stations.end());
+    pl.stations.erase(std::unique(pl.stations.begin() + b, pl.stations.end()), pl.stations.end());
+    pl.first.push_back(static_cast<int>(pl.stations.size()));
+  }
+  return pl;
+}
+
+// Stations per segment: enough segments that the accumulate kernel has about 2^15 work items (one warp each) per
+// chunk, so that a small ensemble spreads over the GPU, and no more, so that a large one makes few atomics and
+// reads a segment's member values in one pass; between 1 and 64.
+int area_segment_length(const AreaPlan& pl, int n_events, int n_slots, long long chunks)
+{
+  const long long items = static_cast<long long>(pl.stations.size()) * n_events * rs_area_tiles(n_slots);
+  return static_cast<int>(std::min<long long>(64, std::max<long long>(1, items / (chunks << 15))));
+}
+
+// Appends the segments of the stations [p0, p0 + n), at most `len` stations each, and returns their count.
+int plan_segments(AreaPlan& pl, long long p0, long long n, int len)
+{
+  const size_t n0 = pl.segments.size();
+  for (int a = 0; a < pl.n_areas; ++a)
+  {
+    const auto b = pl.stations.begin();
+    const int lo = static_cast<int>(std::lower_bound(b + pl.first[a], b + pl.first[a + 1], p0) - b);
+    const int hi = static_cast<int>(std::lower_bound(b + pl.first[a], b + pl.first[a + 1], p0 + n) - b);
+    for (int k = lo; k < hi; k += len) pl.segments.insert(pl.segments.end(), {a, k, std::min(k + len, hi), 0});
+  }
+  return static_cast<int>((pl.segments.size() - n0) / 4);
+}
+
+// Device copy of a plan and its accumulators in one buffer of area_bytes(): the accumulators
+// [n_areas][n_events][tiles][members] (valid, then hit), the segments, the stations.  `max_segments` bounds the
+// plan's segments where the buffer is sized before they are planned (a segment holds one station at least).
+struct AreaDevice
+{
+  size_t words = 0;  // accumulator words of each kind
+  unsigned long long *valid = nullptr, *hit = nullptr;
+  int *segments = nullptr, *stations = nullptr;
+};
+
+size_t area_bytes(const AreaPlan& pl, int n_events, int n_slots, int members, size_t max_segments)
+{
+  const size_t words = static_cast<size_t>(pl.n_areas) * n_events * rs_area_tiles(n_slots) * members;
+  return 2 * sizeof(unsigned long long) * words + sizeof(int) * (4 * max_segments + pl.stations.size());
+}
+
+// Places the buffer's parts, uploads the plan and resets the accumulators (all valid, no hit) on `st`; returns the
+// bytes copied to the device in *h2d.
+int area_upload(const AreaPlan& pl, int n_events, int n_slots, int members, void* base, cudaStream_t st, AreaDevice* d,
+                size_t* h2d)
+{
+  d->words = static_cast<size_t>(pl.n_areas) * n_events * rs_area_tiles(n_slots) * members;
+  d->valid = static_cast<unsigned long long*>(base);
+  d->hit = d->valid + d->words;
+  d->segments = reinterpret_cast<int*>(d->hit + d->words);  // 16-byte aligned: 2 * words * 8 bytes from base
+  d->stations = d->segments + pl.segments.size();
+  CU(cudaMemsetAsync(d->valid, 0xff, sizeof(unsigned long long) * d->words, st));
+  CU(cudaMemsetAsync(d->hit, 0, sizeof(unsigned long long) * d->words, st));
+  CU(cudaMemcpyAsync(d->segments, pl.segments.data(), sizeof(int) * pl.segments.size(), cudaMemcpyHostToDevice, st));
+  CU(cudaMemcpyAsync(d->stations, pl.stations.data(), sizeof(int) * pl.stations.size(), cudaMemcpyHostToDevice, st));
+  *h2d = sizeof(int) * (pl.segments.size() + pl.stations.size());
+  return RS_OK;
+}
+
+int area_accumulate(const AreaDevice& d, const double* member_out, int n_slots, int mo_slots, int ldm, int members,
+                    const RsEnsembleStatsSpec* spec, int p0, int first_segment, int n_segments, cudaStream_t st)
+{
+  if (n_segments == 0 || n_slots == 0) return RS_OK;
+  CU(static_cast<cudaError_t>(rs_launch_ens_area_accumulate(member_out, n_slots, mo_slots, ldm, members, spec, d.stations,
+                                                            p0, d.segments + 4 * static_cast<size_t>(first_segment),
+                                                            n_segments, d.valid, d.hit, st)));
+  ++g_launches_total;
+  return RS_OK;
+}
+
+int area_finalize(const AreaDevice& d, int n_areas, int n_events, int n_slots, int members, double* area_prob, int st_slots,
+                  cudaStream_t st)
+{
+  if (n_slots == 0) return RS_OK;
+  CU(static_cast<cudaError_t>(
+      rs_launch_ens_area_finalize(d.valid, d.hit, n_areas, n_events, n_slots, members, area_prob, st_slots, st)));
+  ++g_launches_total;
+  return RS_OK;
+}
+
 // Where the fork may sit (pure host checks).  record_step: host copy (forcing_mode 1) or null.
 int check_fork(int forcing_mode, int sim_len, int fork_step, int members, const int* record_step, int n_records, int* r_f)
 {
@@ -2293,6 +2414,35 @@ int roadsurf_ensemble_stats(const double* member_out, int out_nvar, int n_out, i
   }
   return launch_stats_and_events(member_out, out_nvar, n_out, n_out, ld_members, npoints, members, spec, stats, prob, n_out,
                                  ld, stream);
+}
+
+int roadsurf_ensemble_area_events(const double* member_out, int out_nvar, int n_out, int ld_members, int npoints,
+                                  int members, const RsEnsembleStatsSpec* spec, const RsEnsembleAreas* areas,
+                                  double* area_prob, void* stream)
+{
+  if (!member_out || !spec || !area_prob || members < 1 || members > RS_ENS_MAX_MEMBERS || npoints < 0 || n_out < 0 ||
+      (out_nvar != RS_O_NVAR && out_nvar != RS_O_NVAR_EXT) || static_cast<long long>(ld_members) < static_cast<long long>(npoints) * members)
+    return fail(RS_ERR_BAD_ARGUMENT, "bad arguments");
+  {
+    int rc = check_stats_spec(*spec, out_nvar);
+    if (rc == RS_OK) rc = check_areas(areas, npoints, *spec);
+    if (rc != RS_OK) return rc;
+  }
+  if (n_out == 0) return RS_OK;
+  AreaPlan pl = plan_areas(*areas);
+  const int n_segments = plan_segments(pl, 0, npoints, area_segment_length(pl, spec->n_events, n_out, 1));
+  const size_t bytes = area_bytes(pl, spec->n_events, n_out, members, n_segments);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  void* buf = nullptr;
+  CU(cudaMallocAsync(&buf, bytes, st));
+  AreaDevice d;
+  size_t h2d = 0;
+  int rc = area_upload(pl, spec->n_events, n_out, members, buf, st, &d, &h2d);
+  if (rc == RS_OK) rc = area_accumulate(d, member_out, n_out, n_out, ld_members, members, spec, 0, 0, n_segments, st);
+  if (rc == RS_OK) rc = area_finalize(d, pl.n_areas, spec->n_events, n_out, members, area_prob, n_out, st);
+  const cudaError_t e = cudaFreeAsync(buf, st);
+  if (rc == RS_OK && e != cudaSuccess) return fail(RS_ERR_CUDA, std::string("cudaFreeAsync: ") + cudaGetErrorString(e));
+  return rc;
 }
 
 }  // extern "C"
@@ -2449,6 +2599,15 @@ int roadsurf_run_ensemble_host_soa(const RsHostBatch* b, const double* member_re
                                    const int* latest_obs_index, const RsEnsembleStatsSpec* spec, double* stats, double* prob, double* member_out,
                                    int* member_status, const InputSettings* settings, const InputParameters* params)
 {
+  return roadsurf_run_ensemble_host_soa_areas(b, member_records, members, fork_step, latest_obs_index, spec, stats, prob,
+                                              member_out, member_status, nullptr, nullptr, settings, params);
+}
+
+int roadsurf_run_ensemble_host_soa_areas(const RsHostBatch* b, const double* member_records, int members, int fork_step,
+                                         const int* latest_obs_index, const RsEnsembleStatsSpec* spec, double* stats,
+                                         double* prob, double* member_out, int* member_status, const RsEnsembleAreas* areas,
+                                         double* area_prob, const InputSettings* settings, const InputParameters* params)
+{
   g_err.clear();
   std::memset(&g_stats, 0, sizeof g_stats);
   const double wall0 = now_ms();
@@ -2471,6 +2630,13 @@ int roadsurf_run_ensemble_host_soa(const RsHostBatch* b, const double* member_re
   }
   {
     const int rc = check_stats_spec(*spec, RS_O_NVAR);
+    if (rc != RS_OK) return rc;
+  }
+  if ((areas == nullptr) != (area_prob == nullptr))
+    return fail(RS_ERR_BAD_ARGUMENT, "null area pointer: areas and area_prob go together");
+  if (areas)
+  {
+    const int rc = check_areas(areas, P, *spec);
     if (rc != RS_OK) return rc;
   }
   if (P > 0 && !member_records) return fail(RS_ERR_BAD_ARGUMENT, "null member_records");
@@ -2543,11 +2709,31 @@ int roadsurf_run_ensemble_host_soa(const RsHostBatch* b, const double* member_re
       sizeof(double) * M * (frows_m + RS_L_NLOCAL + (hor ? 360 : 0) + NS + (cpl ? SC : 0) + 1 + 3 + RS_O_NVAR * n_m);
   size_t free_b = 0, total_b = 0;
   CU(cudaMemGetInfo(&free_b, &total_b));
-  long long pc = static_cast<long long>(free_b * 0.8 / per_station) - 64;
+  // areas: the plan and the accumulators stay on the device for the whole call, beside area_prob
+  AreaPlan area_plan;
+  const int E = spec->n_events;
+  size_t area_fixed = 0;
+  if (areas)
+  {
+    area_plan = plan_areas(*areas);
+    area_fixed = area_bytes(area_plan, E, n_m, M, area_plan.stations.size()) + sizeof(double) * E * n_m * areas->n_areas;
+    if (static_cast<double>(area_fixed) >= free_b * 0.8)
+      return fail(RS_ERR_CUDA, "not enough device memory for the area accumulators (2 * n_areas * n_events * "
+                               "ceil(n_out_m / 64) * members * 8 bytes) and area_prob");
+  }
+  long long pc = static_cast<long long>((free_b * 0.8 - static_cast<double>(area_fixed)) / per_station) - 64;
   if (const int cap = g_opt_max_slots.load()) pc = std::min<long long>(pc, std::max(1, cap / M));
   pc = std::min<long long>(pc, P);
   if (pc < 1) return fail(RS_ERR_CUDA, "not enough device memory for one station's members");
   const int ldc = static_cast<int>((pc + 31) / 32 * 32), ldmc = static_cast<int>((pc * M + 31) / 32 * 32);
+  std::vector<int> chunk_segments;  // [chunks + 1]: the segments of chunk c are [chunk_segments[c], chunk_segments[c + 1])
+  if (areas)
+  {
+    const int len = area_segment_length(area_plan, E, n_m, (P + pc - 1) / pc);
+    chunk_segments.push_back(0);
+    for (long long p0 = 0; p0 < P; p0 += pc)
+      chunk_segments.push_back(chunk_segments.back() + plan_segments(area_plan, p0, std::min<long long>(pc, P - p0), len));
+  }
 
   SoaStreams* ss = nullptr;
   {
@@ -2587,6 +2773,19 @@ int roadsurf_run_ensemble_host_soa(const RsHostBatch* b, const double* member_re
   CU(cudaMemcpyAsync(d_rs, b->record_step, sizeof(int) * nrec, cudaMemcpyHostToDevice, st));
   CU(cudaMemsetAsync(d_counters, 0, sizeof(unsigned long long) * RS_CNT_N, st));
   g_stats.h2d_bytes += sizeof(int) * (6 * sim_len + nrec);
+  AreaDevice d_areas;
+  double* d_area_prob = nullptr;
+  const size_t area_prob_n = areas ? static_cast<size_t>(E) * n_m * areas->n_areas : 0;
+  if (areas)
+  {
+    unsigned long long* buf;
+    CU(pooled(dev, EH_AREAS, (area_bytes(area_plan, E, n_m, M, area_plan.segments.size() / 4) + 7) / 8, &buf));
+    CU(pooled(dev, EH_AREA_PROB, std::max<size_t>(1, area_prob_n), &d_area_prob));
+    size_t h2d = 0;
+    const int rc = area_upload(area_plan, E, n_m, M, buf, st, &d_areas, &h2d);
+    if (rc != RS_OK) return rc;
+    g_stats.h2d_bytes += h2d;
+  }
   g_stats.setup_ms = now_ms() - setup0;
   const int launches0 = g_launches_total.load();
 
@@ -2648,6 +2847,15 @@ int roadsurf_run_ensemble_host_soa(const RsHostBatch* b, const double* member_re
       const int rc = run_ensemble(&e, st, b->record_step);
       if (rc != RS_OK) return rc;
     }
+    const long long chunk = p0 / pc;
+    const bool last = p0 + pc >= P;
+    if (areas)
+    {
+      int rc = area_accumulate(d_areas, d_mo, n_m, e.n_out_members, ldm, M, spec, static_cast<int>(p0),
+                               chunk_segments[chunk], chunk_segments[chunk + 1] - chunk_segments[chunk], st);
+      if (rc == RS_OK && last) rc = area_finalize(d_areas, areas->n_areas, E, n_m, M, d_area_prob, n_m, st);
+      if (rc != RS_OK) return rc;
+    }
     CU(cudaEventRecord(ev[2], st));
     if (b->out && pre1 > pre0)
       CU(cudaMemcpy2DAsync(b->out + col, D * np, d_out, D * ld, D * n, static_cast<size_t>(RS_O_NVAR) * (pre1 - pre0),
@@ -2662,6 +2870,11 @@ int roadsurf_run_ensemble_host_soa(const RsHostBatch* b, const double* member_re
       CU(cudaMemcpyAsync(member_status + colm, d_mstatus, sizeof(int) * nm, cudaMemcpyDeviceToHost, st));
     g_stats.d2h_bytes += D * (n * ((b->out ? RS_O_NVAR * (pre1 - pre0) : 0) + (stats ? srows : 0) + (prob ? prows : 0)) +
                               (member_out ? nm * RS_O_NVAR * n_m : 0)) + (member_status ? sizeof(int) * nm : 0);
+    if (areas && last && area_prob_n > 0)
+    {
+      CU(cudaMemcpyAsync(area_prob, d_area_prob, D * area_prob_n, cudaMemcpyDeviceToHost, st));
+      g_stats.d2h_bytes += D * area_prob_n;
+    }
     CU(cudaEventRecord(ev[3], st));
     CU(cudaStreamSynchronize(st));
     add_stage_times(g_stats, ev);

@@ -40,7 +40,8 @@ EXPORTS = ("runsimulation", "roadsurf_last_error", "roadsurf_device_count", "roa
            "roadsurf_session_done", "roadsurf_session_close", "roadsurf_expand_records",
            "roadsurf_sun_position", "roadsurf_eval_primitive",
            "roadsurf_version",
-           "roadsurf_run_ensemble_device", "roadsurf_ensemble_stats", "roadsurf_run_ensemble_host_soa")
+           "roadsurf_run_ensemble_device", "roadsurf_ensemble_stats", "roadsurf_run_ensemble_host_soa",
+           "roadsurf_ensemble_area_events", "roadsurf_run_ensemble_host_soa_areas")
 (PRIM_EXP, PRIM_EXP_SMEM, PRIM_LOG, PRIM_LOG_SMEM, PRIM_EXP_FLAT, PRIM_EXP_FLAT_SMEM, PRIM_PSIH_UNSTABLE,
  PRIM_PSIH_UNSTABLE_SMEM, PRIM_FRCP, PRIM_FDIV, PRIM_DIV_CONST, PRIM_N) = range(12)
 ENS_MAX_MEMBERS, ENS_MAX_QUANTILES, ENS_MAX_THRESHOLDS = 128, 8, 8
@@ -117,6 +118,22 @@ class RsEnsembleBatch(C.Structure):
                 ("member_status", C.c_void_p), ("member_out", C.c_void_p), ("n_out_members", C.c_int),
                 ("member_order", C.c_void_p), ("spec", RsEnsembleStatsSpec), ("stats", C.c_void_p),
                 ("prob", C.c_void_p)]
+
+
+class RsEnsembleAreas(C.Structure):
+    _fields_ = [("n_areas", C.c_int), ("offsets", C.c_void_p), ("stations", C.c_void_p)]
+
+
+def ensemble_areas(station_lists):
+    """RsEnsembleAreas from a list of areas, each a list of station indices (a route, a district, ...).  The struct
+    keeps the int32 arrays it points to alive (attributes `offsets_array`, `stations_array`)."""
+    lists = [np.asarray(a, dtype=np.int32).ravel() for a in station_lists]
+    offsets = np.zeros(len(lists) + 1, dtype=np.int32)
+    offsets[1:] = np.cumsum([len(a) for a in lists])
+    stations = np.ascontiguousarray(np.concatenate(lists) if lists else np.zeros(0, dtype=np.int32))
+    areas = RsEnsembleAreas(n_areas=len(lists), offsets=offsets.ctypes.data, stations=stations.ctypes.data)
+    areas.offsets_array, areas.stations_array = offsets, stations
+    return areas
 
 
 def stats_spec(quantiles=(), thresholds=(), events=()):
@@ -216,6 +233,13 @@ def load():
                                                    P(RsEnsembleStatsSpec), C.c_void_p, C.c_void_p, C.c_void_p,
                                                    C.c_void_p, P(IS), P(IPa)]
     lib.roadsurf_run_ensemble_host_soa.restype = C.c_int
+    lib.roadsurf_ensemble_area_events.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                                                  P(RsEnsembleStatsSpec), P(RsEnsembleAreas), C.c_void_p, C.c_void_p]
+    lib.roadsurf_ensemble_area_events.restype = C.c_int
+    lib.roadsurf_run_ensemble_host_soa_areas.argtypes = [P(RsHostBatch), C.c_void_p, C.c_int, C.c_int, C.c_void_p,
+                                                         P(RsEnsembleStatsSpec), C.c_void_p, C.c_void_p, C.c_void_p,
+                                                         C.c_void_p, P(RsEnsembleAreas), C.c_void_p, P(IS), P(IPa)]
+    lib.roadsurf_run_ensemble_host_soa_areas.restype = C.c_int
     _lib = lib
     return lib
 
@@ -642,6 +666,22 @@ def ensemble_stats(member_out, npoints, members, spec, stream=None):
     return stats[..., :npoints], prob[:spec.n_prob, :, :npoints]
 
 
+def ensemble_area_events(member_out, npoints, members, spec, areas, stream=None):
+    """roadsurf_ensemble_area_events on a torch CUDA tensor member_out [out_nvar, n_out, ld_members] (lane
+    p * members + m); areas is an RsEnsembleAreas (ensemble_areas).  Returns area_prob
+    [n_events, n_out, n_areas] as a CUDA tensor (synchronised)."""
+    import torch
+    out_nvar, n_out, ldm = member_out.shape
+    area_prob = torch.full((spec.n_events, n_out, areas.n_areas), 12345.0, dtype=torch.float64,
+                           device=member_out.device)
+    st = stream if stream is not None else torch.cuda.current_stream()
+    _check(load().roadsurf_ensemble_area_events(member_out.data_ptr(), out_nvar, n_out, ldm, int(npoints),
+                                                int(members), C.byref(spec), C.byref(areas), area_prob.data_ptr(),
+                                                C.c_void_p(st.cuda_stream)))
+    torch.cuda.synchronize()
+    return area_prob
+
+
 def fork_record(record_step, fork_step):
     """r_f: the last record at or before 0-based step fork_step - 1."""
     rs = np.asarray(record_step)
@@ -765,30 +805,34 @@ class EnsembleBatch:
 
 def run_ensemble_host_soa(settings, params, forcing, record_step, time_fields, local, member_records, members,
                           fork_step, spec, horizons=None, out_stride=1, coupling_window_end=0, out=None,
-                          member_out=False, member_status=False, latest_obs_index=None):
-    """roadsurf_run_ensemble_host_soa on host arrays: forcing [n_records, nvar, P], record_step [n_records],
+                          member_out=False, member_status=False, latest_obs_index=None, areas=None, prob=True):
+    """roadsurf_run_ensemble_host_soa_areas on host arrays: forcing [n_records, nvar, P], record_step [n_records],
     local [L_NLOCAL, P], member_records [n_records - r_f - 1, nvar, P * members], latest_obs_index [P] int32 (the
-    relaxation rule of read_input_derive_records; None = no observations).  Returns a dict with
-    stats [5 + nq, 6, n_out_m, P], prob [nt + n_events, n_out_m, P] and, when asked for, member_out [6, n_out_m, P * M]
-    and member_status [P * M]."""
+    relaxation rule of read_input_derive_records; None = no observations), areas an RsEnsembleAreas (ensemble_areas)
+    or None.  Returns a dict with stats [5 + nq, 6, n_out_m, P], prob [nt + n_events, n_out_m, P] (unless prob=False:
+    NULL is passed) and, when asked for, member_out [6, n_out_m, P * M], member_status [P * M] and area_prob
+    [n_events, n_out_m, n_areas]."""
     n_records, nvar, npoints = forcing.shape
     sim_len = time_fields.shape[1]
     k0 = fork_step - 1
     slot0 = (k0 + out_stride - 1) // out_stride
     n_m = (sim_len + out_stride - 1) // out_stride - slot0
-    res = dict(stats=np.zeros((ENS_NFIXED + spec.n_quantiles, O_NVAR, n_m, npoints)),
-               prob=np.zeros((spec.n_prob, n_m, npoints)))
+    res = dict(stats=np.zeros((ENS_NFIXED + spec.n_quantiles, O_NVAR, n_m, npoints)))
+    if prob:
+        res["prob"] = np.zeros((spec.n_prob, n_m, npoints))
     if member_out:
         res["member_out"] = np.zeros((O_NVAR, n_m, npoints * members))
     if member_status:
         res["member_status"] = np.zeros(npoints * members, dtype=np.int32)
+    if areas is not None:
+        res["area_prob"] = np.zeros((spec.n_events, n_m, areas.n_areas))
     hb = RsHostBatch(npoints=npoints, sim_len=sim_len, forcing_mode=1, n_records=n_records, nvar=nvar,
                      out_stride=out_stride, forcing=_ptr(forcing), record_step=_ptr(record_step),
                      time_fields=_ptr(time_fields), local=_ptr(local), horizons=_ptr(horizons), out=_ptr(out),
                      coupling_window_end=int(coupling_window_end))
     lat = None if latest_obs_index is None else np.ascontiguousarray(latest_obs_index, dtype=np.int32)
-    _check(load().roadsurf_run_ensemble_host_soa(C.byref(hb), _ptr(member_records), int(members), int(fork_step),
-                                                 _ptr(lat), C.byref(spec), _ptr(res["stats"]), _ptr(res["prob"]),
-                                                 _ptr(res.get("member_out")), _ptr(res.get("member_status")),
-                                                 C.byref(settings), C.byref(params)))
+    _check(load().roadsurf_run_ensemble_host_soa_areas(
+        C.byref(hb), _ptr(member_records), int(members), int(fork_step), _ptr(lat), C.byref(spec), _ptr(res["stats"]),
+        _ptr(res.get("prob")), _ptr(res.get("member_out")), _ptr(res.get("member_status")),
+        None if areas is None else C.byref(areas), _ptr(res.get("area_prob")), C.byref(settings), C.byref(params)))
     return res
