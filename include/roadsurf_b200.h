@@ -725,6 +725,25 @@ typedef struct RsEnsembleAreas
                           [0, npoints) */
 } RsEnsembleAreas;
 
+/* Event onset: the probability that an event of spec.events has begun by each member slot, per station and per
+ * area ("by 03:00, how likely is it that freezing has begun on this route?").  It uses the events' conditions; their
+ * window does not enter.  For station p, event e, member m and member slot s < S (the slots the station events cover):
+ *   - valid: every plane the conditions name holds a valid value (value == value and > -9000) at every slot of
+ *     [0, s];
+ *   - hit: valid, and the conjunction of the conditions holds at one slot or more of [0, s];
+ *   - result: onset[e][s][p] = (double)hits / (double)valid, -9999.0 where no member is valid;
+ *   - areas (RsEnsembleAreas): a member is valid for area A at s when it is valid at every station of A, and hits
+ *     when it is also a hit at one station of A or more; area_onset[e][s][a] likewise.
+ * This is the event rule and the area rule applied to the growing window [0, s].  So onset[e][s][p] equals, bit for
+ * bit, the station event probability at slot 0 of an event with the same conditions and window = s + 1, and
+ * area_onset[e][s][a] equals area_prob of that event at slot 0.  An area of one station equals that station's onset
+ * plane.  Per (station, event, member) the library keeps two integers: X, the first slot where a named plane is
+ * invalid (S if none), and O, the first slot before X where the conditions hold (none if there is none); then valid(s)
+ * <=> X > s and hit(s) <=> O <= s, and an area takes per member the minimum X and the minimum O over its stations.
+ * Where a station's valid members do not change with s (no invalid value after slot 0), its onset never decreases
+ * with s, so the lead time by which a fraction q of the members have seen the event is the first s with
+ * onset >= q. */
+
 /* A device-resident ensemble (DEVICE pointers on the current device). */
 typedef struct RsEnsembleBatch
 {
@@ -790,6 +809,18 @@ int roadsurf_ensemble_area_events(const double* member_out, int out_nvar, int n_
                                   int members, const RsEnsembleStatsSpec* spec, const RsEnsembleAreas* areas,
                                   double* area_prob, void* stream);
 
+/* Event onset (defined after RsEnsembleAreas) over a station-major member tensor member_out
+ * [out_nvar][n_out][ld_members] (lane p * members + m), as for roadsurf_ensemble_stats: onset DEVICE [n_events][n_out][ld] or NULL, area_onset
+ * DEVICE [n_events][n_out][n_areas] or NULL (then areas must be NULL too); one of the two at least.
+ * spec->n_events >= 1; quantiles and thresholds are ignored.  The area arrays are host memory, checked and copied as
+ * for roadsurf_ensemble_area_events; asynchronous on `stream` otherwise.  After roadsurf_run_ensemble_device:
+ *   roadsurf_run_ensemble_device(&e, stream);
+ *   roadsurf_ensemble_onset(e.member_out, e.shared.out_nvar, e.n_out_members, e.ld_members, e.shared.npoints,
+ *                           e.members, &e.spec, d_onset, e.shared.ld, &areas, d_area_onset, stream); */
+int roadsurf_ensemble_onset(const double* member_out, int out_nvar, int n_out, int ld_members, int npoints, int members,
+                            const RsEnsembleStatsSpec* spec, double* onset, int ld, const RsEnsembleAreas* areas,
+                            double* area_onset, void* stream);
+
 /* Host form on the current device, forcing_mode 1 only.  `shared` is the stations' host SoA batch
  * (as for roadsurf_run_host_soa, with the full record axis); its `out`, if not NULL, receives the
  * station outputs of the steps before F, [RS_O_NVAR][n_out_pre][P] with n_out_pre = ceil((F - 1) /
@@ -821,6 +852,21 @@ int roadsurf_run_ensemble_host_soa_areas(const RsHostBatch* shared, const double
                                          double* stats, double* prob, double* member_out, int* member_status,
                                          const RsEnsembleAreas* areas, double* area_prob,
                                          const InputSettings* settings, const InputParameters* params);
+
+/* roadsurf_run_ensemble_host_soa_areas plus event onset (defined after RsEnsembleAreas): onset HOST
+ * [n_events][n_out_m][P] and area_onset HOST [n_events][n_out_m][n_areas], each NULL or not.  The onset planes are copied back after each
+ * station chunk, area_onset once at the end (both counted in d2h_bytes; the onset kernels in kernel_ms).  Any of
+ * prob, area_prob, onset and area_onset may be NULL; areas go with area_prob or area_onset, and area_prob or
+ * area_onset without areas is RS_ERR_BAD_ARGUMENT, as are onset outputs with a spec without events.  With onset and
+ * area_onset NULL it is exactly roadsurf_run_ensemble_host_soa_areas.  Device memory for the whole call, beside the
+ * area event accumulators: the area onset accumulators, n_areas * n_events * members * 8 bytes, and area_onset,
+ * n_events * n_out_m * n_areas * 8 bytes (RS_ERR_CUDA where they do not fit); per station chunk a workspace of
+ * n_events * 8 bytes per member lane. */
+int roadsurf_run_ensemble_host_soa_onset(const RsHostBatch* shared, const double* member_records, int members,
+                                         int fork_step, const int* latest_obs_index, const RsEnsembleStatsSpec* spec,
+                                         double* stats, double* prob, double* member_out, int* member_status,
+                                         const RsEnsembleAreas* areas, double* area_prob, double* onset,
+                                         double* area_onset, const InputSettings* settings, const InputParameters* params);
 
 #ifdef __cplusplus
 }

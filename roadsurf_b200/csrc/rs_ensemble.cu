@@ -440,6 +440,135 @@ __global__ void __launch_bounds__(kRsAreaBlock) rs_ens_area_finalize_kernel(
 
 // Items of one (member-)thread group per block: as many as fill kRsAreaBlock threads.
 inline int area_groups(int members) { return kRsAreaBlock / (32 * ((members + 31) / 32)); }
+
+constexpr int kOnsetStations = 64;  // stations of an onset block
+constexpr int kOnsetBlock = 256;
+
+// Event onset (roadsurf_ensemble_onset).  A block is one event and kOnsetStations stations; the event index varies
+// fastest over the blocks, so that the events of a station block run side by side and share the member values
+// through L2.  Step 1: thread t scans the member lanes t, t + kOnsetBlock, ... of the block's stations forward from
+// slot 0 and stops at X, the first slot where a named plane is invalid (n_slots if none), keeping O, the first slot
+// before X where the conditions all hold (n_slots if none).  Consecutive threads read consecutive lanes, and each
+// member value is read at most once.  {O, X} goes to the workspace ws[e][lane] (areas) and to shared memory
+// (os[m * kOnsetStations + station]).  Step 2 (onset planes): a thread per (slot, station), the station varying
+// fastest, counts the members with X > s (valid) and with O <= s too (hit) and writes onset[e][s][p], so that the
+// writes of a warp are consecutive stations of one plane row.
+__global__ void __launch_bounds__(kOnsetBlock) rs_ens_onset_kernel(const double* __restrict__ mout, int n_slots, int mo_slots,
+                                                                   int ldm, int npoints, int members, int n_events,
+                                                                   const RsEnsembleStatsSpec spec, double* __restrict__ onset,
+                                                                   int st_slots, int ld, int2* __restrict__ ws)
+{
+  extern __shared__ int2 os_smem[];
+  const int e = static_cast<int>(blockIdx.x % n_events);
+  const int pb = static_cast<int>(blockIdx.x / n_events) * kOnsetStations;
+  const int nst = min(kOnsetStations, npoints - pb);
+  const RsEnsembleEvent& ev = spec.events[e];
+  const int nc = ev.n_conditions;
+  const double* src[RS_ENS_MAX_CONDITIONS];
+  int op[RS_ENS_MAX_CONDITIONS];
+  double val[RS_ENS_MAX_CONDITIONS];
+#pragma unroll
+  for (int c = 0; c < RS_ENS_MAX_CONDITIONS; ++c)
+  {
+    const RsEnsembleThreshold th = ev.conditions[c < nc ? c : 0];
+    src[c] = mout + static_cast<size_t>(th.plane) * mo_slots * ldm + static_cast<size_t>(pb) * members;
+    op[c] = th.op;
+    val[c] = th.value;
+  }
+  const int lanes = nst * members;
+  for (int l = threadIdx.x; l < lanes; l += kOnsetBlock)
+  {
+    int x = n_slots, o = n_slots;
+    for (int s = 0; s < n_slots; ++s)
+    {
+      const size_t off = static_cast<size_t>(s) * ldm + l;
+      bool ok = true, hit = true;
+#pragma unroll
+      for (int c = 0; c < RS_ENS_MAX_CONDITIONS; ++c)
+        if (c < nc)
+        {
+          const double v = __ldg(src[c] + off);
+          ok &= valid_value(v);
+          hit &= op[c] == RS_ENS_LT ? v < val[c] : op[c] == RS_ENS_LE ? v <= val[c] : op[c] == RS_ENS_GT ? v > val[c] : v >= val[c];
+        }
+      if (!ok)
+      {
+        x = s;
+        break;
+      }
+      if (hit && o == n_slots) o = s;
+    }
+    if (ws) ws[static_cast<size_t>(e) * npoints * members + static_cast<size_t>(pb) * members + l] = make_int2(o, x);
+    if (onset) os_smem[(l % members) * kOnsetStations + l / members] = make_int2(o, x);
+  }
+  if (!onset) return;
+  __syncthreads();
+  for (int i = threadIdx.x; i < nst * n_slots; i += kOnsetBlock)
+  {
+    const int q = i % nst, s = i / nst;
+    int n = 0, count = 0;
+    for (int m = 0; m < members; ++m)
+    {
+      const int2 t = os_smem[m * kOnsetStations + q];
+      const bool valid = t.y > s;
+      n += valid ? 1 : 0;
+      count += (valid && t.x <= s) ? 1 : 0;
+    }
+    onset[(static_cast<size_t>(e) * st_slots + s) * ld + pb + q] =
+        n == 0 ? -9999.0 : static_cast<double>(count) / static_cast<double>(n);
+  }
+}
+
+// Area onset, step 1: the stations of one chunk into the accumulators.  A work item is one (segment, event), the
+// event varying fastest; a block holds blockDim.y items of 32 * ceil(M / 32) threads, one per member.  A thread takes
+// the minimum O and the minimum X of its member over the segment's stations from the workspace, then one atomicMin
+// each into acc[area][event][member] = {O, X}.  The minimum is exact whatever the order, so the result does not
+// depend on chunks, segments or launch geometry.
+__global__ void __launch_bounds__(kRsAreaBlock) rs_ens_area_onset_accumulate_kernel(
+    const int2* __restrict__ ws, int lanes, int members, int n_events, long long n_items, const int* __restrict__ stations,
+    int p0, const int4* __restrict__ segments, int* __restrict__ acc)
+{
+  const long long item = static_cast<long long>(blockIdx.x) * blockDim.y + threadIdx.y;
+  const int m = threadIdx.x;
+  if (item >= n_items || m >= members) return;
+  const int e = static_cast<int>(item % n_events);
+  const int4 seg = __ldg(segments + item / n_events);  // area, first and end index into `stations`
+  const int2* w = ws + static_cast<size_t>(e) * lanes + m;
+  int o = INT_MAX, x = INT_MAX;
+  for (int k = seg.y; k < seg.z; ++k)
+  {
+    const int2 t = __ldg(w + static_cast<size_t>(__ldg(stations + k) - p0) * members);
+    o = min(o, t.x);
+    x = min(x, t.y);
+  }
+  int* a = acc + 2 * ((static_cast<size_t>(seg.x) * n_events + e) * members + m);
+  atomicMin(a, o);
+  atomicMin(a + 1, x);
+}
+
+// Area onset, step 2, once after the last chunk: one thread per (event, slot, area), the area varying fastest, counts
+// the members with X > s (valid) and with O <= s too (hit) and writes area_onset[e][s][a].
+__global__ void __launch_bounds__(kRsAreaBlock) rs_ens_area_onset_finalize_kernel(
+    const int* __restrict__ acc, int n_areas, int n_events, int n_slots, int members, double* __restrict__ area_onset,
+    int st_slots)
+{
+  const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i >= static_cast<long long>(n_areas) * n_slots * n_events) return;
+  const int a = static_cast<int>(i % n_areas);
+  const int s = static_cast<int>((i / n_areas) % n_slots);
+  const int e = static_cast<int>(i / (static_cast<long long>(n_areas) * n_slots));
+  const int2* t = reinterpret_cast<const int2*>(acc) + (static_cast<size_t>(a) * n_events + e) * members;
+  int n = 0, count = 0;
+  for (int m = 0; m < members; ++m)
+  {
+    const int2 v = __ldg(t + m);
+    const bool valid = v.y > s;
+    n += valid ? 1 : 0;
+    count += (valid && v.x <= s) ? 1 : 0;
+  }
+  area_onset[(static_cast<size_t>(e) * st_slots + s) * n_areas + a] =
+      n == 0 ? -9999.0 : static_cast<double>(count) / static_cast<double>(n);
+}
 }  // namespace
 
 int rs_launch_ens_prefix_local(const double* local, int ld, int npoints, const double* member_relax, int ldm,
@@ -523,5 +652,44 @@ int rs_launch_ens_area_finalize(const unsigned long long* acc_valid, const unsig
   rs_ens_area_finalize_kernel<<<static_cast<unsigned>(blocks), 32 * ((members + 31) / 32), 0,
                                 static_cast<cudaStream_t>(stream)>>>(acc_valid, acc_hit, n_areas, n_events, tiles,
                                                                      n_slots, members, area_prob, st_slots);
+  return static_cast<int>(cudaGetLastError());
+}
+
+int rs_launch_ens_onset(const double* member_out, int n_slots, int mo_slots, int ldm, int npoints, int members,
+                        const RsEnsembleStatsSpec* spec, double* onset, int st_slots, int ld, int* ws, void* stream)
+{
+  const int E = spec->n_events;
+  if (E == 0 || npoints == 0 || n_slots == 0 || (!onset && !ws)) return 0;
+  const long long blocks = static_cast<long long>(E) * ((npoints + kOnsetStations - 1) / kOnsetStations);
+  const int smem = onset ? static_cast<int>(sizeof(int2)) * kOnsetStations * members : 0;
+  cudaError_t e = cudaFuncSetAttribute(rs_ens_onset_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+  if (e != cudaSuccess) return static_cast<int>(e);
+  rs_ens_onset_kernel<<<static_cast<unsigned>(blocks), kOnsetBlock, smem, static_cast<cudaStream_t>(stream)>>>(
+      member_out, n_slots, mo_slots, ldm, npoints, members, E, *spec, onset, st_slots, ld, reinterpret_cast<int2*>(ws));
+  return static_cast<int>(cudaGetLastError());
+}
+
+int rs_launch_ens_area_onset_accumulate(const int* ws, int npoints, int members, int n_events, const int* stations, int p0,
+                                        const int* segments, int n_segments, int* acc, void* stream)
+{
+  if (n_events == 0 || n_segments == 0) return 0;
+  const int groups = area_groups(members);
+  const long long items = static_cast<long long>(n_segments) * n_events;
+  const dim3 block(32 * ((members + 31) / 32), groups);
+  rs_ens_area_onset_accumulate_kernel<<<static_cast<unsigned>((items + groups - 1) / groups), block, 0,
+                                        static_cast<cudaStream_t>(stream)>>>(
+      reinterpret_cast<const int2*>(ws), npoints * members, members, n_events, items, stations, p0,
+      reinterpret_cast<const int4*>(segments), acc);
+  return static_cast<int>(cudaGetLastError());
+}
+
+int rs_launch_ens_area_onset_finalize(const int* acc, int n_areas, int n_events, int n_slots, int members,
+                                      double* area_onset, int st_slots, void* stream)
+{
+  const long long total = static_cast<long long>(n_areas) * n_slots * n_events;
+  if (total == 0) return 0;
+  rs_ens_area_onset_finalize_kernel<<<static_cast<unsigned>((total + kRsAreaBlock - 1) / kRsAreaBlock), kRsAreaBlock, 0,
+                                      static_cast<cudaStream_t>(stream)>>>(acc, n_areas, n_events, n_slots, members,
+                                                                           area_onset, st_slots);
   return static_cast<int>(cudaGetLastError());
 }

@@ -61,3 +61,17 @@ int rs_launch_ens_area_accumulate(const double* member_out, int n_slots, int mo_
 // area_prob [n_events][st_slots][n_areas] from the accumulators; slots >= n_slots are not written.
 int rs_launch_ens_area_finalize(const unsigned long long* acc_valid, const unsigned long long* acc_hit, int n_areas,
                                 int n_events, int n_slots, int members, double* area_prob, int st_slots, void* stream);
+
+// Event onset (roadsurf_ensemble_onset) of the first n_slots slots of member_out [..][mo_slots][ldm].  Per (station,
+// event, member): X, the first slot where a named plane is invalid (n_slots if none), and O, the first slot before X
+// where the conditions all hold (n_slots if none).  onset [n_events][st_slots][ld] (slots >= n_slots are not
+// written) and ws [n_events][npoints * members] {O, X} int pairs are each written where not null.
+int rs_launch_ens_onset(const double* member_out, int n_slots, int mo_slots, int ldm, int npoints, int members,
+                        const RsEnsembleStatsSpec* spec, double* onset, int st_slots, int ld, int* ws, void* stream);
+// Area onset: the minimum {O, X} over each segment's stations (as for rs_launch_ens_area_accumulate; station p at
+// ws lane (p - p0) * members + m) into acc [n_areas][n_events][members] {O, X}, set to INT_MAX-like values (bytes
+// 0x7f) before the first chunk; then area_onset [n_events][st_slots][n_areas] from acc.
+int rs_launch_ens_area_onset_accumulate(const int* ws, int npoints, int members, int n_events, const int* stations, int p0,
+                                        const int* segments, int n_segments, int* acc, void* stream);
+int rs_launch_ens_area_onset_finalize(const int* acc, int n_areas, int n_events, int n_slots, int members,
+                                      double* area_onset, int st_slots, void* stream);

@@ -47,7 +47,8 @@ enum PoolSlot : int
   EH_FORCING = 400, EH_LOCAL = 401, EH_HOR = 402, EH_OUT = 403, EH_STATE = 404, EH_SCRATCH = 405, EH_M_FORCING = 406,
   EH_M_LOCAL = 407, EH_M_HOR = 408, EH_M_STATE = 409, EH_M_SCRATCH = 410, EH_M_OUT = 411, EH_RELAX = 412,
   EH_STATS = 413, EH_PROB = 414, EH_SOLAR = 415, EH_STATUS = 416, EH_M_STATUS = 417, EH_TIME_FIELDS = 418,
-  EH_RECORD_STEP = 419, EH_COUNTERS = 420, EH_AREAS = 421, EH_AREA_PROB = 422,
+  EH_RECORD_STEP = 419, EH_COUNTERS = 420, EH_AREAS = 421, EH_AREA_PROB = 422, EH_ONSET = 423, EH_ONSET_WS = 424,
+  EH_ONSET_ACC = 425, EH_AREA_ONSET = 426,
   EH_H_RELAX = 400,  // pinned
 };
 
@@ -1593,7 +1594,7 @@ void roadsurf_session_close(void* session)
 
 const char* roadsurf_last_error(void) { return g_err.c_str(); }
 
-const char* roadsurf_version(void) { return "roadsurf_b200 0.3 (RoadSurf 1.6.1 per-point loop, sm_100a)"; }
+const char* roadsurf_version(void) { return "roadsurf_b200 0.4 (RoadSurf 1.6.1 per-point loop, sm_100a)"; }
 
 int roadsurf_device_count(void)
 {
@@ -2373,6 +2374,60 @@ int area_finalize(const AreaDevice& d, int n_areas, int n_events, int n_slots, i
   return RS_OK;
 }
 
+// ---- event onset (roadsurf_ensemble_onset) ----
+// Which outputs may go together, before any device work.  `device`: roadsurf_ensemble_onset, which has no area_prob
+// and needs one output at least.
+int check_onset_outputs(const RsEnsembleStatsSpec& spec, const double* onset, const RsEnsembleAreas* areas,
+                        const double* area_prob, const double* area_onset, bool device)
+{
+  if (device && !onset && !area_onset) return fail(RS_ERR_BAD_ARGUMENT, "onset and area_onset are both NULL");
+  if ((onset || area_onset) && spec.n_events == 0)
+    return fail(RS_ERR_BAD_ARGUMENT, "event onset needs at least one event in the spec");
+  if (!areas && (area_prob || area_onset))
+    return fail(RS_ERR_BAD_ARGUMENT, "null area pointer: area_prob and area_onset need areas");
+  if (areas && !area_prob && !area_onset)
+    return fail(RS_ERR_BAD_ARGUMENT, device ? "null area pointer: areas need area_onset"
+                                            : "null area pointer: areas need area_prob or area_onset");
+  return RS_OK;
+}
+
+// Area onset accumulators [n_areas][n_events][members] {O, X}, in ints.
+size_t onset_acc_ints(int n_areas, int n_events, int members)
+{
+  return 2 * static_cast<size_t>(n_areas) * n_events * members;
+}
+
+int onset_launch(const double* member_out, int n_slots, int mo_slots, int ldm, int npoints, int members,
+                 const RsEnsembleStatsSpec* spec, double* onset, int st_slots, int ld, int* ws, cudaStream_t st)
+{
+  if (n_slots == 0 || npoints == 0 || (!onset && !ws)) return RS_OK;
+  CU(static_cast<cudaError_t>(
+      rs_launch_ens_onset(member_out, n_slots, mo_slots, ldm, npoints, members, spec, onset, st_slots, ld, ws, st)));
+  ++g_launches_total;
+  return RS_OK;
+}
+
+int onset_area_accumulate(const AreaDevice& d, const int* ws, int npoints, int members, int n_events, int p0,
+                          int first_segment, int n_segments, int* acc, cudaStream_t st)
+{
+  if (n_segments == 0) return RS_OK;
+  CU(static_cast<cudaError_t>(rs_launch_ens_area_onset_accumulate(
+      ws, npoints, members, n_events, d.stations, p0, d.segments + 4 * static_cast<size_t>(first_segment), n_segments,
+      acc, st)));
+  ++g_launches_total;
+  return RS_OK;
+}
+
+int onset_area_finalize(const int* acc, int n_areas, int n_events, int n_slots, int members, double* area_onset,
+                        int st_slots, cudaStream_t st)
+{
+  if (n_slots == 0) return RS_OK;
+  CU(static_cast<cudaError_t>(
+      rs_launch_ens_area_onset_finalize(acc, n_areas, n_events, n_slots, members, area_onset, st_slots, st)));
+  ++g_launches_total;
+  return RS_OK;
+}
+
 // Where the fork may sit (pure host checks).  record_step: host copy (forcing_mode 1) or null.
 int check_fork(int forcing_mode, int sim_len, int fork_step, int members, const int* record_step, int n_records, int* r_f)
 {
@@ -2440,6 +2495,47 @@ int roadsurf_ensemble_area_events(const double* member_out, int out_nvar, int n_
   int rc = area_upload(pl, spec->n_events, n_out, members, buf, st, &d, &h2d);
   if (rc == RS_OK) rc = area_accumulate(d, member_out, n_out, n_out, ld_members, members, spec, 0, 0, n_segments, st);
   if (rc == RS_OK) rc = area_finalize(d, pl.n_areas, spec->n_events, n_out, members, area_prob, n_out, st);
+  const cudaError_t e = cudaFreeAsync(buf, st);
+  if (rc == RS_OK && e != cudaSuccess) return fail(RS_ERR_CUDA, std::string("cudaFreeAsync: ") + cudaGetErrorString(e));
+  return rc;
+}
+
+int roadsurf_ensemble_onset(const double* member_out, int out_nvar, int n_out, int ld_members, int npoints, int members,
+                            const RsEnsembleStatsSpec* spec, double* onset, int ld, const RsEnsembleAreas* areas,
+                            double* area_onset, void* stream)
+{
+  if (!member_out || !spec || members < 1 || members > RS_ENS_MAX_MEMBERS || npoints < 0 || n_out < 0 ||
+      (out_nvar != RS_O_NVAR && out_nvar != RS_O_NVAR_EXT) || (onset && ld < npoints) ||
+      static_cast<long long>(ld_members) < static_cast<long long>(npoints) * members)
+    return fail(RS_ERR_BAD_ARGUMENT, "bad arguments");
+  {
+    int rc = check_stats_spec(*spec, out_nvar);
+    if (rc == RS_OK) rc = check_onset_outputs(*spec, onset, areas, nullptr, area_onset, true);
+    if (rc == RS_OK && areas) rc = check_areas(areas, npoints, *spec);
+    if (rc != RS_OK) return rc;
+  }
+  if (n_out == 0) return RS_OK;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int E = spec->n_events;
+  if (!areas) return onset_launch(member_out, n_out, n_out, ld_members, npoints, members, spec, onset, n_out, ld, nullptr, st);
+  // one buffer: the plan (segments, stations; no area event accumulators), the accumulators, the workspace
+  AreaPlan pl = plan_areas(*areas);
+  const int n_segments = plan_segments(pl, 0, npoints, area_segment_length(pl, E, n_out, 1));
+  const size_t plan_bytes = (area_bytes(pl, 0, n_out, members, n_segments) + 15) / 16 * 16;
+  const size_t acc_ints = onset_acc_ints(pl.n_areas, E, members);
+  const size_t ws_ints = 2 * static_cast<size_t>(E) * npoints * members;
+  void* buf = nullptr;
+  CU(cudaMallocAsync(&buf, plan_bytes + sizeof(int) * (acc_ints + ws_ints), st));
+  int* acc = reinterpret_cast<int*>(static_cast<char*>(buf) + plan_bytes);
+  int* ws = acc + acc_ints;
+  AreaDevice d;
+  size_t h2d = 0;
+  int rc = area_upload(pl, 0, n_out, members, buf, st, &d, &h2d);
+  if (rc == RS_OK && cudaMemsetAsync(acc, 0x7f, sizeof(int) * acc_ints, st) != cudaSuccess)
+    rc = fail(RS_ERR_CUDA, "cudaMemsetAsync of the area onset accumulators");
+  if (rc == RS_OK) rc = onset_launch(member_out, n_out, n_out, ld_members, npoints, members, spec, onset, n_out, ld, ws, st);
+  if (rc == RS_OK) rc = onset_area_accumulate(d, ws, npoints, members, E, 0, 0, n_segments, acc, st);
+  if (rc == RS_OK) rc = onset_area_finalize(acc, pl.n_areas, E, n_out, members, area_onset, n_out, st);
   const cudaError_t e = cudaFreeAsync(buf, st);
   if (rc == RS_OK && e != cudaSuccess) return fail(RS_ERR_CUDA, std::string("cudaFreeAsync: ") + cudaGetErrorString(e));
   return rc;
@@ -2608,6 +2704,17 @@ int roadsurf_run_ensemble_host_soa_areas(const RsHostBatch* b, const double* mem
                                          double* prob, double* member_out, int* member_status, const RsEnsembleAreas* areas,
                                          double* area_prob, const InputSettings* settings, const InputParameters* params)
 {
+  return roadsurf_run_ensemble_host_soa_onset(b, member_records, members, fork_step, latest_obs_index, spec, stats, prob,
+                                              member_out, member_status, areas, area_prob, nullptr, nullptr, settings,
+                                              params);
+}
+
+int roadsurf_run_ensemble_host_soa_onset(const RsHostBatch* b, const double* member_records, int members, int fork_step,
+                                         const int* latest_obs_index, const RsEnsembleStatsSpec* spec, double* stats,
+                                         double* prob, double* member_out, int* member_status, const RsEnsembleAreas* areas,
+                                         double* area_prob, double* onset, double* area_onset,
+                                         const InputSettings* settings, const InputParameters* params)
+{
   g_err.clear();
   std::memset(&g_stats, 0, sizeof g_stats);
   const double wall0 = now_ms();
@@ -2632,11 +2739,9 @@ int roadsurf_run_ensemble_host_soa_areas(const RsHostBatch* b, const double* mem
     const int rc = check_stats_spec(*spec, RS_O_NVAR);
     if (rc != RS_OK) return rc;
   }
-  if ((areas == nullptr) != (area_prob == nullptr))
-    return fail(RS_ERR_BAD_ARGUMENT, "null area pointer: areas and area_prob go together");
-  if (areas)
   {
-    const int rc = check_areas(areas, P, *spec);
+    int rc = check_onset_outputs(*spec, onset, areas, area_prob, area_onset, false);
+    if (rc == RS_OK && areas) rc = check_areas(areas, P, *spec);
     if (rc != RS_OK) return rc;
   }
   if (P > 0 && !member_records) return fail(RS_ERR_BAD_ARGUMENT, "null member_records");
@@ -2704,22 +2809,31 @@ int roadsurf_run_ensemble_host_soa_areas(const RsHostBatch* b, const double* mem
   const size_t frows = static_cast<size_t>(nrec) * nvar, frows_m = static_cast<size_t>(nrec_m + 1) * nvar;
   const size_t NS = RS_STATE_NPLANES(nl), SC = RS_SCRATCH_NPLANES(nl);
   const size_t srows = static_cast<size_t>(RS_ENS_NFIXED + nq) * RS_O_NVAR * n_m, prows = static_cast<size_t>(np_planes) * n_m;
+  const int E = spec->n_events;
+  const size_t orows = onset ? static_cast<size_t>(E) * n_m : 0;  // onset planes of a station
+  // area onset: the workspace {O, X} of every member lane, E * 8 bytes
   const size_t per_station =
-      sizeof(double) * (frows + RS_L_NLOCAL + (hor ? 360 : 0) + RS_O_NVAR * n_pre + NS + (cpl ? SC : 0) + 1 + srows + prows) +
-      sizeof(double) * M * (frows_m + RS_L_NLOCAL + (hor ? 360 : 0) + NS + (cpl ? SC : 0) + 1 + 3 + RS_O_NVAR * n_m);
+      sizeof(double) * (frows + RS_L_NLOCAL + (hor ? 360 : 0) + RS_O_NVAR * n_pre + NS + (cpl ? SC : 0) + 1 + srows + prows +
+                        orows) +
+      sizeof(double) * M * (frows_m + RS_L_NLOCAL + (hor ? 360 : 0) + NS + (cpl ? SC : 0) + 1 + 3 + RS_O_NVAR * n_m +
+                            (area_onset ? E : 0));
   size_t free_b = 0, total_b = 0;
   CU(cudaMemGetInfo(&free_b, &total_b));
-  // areas: the plan and the accumulators stay on the device for the whole call, beside area_prob
+  // areas: the plan and the accumulators stay on the device for the whole call, beside area_prob and area_onset (the
+  // area event accumulators only where area_prob is asked for)
   AreaPlan area_plan;
-  const int E = spec->n_events;
+  const int E_prob = area_prob ? E : 0;
   size_t area_fixed = 0;
   if (areas)
   {
     area_plan = plan_areas(*areas);
-    area_fixed = area_bytes(area_plan, E, n_m, M, area_plan.stations.size()) + sizeof(double) * E * n_m * areas->n_areas;
+    area_fixed = area_bytes(area_plan, E_prob, n_m, M, area_plan.stations.size()) +
+                 sizeof(double) * E * n_m * areas->n_areas * ((area_prob ? 1 : 0) + (area_onset ? 1 : 0)) +
+                 (area_onset ? sizeof(int) * onset_acc_ints(areas->n_areas, E, M) : 0);
     if (static_cast<double>(area_fixed) >= free_b * 0.8)
-      return fail(RS_ERR_CUDA, "not enough device memory for the area accumulators (2 * n_areas * n_events * "
-                               "ceil(n_out_m / 64) * members * 8 bytes) and area_prob");
+      return fail(RS_ERR_CUDA, "not enough device memory for the area accumulators (area_prob: 2 * n_areas * n_events * "
+                               "ceil(n_out_m / 64) * members * 8 bytes; area_onset: n_areas * n_events * members * 8 "
+                               "bytes) and the area outputs");
   }
   long long pc = static_cast<long long>((free_b * 0.8 - static_cast<double>(area_fixed)) / per_station) - 64;
   if (const int cap = g_opt_max_slots.load()) pc = std::min<long long>(pc, std::max(1, cap / M));
@@ -2779,12 +2893,23 @@ int roadsurf_run_ensemble_host_soa_areas(const RsHostBatch* b, const double* mem
   if (areas)
   {
     unsigned long long* buf;
-    CU(pooled(dev, EH_AREAS, (area_bytes(area_plan, E, n_m, M, area_plan.segments.size() / 4) + 7) / 8, &buf));
-    CU(pooled(dev, EH_AREA_PROB, std::max<size_t>(1, area_prob_n), &d_area_prob));
+    CU(pooled(dev, EH_AREAS, (area_bytes(area_plan, E_prob, n_m, M, area_plan.segments.size() / 4) + 7) / 8, &buf));
+    if (area_prob) CU(pooled(dev, EH_AREA_PROB, std::max<size_t>(1, area_prob_n), &d_area_prob));
     size_t h2d = 0;
-    const int rc = area_upload(area_plan, E, n_m, M, buf, st, &d_areas, &h2d);
+    const int rc = area_upload(area_plan, E_prob, n_m, M, buf, st, &d_areas, &h2d);
     if (rc != RS_OK) return rc;
     g_stats.h2d_bytes += h2d;
+  }
+  double *d_onset = nullptr, *d_area_onset = nullptr;
+  int *d_ws = nullptr, *d_onset_acc = nullptr;
+  if (onset) CU(pooled(dev, EH_ONSET, std::max<size_t>(1, orows * lc), &d_onset));
+  if (area_onset)
+  {
+    const size_t acc_ints = onset_acc_ints(areas->n_areas, E, M);
+    CU(pooled(dev, EH_ONSET_WS, 2 * static_cast<size_t>(E) * lm, &d_ws));
+    CU(pooled(dev, EH_ONSET_ACC, acc_ints, &d_onset_acc));
+    CU(pooled(dev, EH_AREA_ONSET, std::max<size_t>(1, area_prob_n), &d_area_onset));
+    CU(cudaMemsetAsync(d_onset_acc, 0x7f, sizeof(int) * acc_ints, st));
   }
   g_stats.setup_ms = now_ms() - setup0;
   const int launches0 = g_launches_total.load();
@@ -2849,11 +2974,20 @@ int roadsurf_run_ensemble_host_soa_areas(const RsHostBatch* b, const double* mem
     }
     const long long chunk = p0 / pc;
     const bool last = p0 + pc >= P;
-    if (areas)
+    if (area_prob)
     {
       int rc = area_accumulate(d_areas, d_mo, n_m, e.n_out_members, ldm, M, spec, static_cast<int>(p0),
                                chunk_segments[chunk], chunk_segments[chunk + 1] - chunk_segments[chunk], st);
       if (rc == RS_OK && last) rc = area_finalize(d_areas, areas->n_areas, E, n_m, M, d_area_prob, n_m, st);
+      if (rc != RS_OK) return rc;
+    }
+    {
+      int rc = onset_launch(d_mo, n_m, e.n_out_members, ldm, n, M, spec, d_onset, n_m, ld, d_ws, st);
+      if (rc == RS_OK && area_onset)
+        rc = onset_area_accumulate(d_areas, d_ws, n, M, E, static_cast<int>(p0), chunk_segments[chunk],
+                                   chunk_segments[chunk + 1] - chunk_segments[chunk], d_onset_acc, st);
+      if (rc == RS_OK && area_onset && last)
+        rc = onset_area_finalize(d_onset_acc, areas->n_areas, E, n_m, M, d_area_onset, n_m, st);
       if (rc != RS_OK) return rc;
     }
     CU(cudaEventRecord(ev[2], st));
@@ -2870,9 +3004,19 @@ int roadsurf_run_ensemble_host_soa_areas(const RsHostBatch* b, const double* mem
       CU(cudaMemcpyAsync(member_status + colm, d_mstatus, sizeof(int) * nm, cudaMemcpyDeviceToHost, st));
     g_stats.d2h_bytes += D * (n * ((b->out ? RS_O_NVAR * (pre1 - pre0) : 0) + (stats ? srows : 0) + (prob ? prows : 0)) +
                               (member_out ? nm * RS_O_NVAR * n_m : 0)) + (member_status ? sizeof(int) * nm : 0);
-    if (areas && last && area_prob_n > 0)
+    if (onset && n_m > 0)
+    {
+      CU(cudaMemcpy2DAsync(onset + col, D * np, d_onset, D * ld, D * n, orows, cudaMemcpyDeviceToHost, st));
+      g_stats.d2h_bytes += D * n * orows;
+    }
+    if (area_prob && last && area_prob_n > 0)
     {
       CU(cudaMemcpyAsync(area_prob, d_area_prob, D * area_prob_n, cudaMemcpyDeviceToHost, st));
+      g_stats.d2h_bytes += D * area_prob_n;
+    }
+    if (area_onset && last && area_prob_n > 0)
+    {
+      CU(cudaMemcpyAsync(area_onset, d_area_onset, D * area_prob_n, cudaMemcpyDeviceToHost, st));
       g_stats.d2h_bytes += D * area_prob_n;
     }
     CU(cudaEventRecord(ev[3], st));

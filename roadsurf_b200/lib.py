@@ -41,7 +41,8 @@ EXPORTS = ("runsimulation", "roadsurf_last_error", "roadsurf_device_count", "roa
            "roadsurf_sun_position", "roadsurf_eval_primitive",
            "roadsurf_version",
            "roadsurf_run_ensemble_device", "roadsurf_ensemble_stats", "roadsurf_run_ensemble_host_soa",
-           "roadsurf_ensemble_area_events", "roadsurf_run_ensemble_host_soa_areas")
+           "roadsurf_ensemble_area_events", "roadsurf_run_ensemble_host_soa_areas",
+           "roadsurf_ensemble_onset", "roadsurf_run_ensemble_host_soa_onset")
 (PRIM_EXP, PRIM_EXP_SMEM, PRIM_LOG, PRIM_LOG_SMEM, PRIM_EXP_FLAT, PRIM_EXP_FLAT_SMEM, PRIM_PSIH_UNSTABLE,
  PRIM_PSIH_UNSTABLE_SMEM, PRIM_FRCP, PRIM_FDIV, PRIM_DIV_CONST, PRIM_N) = range(12)
 ENS_MAX_MEMBERS, ENS_MAX_QUANTILES, ENS_MAX_THRESHOLDS = 128, 8, 8
@@ -240,6 +241,15 @@ def load():
                                                          P(RsEnsembleStatsSpec), C.c_void_p, C.c_void_p, C.c_void_p,
                                                          C.c_void_p, P(RsEnsembleAreas), C.c_void_p, P(IS), P(IPa)]
     lib.roadsurf_run_ensemble_host_soa_areas.restype = C.c_int
+    lib.roadsurf_ensemble_onset.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                                            P(RsEnsembleStatsSpec), C.c_void_p, C.c_int, P(RsEnsembleAreas),
+                                            C.c_void_p, C.c_void_p]
+    lib.roadsurf_ensemble_onset.restype = C.c_int
+    lib.roadsurf_run_ensemble_host_soa_onset.argtypes = [P(RsHostBatch), C.c_void_p, C.c_int, C.c_int, C.c_void_p,
+                                                         P(RsEnsembleStatsSpec), C.c_void_p, C.c_void_p, C.c_void_p,
+                                                         C.c_void_p, P(RsEnsembleAreas), C.c_void_p, C.c_void_p,
+                                                         C.c_void_p, P(IS), P(IPa)]
+    lib.roadsurf_run_ensemble_host_soa_onset.restype = C.c_int
     _lib = lib
     return lib
 
@@ -682,6 +692,26 @@ def ensemble_area_events(member_out, npoints, members, spec, areas, stream=None)
     return area_prob
 
 
+def ensemble_onset(member_out, npoints, members, spec, areas=None, onset=True, stream=None):
+    """roadsurf_ensemble_onset on a torch CUDA tensor member_out [out_nvar, n_out, ld_members] (lane
+    p * members + m); areas is an RsEnsembleAreas (ensemble_areas) or None.  Returns (onset [n_events, n_out, npoints]
+    or None when onset=False, area_onset [n_events, n_out, n_areas] or None without areas) as CUDA tensors
+    (synchronised)."""
+    import torch
+    out_nvar, n_out, ldm = member_out.shape
+    ld = max(32, (npoints + 31) // 32 * 32)
+    f64 = dict(dtype=torch.float64, device=member_out.device)
+    on = torch.full((spec.n_events, n_out, ld), 12345.0, **f64) if onset else None
+    area_on = torch.full((spec.n_events, n_out, areas.n_areas), 12345.0, **f64) if areas is not None else None
+    st = stream if stream is not None else torch.cuda.current_stream()
+    _check(load().roadsurf_ensemble_onset(member_out.data_ptr(), out_nvar, n_out, ldm, int(npoints), int(members),
+                                          C.byref(spec), None if on is None else on.data_ptr(), ld,
+                                          None if areas is None else C.byref(areas),
+                                          None if area_on is None else area_on.data_ptr(), C.c_void_p(st.cuda_stream)))
+    torch.cuda.synchronize()
+    return (None if on is None else on[..., :npoints]), area_on
+
+
 def fork_record(record_step, fork_step):
     """r_f: the last record at or before 0-based step fork_step - 1."""
     rs = np.asarray(record_step)
@@ -805,13 +835,15 @@ class EnsembleBatch:
 
 def run_ensemble_host_soa(settings, params, forcing, record_step, time_fields, local, member_records, members,
                           fork_step, spec, horizons=None, out_stride=1, coupling_window_end=0, out=None,
-                          member_out=False, member_status=False, latest_obs_index=None, areas=None, prob=True):
-    """roadsurf_run_ensemble_host_soa_areas on host arrays: forcing [n_records, nvar, P], record_step [n_records],
+                          member_out=False, member_status=False, latest_obs_index=None, areas=None, prob=True,
+                          onset=False, area_prob=True):
+    """roadsurf_run_ensemble_host_soa_onset on host arrays: forcing [n_records, nvar, P], record_step [n_records],
     local [L_NLOCAL, P], member_records [n_records - r_f - 1, nvar, P * members], latest_obs_index [P] int32 (the
     relaxation rule of read_input_derive_records; None = no observations), areas an RsEnsembleAreas (ensemble_areas)
     or None.  Returns a dict with stats [5 + nq, 6, n_out_m, P], prob [nt + n_events, n_out_m, P] (unless prob=False:
     NULL is passed) and, when asked for, member_out [6, n_out_m, P * M], member_status [P * M] and area_prob
-    [n_events, n_out_m, n_areas]."""
+    [n_events, n_out_m, n_areas] (unless area_prob=False: NULL is passed).  With onset=True it also returns
+    onset [n_events, n_out_m, P] and, with areas, area_onset [n_events, n_out_m, n_areas]."""
     n_records, nvar, npoints = forcing.shape
     sim_len = time_fields.shape[1]
     k0 = fork_step - 1
@@ -824,15 +856,20 @@ def run_ensemble_host_soa(settings, params, forcing, record_step, time_fields, l
         res["member_out"] = np.zeros((O_NVAR, n_m, npoints * members))
     if member_status:
         res["member_status"] = np.zeros(npoints * members, dtype=np.int32)
-    if areas is not None:
+    if areas is not None and area_prob:
         res["area_prob"] = np.zeros((spec.n_events, n_m, areas.n_areas))
+    if onset:
+        res["onset"] = np.zeros((spec.n_events, n_m, npoints))
+        if areas is not None:
+            res["area_onset"] = np.zeros((spec.n_events, n_m, areas.n_areas))
     hb = RsHostBatch(npoints=npoints, sim_len=sim_len, forcing_mode=1, n_records=n_records, nvar=nvar,
                      out_stride=out_stride, forcing=_ptr(forcing), record_step=_ptr(record_step),
                      time_fields=_ptr(time_fields), local=_ptr(local), horizons=_ptr(horizons), out=_ptr(out),
                      coupling_window_end=int(coupling_window_end))
     lat = None if latest_obs_index is None else np.ascontiguousarray(latest_obs_index, dtype=np.int32)
-    _check(load().roadsurf_run_ensemble_host_soa_areas(
+    _check(load().roadsurf_run_ensemble_host_soa_onset(
         C.byref(hb), _ptr(member_records), int(members), int(fork_step), _ptr(lat), C.byref(spec), _ptr(res["stats"]),
         _ptr(res.get("prob")), _ptr(res.get("member_out")), _ptr(res.get("member_status")),
-        None if areas is None else C.byref(areas), _ptr(res.get("area_prob")), C.byref(settings), C.byref(params)))
+        None if areas is None else C.byref(areas), _ptr(res.get("area_prob")), _ptr(res.get("onset")),
+        _ptr(res.get("area_onset")), C.byref(settings), C.byref(params)))
     return res
