@@ -744,6 +744,48 @@ typedef struct RsEnsembleAreas
  * with s, so the lead time by which a fraction q of the members have seen the event is the first s with
  * onset >= q. */
 
+/* Window extremes: statistics of each member's minimum or maximum of one plane over a window of member slots, per
+ * station and per area ("how cold will the road get tonight?": the forecast minimum road-surface temperature over the
+ * night, or the maximum ice storage over the next hours).  An extreme is {plane, kind, window}.  For station p,
+ * extreme x, member m and member slot s < S (the slots the statistics cover):
+ *   - valid: the plane holds a valid value (value == value and > -9000) at every slot of
+ *     W(s) = [s, min(s + window, S) - 1], RsEnsembleEvent's window, truncated at the last member slot, not padded;
+ *   - value: the minimum (RS_ENS_WMIN) or maximum (RS_ENS_WMAX) of the plane over W(s) in the total order of the
+ *     order-preserving map of a double's bits b (as int64) to b >= 0 ? b : b ^ 0x7fffffffffffffff, so that -0.0 lies
+ *     below +0.0 and the result does not depend on the order of evaluation;
+ *   - result: ext_stats[j][x][s][p] holds the statistics of RsEnsembleStatsSpec (planes RS_ENS_NVALID, MEAN, STD, MIN
+ *     and MAX, then spec.n_quantiles quantile planes) over the valid members' values, with the definitions, member
+ *     order and operation order of `stats` and its -9999.0 / 0.0 convention where no member is valid.  The layout is
+ *     that of `stats` with the extremes in place of the output planes: [RS_ENS_NFIXED + n_quantiles][n_extremes]
+ *     [n_out][ld].  The spec's thresholds and events are ignored;
+ *   - areas (RsEnsembleAreas): a member is valid for area A at s when it is valid at every station of A, and its value
+ *     is the minimum (maximum) over A's stations of the station values in the same order; area_ext_stats[j][x][s][a],
+ *     [RS_ENS_NFIXED + n_quantiles][n_extremes][n_out][n_areas].
+ * Identities: (1) an extreme with window 1 equals the `stats` planes of its plane bit for bit; (2) an area of one
+ * station equals that station's values bit for bit, and neither repeated stations nor their order change an area's
+ * result; (3) the fraction of valid members whose window minimum is < v is the event probability of
+ * {plane, RS_ENS_LT, v} with the same window (area_prob for areas), and likewise the maximum with RS_ENS_GT. */
+#define RS_ENS_MAX_EXTREMES 8
+
+enum
+{
+  RS_ENS_WMIN = 0,
+  RS_ENS_WMAX = 1
+};
+
+typedef struct RsEnsembleExtreme
+{
+  int plane;  /* output plane (RS_O_*) */
+  int kind;   /* RS_ENS_WMIN / RS_ENS_WMAX */
+  int window; /* >= 1 output slots */
+} RsEnsembleExtreme;
+
+typedef struct RsEnsembleExtremes
+{
+  int n_extremes; /* 1 .. RS_ENS_MAX_EXTREMES */
+  RsEnsembleExtreme extremes[RS_ENS_MAX_EXTREMES];
+} RsEnsembleExtremes;
+
 /* A device-resident ensemble (DEVICE pointers on the current device). */
 typedef struct RsEnsembleBatch
 {
@@ -821,6 +863,23 @@ int roadsurf_ensemble_onset(const double* member_out, int out_nvar, int n_out, i
                             const RsEnsembleStatsSpec* spec, double* onset, int ld, const RsEnsembleAreas* areas,
                             double* area_onset, void* stream);
 
+/* Window extremes (defined after RsEnsembleAreas) over a station-major member tensor member_out
+ * [out_nvar][n_out][ld_members] (lane p * members + m), as for roadsurf_ensemble_stats: ext_stats DEVICE
+ * [RS_ENS_NFIXED + n_quantiles][n_extremes][n_out][ld] or NULL, area_ext_stats DEVICE
+ * [RS_ENS_NFIXED + n_quantiles][n_extremes][n_out][n_areas] or NULL (then areas must be NULL too); one of the two at
+ * least.  Only spec->n_quantiles and spec->quantiles are used (the spec is checked whole).  Extreme planes lie in
+ * [0, out_nvar).  The area arrays are host memory, checked and copied as for roadsurf_ensemble_area_events; a spec
+ * without events is accepted with areas.  Asynchronous on `stream`; it takes a work space with cudaMallocAsync and
+ * frees it with cudaFreeAsync on `stream`: n_extremes * n_out * ceil32(npoints * members) * 8 bytes, and with areas
+ * n_extremes * n_out * n_areas * members * 8 bytes more plus the area plan (about 20 bytes per area station).
+ *   roadsurf_run_ensemble_device(&e, stream);
+ *   roadsurf_ensemble_extremes(e.member_out, e.shared.out_nvar, e.n_out_members, e.ld_members, e.shared.npoints,
+ *                              e.members, &e.spec, &ext, d_ext_stats, e.shared.ld, &areas, d_area_ext_stats, stream); */
+int roadsurf_ensemble_extremes(const double* member_out, int out_nvar, int n_out, int ld_members, int npoints,
+                               int members, const RsEnsembleStatsSpec* spec, const RsEnsembleExtremes* ext,
+                               double* ext_stats, int ld, const RsEnsembleAreas* areas, double* area_ext_stats,
+                               void* stream);
+
 /* Host form on the current device, forcing_mode 1 only.  `shared` is the stations' host SoA batch
  * (as for roadsurf_run_host_soa, with the full record axis); its `out`, if not NULL, receives the
  * station outputs of the steps before F, [RS_O_NVAR][n_out_pre][P] with n_out_pre = ceil((F - 1) /
@@ -867,6 +926,24 @@ int roadsurf_run_ensemble_host_soa_onset(const RsHostBatch* shared, const double
                                          double* stats, double* prob, double* member_out, int* member_status,
                                          const RsEnsembleAreas* areas, double* area_prob, double* onset,
                                          double* area_onset, const InputSettings* settings, const InputParameters* params);
+
+/* roadsurf_run_ensemble_host_soa_onset plus window extremes (defined after RsEnsembleAreas): ext_stats HOST
+ * [RS_ENS_NFIXED + n_quantiles][n_extremes][n_out_m][P] and area_ext_stats HOST
+ * [RS_ENS_NFIXED + n_quantiles][n_extremes][n_out_m][n_areas], each NULL or not; ext goes with one of them at least,
+ * and either needs ext.  Extreme planes are the RS_O_NVAR model planes.  ext_stats is copied back after each station
+ * chunk, area_ext_stats once at the end (both counted in d2h_bytes; the extremes kernels in kernel_ms).  Areas may go
+ * with area_ext_stats alone, and then the spec needs no events.  With ext, ext_stats and area_ext_stats NULL it is
+ * exactly roadsurf_run_ensemble_host_soa_onset.  Device memory for the whole call, beside the area event and onset
+ * buffers: the area extreme accumulators, n_extremes * n_out_m * n_areas * members * 8 bytes, and area_ext_stats
+ * (RS_ERR_CUDA where they do not fit); per station chunk a work space of n_extremes * n_out_m * 8 bytes per member
+ * lane. */
+int roadsurf_run_ensemble_host_soa_extremes(const RsHostBatch* shared, const double* member_records, int members,
+                                            int fork_step, const int* latest_obs_index, const RsEnsembleStatsSpec* spec,
+                                            double* stats, double* prob, double* member_out, int* member_status,
+                                            const RsEnsembleAreas* areas, double* area_prob, double* onset,
+                                            double* area_onset, const RsEnsembleExtremes* ext, double* ext_stats,
+                                            double* area_ext_stats, const InputSettings* settings,
+                                            const InputParameters* params);
 
 #ifdef __cplusplus
 }

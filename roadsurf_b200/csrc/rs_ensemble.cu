@@ -1,6 +1,6 @@
 // rs_ensemble.cu -- the kernels of an ensemble run (roadsurf_run_ensemble_device): the prefix's copy of the
 // station statics, the fork of the station state into the member lanes, the ensemble statistics, the event
-// probabilities and the area event probabilities.
+// probabilities, the area event probabilities, the event onset and the window extremes.
 // Member lanes are station-major: lane = p * members + m.
 #include <cuda_runtime.h>
 
@@ -569,6 +569,117 @@ __global__ void __launch_bounds__(kRsAreaBlock) rs_ens_area_onset_finalize_kerne
   area_onset[(static_cast<size_t>(e) * st_slots + s) * n_areas + a] =
       n == 0 ? -9999.0 : static_cast<double>(count) / static_cast<double>(n);
 }
+
+// Window extremes (roadsurf_ensemble_extremes) compare keys: the header's order-preserving int64 map of a double's
+// bits with its sign bit flipped, an order-preserving map to uint64, so that -0.0 < +0.0.  An invalid value is the
+// absorbing element of the order (0 for the minimum, ~0 for the maximum) and the identity is the other end, so that
+// validity falls out of the same combine.  No valid value has either key (both are NaN bit patterns).
+__device__ __forceinline__ unsigned long long ext_key(double v, bool lo)
+{
+  if (!valid_value(v)) return lo ? 0ULL : ~0ULL;
+  const unsigned long long b = static_cast<unsigned long long>(__double_as_longlong(v));
+  return (b >> 63) ? ~b : b | (1ULL << 63);
+}
+
+__device__ __forceinline__ unsigned long long ext_combine(unsigned long long a, unsigned long long b, bool lo)
+{
+  return lo ? (b < a ? b : a) : (b > a ? b : a);
+}
+
+// The double of a key, as raw bits; -9999.0 for the absorbing element.
+__device__ __forceinline__ unsigned long long ext_bits(unsigned long long k, bool lo)
+{
+  if (k == (lo ? 0ULL : ~0ULL)) return static_cast<unsigned long long>(__double_as_longlong(-9999.0));
+  return (k >> 63) ? k & ~(1ULL << 63) : ~k;
+}
+
+constexpr int kExtBlock = 256;
+
+// Station window extremes: one thread per (extreme, member lane), blockIdx.y the extreme and the lanes fastest, so that
+// every warp access is one row of consecutive lanes.  Van Herk / Gil-Werman over blocks of w = min(window, S) slots:
+// a backward pass writes each slot's suffix extreme within its block into ws; a forward pass keeps the prefix extreme
+// of the current block and, at t = s + w - 1, combines it with the suffix of s (W(s) = s's suffix alone where s starts
+// a block) and writes the value of W(s); the windows cut at S combine with the prefix of the last block at the end.
+// Each member value is read twice and each ws value written twice and read once, whatever the window.
+__global__ void __launch_bounds__(kExtBlock) rs_ens_window_extremes_kernel(const double* __restrict__ mout, int n_slots,
+                                                                           int mo_slots, int ldm, int lanes,
+                                                                           const RsEnsembleExtremes ext,
+                                                                           unsigned long long* __restrict__ ws, int ldw)
+{
+  const int l = blockIdx.x * kExtBlock + threadIdx.x;
+  if (l >= lanes) return;
+  const RsEnsembleExtreme xt = ext.extremes[blockIdx.y];
+  const bool lo = xt.kind == RS_ENS_WMIN;
+  const int S = n_slots, w = min(xt.window, S);
+  const double* src = mout + static_cast<size_t>(xt.plane) * mo_slots * ldm + l;
+  unsigned long long* out = ws + static_cast<size_t>(blockIdx.y) * S * ldw + l;
+  const unsigned long long id = lo ? ~0ULL : 0ULL;
+  unsigned long long acc = id;
+  for (int t = S - 1; t >= 0; --t)
+  {
+    if (t % w == w - 1) acc = id;
+    acc = ext_combine(acc, ext_key(__ldg(src + static_cast<size_t>(t) * ldm), lo), lo);
+    out[static_cast<size_t>(t) * ldw] = acc;
+  }
+  acc = id;
+  for (int t = 0; t < S; ++t)
+  {
+    if (t % w == 0) acc = id;
+    acc = ext_combine(acc, ext_key(__ldg(src + static_cast<size_t>(t) * ldm), lo), lo);
+    const int s = t - w + 1;
+    if (s < 0) continue;
+    unsigned long long* o = out + static_cast<size_t>(s) * ldw;
+    *o = ext_bits(s % w == 0 ? *o : ext_combine(*o, acc, lo), lo);
+  }
+  const int last_block = (S - 1) / w * w;  // first slot of the last block
+  for (int s = max(0, S - w + 1); s < S; ++s)
+  {
+    unsigned long long* o = out + static_cast<size_t>(s) * ldw;
+    *o = ext_bits(s < last_block ? ext_combine(*o, acc, lo) : *o, lo);
+  }
+}
+
+// Area window extremes, step 1: the stations of one chunk into the accumulators.  A work item is one (segment,
+// extreme), the extreme varying fastest; a block holds blockDim.y items of 32 * ceil(M / 32) threads, one per member.
+// Per slot a thread combines its member's station extremes (ws, station p at lane (p - p0) * members + m) over the
+// segment in key space and makes one atomicMin (minimum) or atomicMax (maximum) into acc[x][s][area * members + m].
+// Both are exact whatever the order, so the result does not depend on chunks, segments or launch geometry.
+__global__ void __launch_bounds__(kRsAreaBlock) rs_ens_area_extremes_accumulate_kernel(
+    const double* __restrict__ ws, int n_slots, int ldw, int members, long long n_items, int n_extremes,
+    unsigned min_mask, const int* __restrict__ stations, int p0, const int4* __restrict__ segments, int n_areas,
+    unsigned long long* __restrict__ acc)
+{
+  const long long item = static_cast<long long>(blockIdx.x) * blockDim.y + threadIdx.y;
+  const int m = threadIdx.x;
+  if (item >= n_items || m >= members) return;
+  const int x = static_cast<int>(item % n_extremes);
+  const int4 seg = __ldg(segments + item / n_extremes);  // area, first and end index into `stations`
+  const bool lo = (min_mask >> x) & 1u;
+  const double* src = ws + static_cast<size_t>(x) * n_slots * ldw + m;
+  const size_t row = static_cast<size_t>(n_areas) * members;
+  unsigned long long* dst = acc + static_cast<size_t>(x) * n_slots * row + static_cast<size_t>(seg.x) * members + m;
+  for (int s = 0; s < n_slots; ++s)
+  {
+    unsigned long long v = lo ? ~0ULL : 0ULL;
+    for (int k = seg.y; k < seg.z; ++k)
+      v = ext_combine(v, ext_key(__ldg(src + static_cast<size_t>(s) * ldw + static_cast<size_t>(__ldg(stations + k) - p0) * members), lo), lo);
+    if (lo)
+      atomicMin(dst + s * row, v);
+    else
+      atomicMax(dst + s * row, v);
+  }
+}
+
+// Area window extremes, step 2, once after the last chunk: the keys of acc [n_extremes][per_extreme] back to doubles
+// in place, -9999.0 where a member is not valid for the area.
+__global__ void __launch_bounds__(kRsAreaBlock) rs_ens_area_extremes_finalize_kernel(unsigned long long* __restrict__ acc,
+                                                                                     long long per_extreme,
+                                                                                     int n_extremes, unsigned min_mask)
+{
+  const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i >= per_extreme * n_extremes) return;
+  acc[i] = ext_bits(acc[i], (min_mask >> (i / per_extreme)) & 1u);
+}
 }  // namespace
 
 int rs_launch_ens_prefix_local(const double* local, int ld, int npoints, const double* member_relax, int ldm,
@@ -692,4 +803,63 @@ int rs_launch_ens_area_onset_finalize(const int* acc, int n_areas, int n_events,
                                       static_cast<cudaStream_t>(stream)>>>(acc, n_areas, n_events, n_slots, members,
                                                                            area_onset, st_slots);
   return static_cast<int>(cudaGetLastError());
+}
+
+// Bit x set where extreme x is a minimum.
+static unsigned min_mask(const RsEnsembleExtremes* ext)
+{
+  unsigned m = 0;
+  for (int x = 0; x < ext->n_extremes; ++x) m |= (ext->extremes[x].kind == RS_ENS_WMIN ? 1u : 0u) << x;
+  return m;
+}
+
+int rs_launch_ens_window_extremes(const double* member_out, int n_slots, int mo_slots, int ldm, int lanes,
+                                  const RsEnsembleExtremes* ext, double* ws, int ldw, void* stream)
+{
+  if (n_slots == 0 || lanes == 0) return 0;
+  const dim3 grid((lanes + kExtBlock - 1) / kExtBlock, ext->n_extremes);
+  rs_ens_window_extremes_kernel<<<grid, kExtBlock, 0, static_cast<cudaStream_t>(stream)>>>(
+      member_out, n_slots, mo_slots, ldm, lanes, *ext, reinterpret_cast<unsigned long long*>(ws), ldw);
+  return static_cast<int>(cudaGetLastError());
+}
+
+int rs_launch_ens_area_extremes_accumulate(const double* ws, int n_slots, int ldw, int members,
+                                           const RsEnsembleExtremes* ext, const int* stations, int p0,
+                                           const int* segments, int n_segments, int n_areas, double* acc, void* stream)
+{
+  if (n_segments == 0 || n_slots == 0) return 0;
+  const int groups = area_groups(members);
+  const long long items = static_cast<long long>(n_segments) * ext->n_extremes;
+  const dim3 block(32 * ((members + 31) / 32), groups);
+  rs_ens_area_extremes_accumulate_kernel<<<static_cast<unsigned>((items + groups - 1) / groups), block, 0,
+                                           static_cast<cudaStream_t>(stream)>>>(
+      ws, n_slots, ldw, members, items, ext->n_extremes, min_mask(ext), stations, p0, reinterpret_cast<const int4*>(segments), n_areas,
+      reinterpret_cast<unsigned long long*>(acc));
+  return static_cast<int>(cudaGetLastError());
+}
+
+int rs_launch_ens_area_extremes_finalize(double* acc, int n_slots, int n_areas, int members,
+                                         const RsEnsembleExtremes* ext, void* stream)
+{
+  const long long per_extreme = static_cast<long long>(n_slots) * n_areas * members;
+  if (per_extreme == 0) return 0;
+  const long long total = per_extreme * ext->n_extremes;
+  rs_ens_area_extremes_finalize_kernel<<<static_cast<unsigned>((total + kRsAreaBlock - 1) / kRsAreaBlock), kRsAreaBlock,
+                                         0, static_cast<cudaStream_t>(stream)>>>(
+      reinterpret_cast<unsigned long long*>(acc), per_extreme, ext->n_extremes, min_mask(ext));
+  return static_cast<int>(cudaGetLastError());
+}
+
+int rs_init_ens_area_extremes(double* acc, int n_slots, int n_areas, int members, const RsEnsembleExtremes* ext,
+                              void* stream)
+{
+  const size_t bytes = sizeof(double) * n_slots * n_areas * members;
+  for (int x = 0; x < ext->n_extremes; ++x)
+  {
+    const cudaError_t e = cudaMemsetAsync(reinterpret_cast<char*>(acc) + x * bytes,
+                                          ext->extremes[x].kind == RS_ENS_WMIN ? 0xff : 0, bytes,
+                                          static_cast<cudaStream_t>(stream));
+    if (e != cudaSuccess) return static_cast<int>(e);
+  }
+  return 0;
 }

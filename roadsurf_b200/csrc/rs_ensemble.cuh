@@ -75,3 +75,20 @@ int rs_launch_ens_area_onset_accumulate(const int* ws, int npoints, int members,
                                         const int* segments, int n_segments, int* acc, void* stream);
 int rs_launch_ens_area_onset_finalize(const int* acc, int n_areas, int n_events, int n_slots, int members,
                                       double* area_onset, int st_slots, void* stream);
+
+// Window extremes (roadsurf_ensemble_extremes) of the first n_slots slots of member_out [..][mo_slots][ldm], lanes
+// [0, lanes), into ws [n_extremes][n_slots][ldw] (-9999.0 where the window is not valid).  The extremes have been
+// checked.  The statistics of ws are rs_launch_ens_stats with out_nvar = n_extremes, mo_slots = n_slots and ldm = ldw.
+int rs_launch_ens_window_extremes(const double* member_out, int n_slots, int mo_slots, int ldm, int lanes,
+                                  const RsEnsembleExtremes* ext, double* ws, int ldw, void* stream);
+// Area window extremes: acc [n_extremes][n_slots][n_areas * members] keys, set to each extreme's identity by
+// rs_init_ens_area_extremes before the first chunk; each chunk's segments (as for rs_launch_ens_area_accumulate;
+// station p at ws lane (p - p0) * members + m) are combined into it; after the last chunk the finalize turns acc into
+// doubles in place, which rs_launch_ens_stats reads with npoints = n_areas, ldm = n_areas * members and ld = n_areas.
+int rs_init_ens_area_extremes(double* acc, int n_slots, int n_areas, int members, const RsEnsembleExtremes* ext,
+                              void* stream);
+int rs_launch_ens_area_extremes_accumulate(const double* ws, int n_slots, int ldw, int members,
+                                           const RsEnsembleExtremes* ext, const int* stations, int p0,
+                                           const int* segments, int n_segments, int n_areas, double* acc, void* stream);
+int rs_launch_ens_area_extremes_finalize(double* acc, int n_slots, int n_areas, int members,
+                                         const RsEnsembleExtremes* ext, void* stream);

@@ -48,7 +48,8 @@ enum PoolSlot : int
   EH_M_LOCAL = 407, EH_M_HOR = 408, EH_M_STATE = 409, EH_M_SCRATCH = 410, EH_M_OUT = 411, EH_RELAX = 412,
   EH_STATS = 413, EH_PROB = 414, EH_SOLAR = 415, EH_STATUS = 416, EH_M_STATUS = 417, EH_TIME_FIELDS = 418,
   EH_RECORD_STEP = 419, EH_COUNTERS = 420, EH_AREAS = 421, EH_AREA_PROB = 422, EH_ONSET = 423, EH_ONSET_WS = 424,
-  EH_ONSET_ACC = 425, EH_AREA_ONSET = 426,
+  EH_ONSET_ACC = 425, EH_AREA_ONSET = 426, EH_EXT_WS = 427, EH_EXT_STATS = 428, EH_EXT_ACC = 429,
+  EH_AREA_EXT_STATS = 430,
   EH_H_RELAX = 400,  // pinned
 };
 
@@ -2255,11 +2256,12 @@ int launch_stats_and_events(const double* member_out, int out_nvar, int n_slots,
 
 // ---- area event probabilities (RsEnsembleAreas) ----
 // Every index the area kernels use comes from here: the arrays are checked against npoints on the host.
-int check_areas(const RsEnsembleAreas* areas, int npoints, const RsEnsembleStatsSpec& spec)
+// `events`: an area event or onset output is asked for, so the spec needs events.
+int check_areas(const RsEnsembleAreas* areas, int npoints, const RsEnsembleStatsSpec& spec, bool events = true)
 {
   if (!areas || !areas->offsets || !areas->stations) return fail(RS_ERR_BAD_ARGUMENT, "null area pointer (areas, offsets or stations)");
   if (areas->n_areas < 1) return fail(RS_ERR_BAD_ARGUMENT, "n_areas must be at least 1");
-  if (spec.n_events == 0) return fail(RS_ERR_BAD_ARGUMENT, "area probabilities need at least one event in the spec");
+  if (events && spec.n_events == 0) return fail(RS_ERR_BAD_ARGUMENT, "area probabilities need at least one event in the spec");
   const int* o = areas->offsets;
   if (o[0] != 0) return fail(RS_ERR_BAD_ARGUMENT, "area offsets[0] must be 0");
   for (int a = 0; a < areas->n_areas; ++a)
@@ -2298,11 +2300,16 @@ AreaPlan plan_areas(const RsEnsembleAreas& a)
 
 // Stations per segment: enough segments that the accumulate kernel has about 2^15 work items (one warp each) per
 // chunk, so that a small ensemble spreads over the GPU, and no more, so that a large one makes few atomics and
-// reads a segment's member values in one pass; between 1 and 64.
+// reads a segment's member values in one pass; between 1 and 64.  `per_station`: the work items of one station.
+int segment_length(const AreaPlan& pl, long long per_station, long long chunks)
+{
+  const long long items = static_cast<long long>(pl.stations.size()) * per_station;
+  return static_cast<int>(std::min<long long>(64, std::max<long long>(1, items / (chunks << 15))));
+}
+
 int area_segment_length(const AreaPlan& pl, int n_events, int n_slots, long long chunks)
 {
-  const long long items = static_cast<long long>(pl.stations.size()) * n_events * rs_area_tiles(n_slots);
-  return static_cast<int>(std::min<long long>(64, std::max<long long>(1, items / (chunks << 15))));
+  return segment_length(pl, static_cast<long long>(n_events) * rs_area_tiles(n_slots), chunks);
 }
 
 // Appends the segments of the stations [p0, p0 + n), at most `len` stations each, and returns their count.
@@ -2376,16 +2383,17 @@ int area_finalize(const AreaDevice& d, int n_areas, int n_events, int n_slots, i
 
 // ---- event onset (roadsurf_ensemble_onset) ----
 // Which outputs may go together, before any device work.  `device`: roadsurf_ensemble_onset, which has no area_prob
-// and needs one output at least.
+// and needs one output at least.  Areas may go with area_ext_stats alone (host entry with window extremes).
 int check_onset_outputs(const RsEnsembleStatsSpec& spec, const double* onset, const RsEnsembleAreas* areas,
-                        const double* area_prob, const double* area_onset, bool device)
+                        const double* area_prob, const double* area_onset, bool device,
+                        const double* area_ext_stats = nullptr)
 {
   if (device && !onset && !area_onset) return fail(RS_ERR_BAD_ARGUMENT, "onset and area_onset are both NULL");
   if ((onset || area_onset) && spec.n_events == 0)
     return fail(RS_ERR_BAD_ARGUMENT, "event onset needs at least one event in the spec");
   if (!areas && (area_prob || area_onset))
     return fail(RS_ERR_BAD_ARGUMENT, "null area pointer: area_prob and area_onset need areas");
-  if (areas && !area_prob && !area_onset)
+  if (areas && !area_prob && !area_onset && !area_ext_stats)
     return fail(RS_ERR_BAD_ARGUMENT, device ? "null area pointer: areas need area_onset"
                                             : "null area pointer: areas need area_prob or area_onset");
   return RS_OK;
@@ -2425,6 +2433,83 @@ int onset_area_finalize(const int* acc, int n_areas, int n_events, int n_slots, 
   CU(static_cast<cudaError_t>(
       rs_launch_ens_area_onset_finalize(acc, n_areas, n_events, n_slots, members, area_onset, st_slots, st)));
   ++g_launches_total;
+  return RS_OK;
+}
+
+// ---- window extremes (roadsurf_ensemble_extremes) ----
+// Which outputs may go together and the extremes themselves, before any device work.  `device`:
+// roadsurf_ensemble_extremes, where areas go with area_ext_stats (the host entry's areas may serve other outputs).
+int check_extremes(const RsEnsembleExtremes* ext, const double* ext_stats, const RsEnsembleAreas* areas,
+                   const double* area_ext_stats, int out_nvar, bool device)
+{
+  if (!ext && (device || ext_stats || area_ext_stats))
+    return fail(RS_ERR_BAD_ARGUMENT, "null extremes pointer: ext_stats and area_ext_stats need ext");
+  if (!ext) return RS_OK;
+  if (!ext_stats && !area_ext_stats) return fail(RS_ERR_BAD_ARGUMENT, "ext_stats and area_ext_stats are both NULL");
+  if (area_ext_stats && !areas) return fail(RS_ERR_BAD_ARGUMENT, "null area pointer: area_ext_stats needs areas");
+  if (device && areas && !area_ext_stats) return fail(RS_ERR_BAD_ARGUMENT, "null area pointer: areas need area_ext_stats");
+  if (ext->n_extremes < 1 || ext->n_extremes > RS_ENS_MAX_EXTREMES)
+    return fail(RS_ERR_BAD_ARGUMENT, "an extremes set has 1 to 8 extremes");
+  for (int x = 0; x < ext->n_extremes; ++x)
+  {
+    const RsEnsembleExtreme& e = ext->extremes[x];
+    if (e.kind != RS_ENS_WMIN && e.kind != RS_ENS_WMAX)
+      return fail(RS_ERR_BAD_ARGUMENT, "unknown extreme kind (RS_ENS_WMIN or RS_ENS_WMAX)");
+    if (e.window < 1) return fail(RS_ERR_BAD_ARGUMENT, "an extreme window is at least 1 output slot");
+    if (e.plane < 0 || e.plane >= out_nvar) return fail(RS_ERR_BAD_ARGUMENT, "extreme plane outside the output planes");
+  }
+  return RS_OK;
+}
+
+// The statistics spec of window extremes: the quantiles of `spec`, no thresholds and no events.
+RsEnsembleStatsSpec extremes_spec(const RsEnsembleStatsSpec& spec)
+{
+  RsEnsembleStatsSpec s;
+  std::memset(&s, 0, sizeof s);
+  s.n_quantiles = spec.n_quantiles;
+  std::memcpy(s.quantiles, spec.quantiles, sizeof s.quantiles);
+  return s;
+}
+
+// The window kernel over the lanes of `npoints` stations into ws [n_extremes][n_slots][ldw], then, with ext_stats,
+// the statistics kernel on ws into ext_stats [..][n_extremes][st_slots][ld].
+int extremes_launch(const double* member_out, int n_slots, int mo_slots, int ldm, int npoints, int members,
+                    const RsEnsembleStatsSpec& xspec, const RsEnsembleExtremes* ext, double* ws, int ldw,
+                    double* ext_stats, int st_slots, int ld, cudaStream_t st)
+{
+  if (n_slots == 0 || npoints == 0) return RS_OK;
+  CU(static_cast<cudaError_t>(
+      rs_launch_ens_window_extremes(member_out, n_slots, mo_slots, ldm, npoints * members, ext, ws, ldw, st)));
+  ++g_launches_total;
+  if (!ext_stats) return RS_OK;
+  CU(static_cast<cudaError_t>(rs_launch_ens_stats(ws, ext->n_extremes, n_slots, n_slots, ldw, npoints, members, &xspec,
+                                                  ext_stats, nullptr, st_slots, ld, st)));
+  ++g_launches_total;
+  return RS_OK;
+}
+
+int extremes_area_accumulate(const AreaDevice& d, const double* ws, int n_slots, int ldw, int members,
+                             const RsEnsembleExtremes* ext, int p0, int first_segment, int n_segments, int n_areas,
+                             double* acc, cudaStream_t st)
+{
+  if (n_segments == 0 || n_slots == 0) return RS_OK;
+  CU(static_cast<cudaError_t>(rs_launch_ens_area_extremes_accumulate(
+      ws, n_slots, ldw, members, ext, d.stations, p0, d.segments + 4 * static_cast<size_t>(first_segment), n_segments,
+      n_areas, acc, st)));
+  ++g_launches_total;
+  return RS_OK;
+}
+
+// The finalize kernel, then the statistics kernel on the accumulators into area_ext_stats [..][n_extremes][st_slots]
+// [n_areas].
+int extremes_area_finalize(double* acc, int n_slots, int n_areas, int members, const RsEnsembleStatsSpec& xspec,
+                           const RsEnsembleExtremes* ext, double* area_ext_stats, int st_slots, cudaStream_t st)
+{
+  if (n_slots == 0) return RS_OK;
+  CU(static_cast<cudaError_t>(rs_launch_ens_area_extremes_finalize(acc, n_slots, n_areas, members, ext, st)));
+  CU(static_cast<cudaError_t>(rs_launch_ens_stats(acc, ext->n_extremes, n_slots, n_slots, n_areas * members, n_areas,
+                                                  members, &xspec, area_ext_stats, nullptr, st_slots, n_areas, st)));
+  g_launches_total += 2;
   return RS_OK;
 }
 
@@ -2536,6 +2621,62 @@ int roadsurf_ensemble_onset(const double* member_out, int out_nvar, int n_out, i
   if (rc == RS_OK) rc = onset_launch(member_out, n_out, n_out, ld_members, npoints, members, spec, onset, n_out, ld, ws, st);
   if (rc == RS_OK) rc = onset_area_accumulate(d, ws, npoints, members, E, 0, 0, n_segments, acc, st);
   if (rc == RS_OK) rc = onset_area_finalize(acc, pl.n_areas, E, n_out, members, area_onset, n_out, st);
+  const cudaError_t e = cudaFreeAsync(buf, st);
+  if (rc == RS_OK && e != cudaSuccess) return fail(RS_ERR_CUDA, std::string("cudaFreeAsync: ") + cudaGetErrorString(e));
+  return rc;
+}
+
+int roadsurf_ensemble_extremes(const double* member_out, int out_nvar, int n_out, int ld_members, int npoints,
+                               int members, const RsEnsembleStatsSpec* spec, const RsEnsembleExtremes* ext,
+                               double* ext_stats, int ld, const RsEnsembleAreas* areas, double* area_ext_stats,
+                               void* stream)
+{
+  if (!member_out || !spec || members < 1 || members > RS_ENS_MAX_MEMBERS || npoints < 0 || n_out < 0 ||
+      (out_nvar != RS_O_NVAR && out_nvar != RS_O_NVAR_EXT) || (ext_stats && ld < npoints) ||
+      static_cast<long long>(ld_members) < static_cast<long long>(npoints) * members)
+    return fail(RS_ERR_BAD_ARGUMENT, "bad arguments");
+  {
+    int rc = check_stats_spec(*spec, out_nvar);
+    if (rc == RS_OK) rc = check_extremes(ext, ext_stats, areas, area_ext_stats, out_nvar, true);
+    if (rc == RS_OK && areas) rc = check_areas(areas, npoints, *spec, false);
+    if (rc != RS_OK) return rc;
+  }
+  if (n_out == 0 || npoints == 0) return RS_OK;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const RsEnsembleStatsSpec xspec = extremes_spec(*spec);
+  const int X = ext->n_extremes, ldw = (npoints * members + 31) / 32 * 32;
+  // one buffer: the area plan (segments, stations; no area event accumulators), the area accumulators, the work space
+  AreaPlan pl;
+  int n_segments = 0;
+  size_t plan_bytes = 0, acc_n = 0;
+  if (areas)
+  {
+    pl = plan_areas(*areas);
+    n_segments = plan_segments(pl, 0, npoints, segment_length(pl, X, 1));
+    plan_bytes = (area_bytes(pl, 0, n_out, members, n_segments) + 15) / 16 * 16;
+    acc_n = static_cast<size_t>(X) * n_out * pl.n_areas * members;
+  }
+  const size_t ws_n = static_cast<size_t>(X) * n_out * ldw;
+  void* buf = nullptr;
+  CU(cudaMallocAsync(&buf, plan_bytes + sizeof(double) * (acc_n + ws_n), st));
+  double* acc = reinterpret_cast<double*>(static_cast<char*>(buf) + plan_bytes);
+  double* ws = acc + acc_n;
+  AreaDevice d;
+  int rc = RS_OK;
+  if (areas)
+  {
+    size_t h2d = 0;
+    rc = area_upload(pl, 0, n_out, members, buf, st, &d, &h2d);
+    if (rc == RS_OK && rs_init_ens_area_extremes(acc, n_out, pl.n_areas, members, ext, st) != 0)
+      rc = fail(RS_ERR_CUDA, "cudaMemsetAsync of the area extreme accumulators");
+  }
+  if (rc == RS_OK)
+    rc = extremes_launch(member_out, n_out, n_out, ld_members, npoints, members, xspec, ext, ws, ldw, ext_stats, n_out, ld,
+                         st);
+  if (rc == RS_OK && areas)
+    rc = extremes_area_accumulate(d, ws, n_out, ldw, members, ext, 0, 0, n_segments, pl.n_areas, acc, st);
+  if (rc == RS_OK && areas)
+    rc = extremes_area_finalize(acc, n_out, pl.n_areas, members, xspec, ext, area_ext_stats, n_out, st);
   const cudaError_t e = cudaFreeAsync(buf, st);
   if (rc == RS_OK && e != cudaSuccess) return fail(RS_ERR_CUDA, std::string("cudaFreeAsync: ") + cudaGetErrorString(e));
   return rc;
@@ -2715,6 +2856,19 @@ int roadsurf_run_ensemble_host_soa_onset(const RsHostBatch* b, const double* mem
                                          double* area_prob, double* onset, double* area_onset,
                                          const InputSettings* settings, const InputParameters* params)
 {
+  return roadsurf_run_ensemble_host_soa_extremes(b, member_records, members, fork_step, latest_obs_index, spec, stats,
+                                                 prob, member_out, member_status, areas, area_prob, onset, area_onset,
+                                                 nullptr, nullptr, nullptr, settings, params);
+}
+
+int roadsurf_run_ensemble_host_soa_extremes(const RsHostBatch* b, const double* member_records, int members,
+                                            int fork_step, const int* latest_obs_index, const RsEnsembleStatsSpec* spec,
+                                            double* stats, double* prob, double* member_out, int* member_status,
+                                            const RsEnsembleAreas* areas, double* area_prob, double* onset,
+                                            double* area_onset, const RsEnsembleExtremes* ext, double* ext_stats,
+                                            double* area_ext_stats, const InputSettings* settings,
+                                            const InputParameters* params)
+{
   g_err.clear();
   std::memset(&g_stats, 0, sizeof g_stats);
   const double wall0 = now_ms();
@@ -2740,8 +2894,9 @@ int roadsurf_run_ensemble_host_soa_onset(const RsHostBatch* b, const double* mem
     if (rc != RS_OK) return rc;
   }
   {
-    int rc = check_onset_outputs(*spec, onset, areas, area_prob, area_onset, false);
-    if (rc == RS_OK && areas) rc = check_areas(areas, P, *spec);
+    int rc = check_onset_outputs(*spec, onset, areas, area_prob, area_onset, false, area_ext_stats);
+    if (rc == RS_OK) rc = check_extremes(ext, ext_stats, areas, area_ext_stats, RS_O_NVAR, false);
+    if (rc == RS_OK && areas) rc = check_areas(areas, P, *spec, area_prob || area_onset);
     if (rc != RS_OK) return rc;
   }
   if (P > 0 && !member_records) return fail(RS_ERR_BAD_ARGUMENT, "null member_records");
@@ -2811,12 +2966,15 @@ int roadsurf_run_ensemble_host_soa_onset(const RsHostBatch* b, const double* mem
   const size_t srows = static_cast<size_t>(RS_ENS_NFIXED + nq) * RS_O_NVAR * n_m, prows = static_cast<size_t>(np_planes) * n_m;
   const int E = spec->n_events;
   const size_t orows = onset ? static_cast<size_t>(E) * n_m : 0;  // onset planes of a station
+  // window extremes: the work space [X][n_m] of every member lane and the ext_stats rows of a station
+  const int X = ext ? ext->n_extremes : 0;
+  const size_t xws = static_cast<size_t>(X) * n_m, xrows = ext_stats ? static_cast<size_t>(RS_ENS_NFIXED + nq) * xws : 0;
   // area onset: the workspace {O, X} of every member lane, E * 8 bytes
   const size_t per_station =
       sizeof(double) * (frows + RS_L_NLOCAL + (hor ? 360 : 0) + RS_O_NVAR * n_pre + NS + (cpl ? SC : 0) + 1 + srows + prows +
-                        orows) +
+                        orows + xrows) +
       sizeof(double) * M * (frows_m + RS_L_NLOCAL + (hor ? 360 : 0) + NS + (cpl ? SC : 0) + 1 + 3 + RS_O_NVAR * n_m +
-                            (area_onset ? E : 0));
+                            (area_onset ? E : 0) + xws);
   size_t free_b = 0, total_b = 0;
   CU(cudaMemGetInfo(&free_b, &total_b));
   // areas: the plan and the accumulators stay on the device for the whole call, beside area_prob and area_onset (the
@@ -2835,19 +2993,32 @@ int roadsurf_run_ensemble_host_soa_onset(const RsHostBatch* b, const double* mem
                                "ceil(n_out_m / 64) * members * 8 bytes; area_onset: n_areas * n_events * members * 8 "
                                "bytes) and the area outputs");
   }
+  // area window extremes: their own segments, the accumulators [X][n_m][n_areas * M] and area_ext_stats
+  const size_t area_xacc_n = area_ext_stats ? xws * areas->n_areas * M : 0;
+  const size_t area_xstats_n = area_ext_stats ? static_cast<size_t>(RS_ENS_NFIXED + nq) * xws * areas->n_areas : 0;
+  if (area_ext_stats)
+  {
+    area_fixed += sizeof(int) * 4 * area_plan.stations.size() + sizeof(double) * (area_xacc_n + area_xstats_n);
+    if (static_cast<double>(area_fixed) >= free_b * 0.8)
+      return fail(RS_ERR_CUDA, "not enough device memory for the area extreme accumulators (n_extremes * n_out_m * "
+                               "n_areas * members * 8 bytes) and area_ext_stats");
+  }
   long long pc = static_cast<long long>((free_b * 0.8 - static_cast<double>(area_fixed)) / per_station) - 64;
   if (const int cap = g_opt_max_slots.load()) pc = std::min<long long>(pc, std::max(1, cap / M));
   pc = std::min<long long>(pc, P);
   if (pc < 1) return fail(RS_ERR_CUDA, "not enough device memory for one station's members");
   const int ldc = static_cast<int>((pc + 31) / 32 * 32), ldmc = static_cast<int>((pc * M + 31) / 32 * 32);
-  std::vector<int> chunk_segments;  // [chunks + 1]: the segments of chunk c are [chunk_segments[c], chunk_segments[c + 1])
-  if (areas)
-  {
-    const int len = area_segment_length(area_plan, E, n_m, (P + pc - 1) / pc);
-    chunk_segments.push_back(0);
+  // [chunks + 1]: the segments of chunk c are [chunk_segments[c], chunk_segments[c + 1]), those of the area extremes
+  // [ext_segments[c], ext_segments[c + 1]), after the area events' in the same plan
+  std::vector<int> chunk_segments, ext_segments;
+  auto plan_chunks = [&](int len, std::vector<int>& first) {
+    first.push_back(static_cast<int>(area_plan.segments.size() / 4));
     for (long long p0 = 0; p0 < P; p0 += pc)
-      chunk_segments.push_back(chunk_segments.back() + plan_segments(area_plan, p0, std::min<long long>(pc, P - p0), len));
-  }
+      first.push_back(first.back() + plan_segments(area_plan, p0, std::min<long long>(pc, P - p0), len));
+  };
+  const long long chunks = (P + pc - 1) / pc;
+  if (area_prob || area_onset) plan_chunks(area_segment_length(area_plan, E, n_m, chunks), chunk_segments);
+  if (area_ext_stats) plan_chunks(segment_length(area_plan, X, chunks), ext_segments);
 
   SoaStreams* ss = nullptr;
   {
@@ -2910,6 +3081,16 @@ int roadsurf_run_ensemble_host_soa_onset(const RsHostBatch* b, const double* mem
     CU(pooled(dev, EH_ONSET_ACC, acc_ints, &d_onset_acc));
     CU(pooled(dev, EH_AREA_ONSET, std::max<size_t>(1, area_prob_n), &d_area_onset));
     CU(cudaMemsetAsync(d_onset_acc, 0x7f, sizeof(int) * acc_ints, st));
+  }
+  double *d_xws = nullptr, *d_xstats = nullptr, *d_xacc = nullptr, *d_area_xstats = nullptr;
+  const RsEnsembleStatsSpec xspec = extremes_spec(*spec);
+  if (ext) CU(pooled(dev, EH_EXT_WS, std::max<size_t>(1, xws * lm), &d_xws));
+  if (ext_stats) CU(pooled(dev, EH_EXT_STATS, std::max<size_t>(1, xrows * lc), &d_xstats));
+  if (area_ext_stats)
+  {
+    CU(pooled(dev, EH_EXT_ACC, std::max<size_t>(1, area_xacc_n), &d_xacc));
+    CU(pooled(dev, EH_AREA_EXT_STATS, std::max<size_t>(1, area_xstats_n), &d_area_xstats));
+    CU(static_cast<cudaError_t>(rs_init_ens_area_extremes(d_xacc, n_m, areas->n_areas, M, ext, st)));
   }
   g_stats.setup_ms = now_ms() - setup0;
   const int launches0 = g_launches_total.load();
@@ -2990,6 +3171,16 @@ int roadsurf_run_ensemble_host_soa_onset(const RsHostBatch* b, const double* mem
         rc = onset_area_finalize(d_onset_acc, areas->n_areas, E, n_m, M, d_area_onset, n_m, st);
       if (rc != RS_OK) return rc;
     }
+    if (ext)
+    {
+      int rc = extremes_launch(d_mo, n_m, e.n_out_members, ldm, n, M, xspec, ext, d_xws, ldm, d_xstats, n_m, ld, st);
+      if (rc == RS_OK && area_ext_stats)
+        rc = extremes_area_accumulate(d_areas, d_xws, n_m, ldm, M, ext, static_cast<int>(p0), ext_segments[chunk],
+                                      ext_segments[chunk + 1] - ext_segments[chunk], areas->n_areas, d_xacc, st);
+      if (rc == RS_OK && area_ext_stats && last)
+        rc = extremes_area_finalize(d_xacc, n_m, areas->n_areas, M, xspec, ext, d_area_xstats, n_m, st);
+      if (rc != RS_OK) return rc;
+    }
     CU(cudaEventRecord(ev[2], st));
     if (b->out && pre1 > pre0)
       CU(cudaMemcpy2DAsync(b->out + col, D * np, d_out, D * ld, D * n, static_cast<size_t>(RS_O_NVAR) * (pre1 - pre0),
@@ -3018,6 +3209,16 @@ int roadsurf_run_ensemble_host_soa_onset(const RsHostBatch* b, const double* mem
     {
       CU(cudaMemcpyAsync(area_onset, d_area_onset, D * area_prob_n, cudaMemcpyDeviceToHost, st));
       g_stats.d2h_bytes += D * area_prob_n;
+    }
+    if (ext_stats && n_m > 0)
+    {
+      CU(cudaMemcpy2DAsync(ext_stats + col, D * np, d_xstats, D * ld, D * n, xrows, cudaMemcpyDeviceToHost, st));
+      g_stats.d2h_bytes += D * n * xrows;
+    }
+    if (area_ext_stats && last && area_xstats_n > 0)
+    {
+      CU(cudaMemcpyAsync(area_ext_stats, d_area_xstats, D * area_xstats_n, cudaMemcpyDeviceToHost, st));
+      g_stats.d2h_bytes += D * area_xstats_n;
     }
     CU(cudaEventRecord(ev[3], st));
     CU(cudaStreamSynchronize(st));

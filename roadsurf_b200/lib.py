@@ -42,7 +42,8 @@ EXPORTS = ("runsimulation", "roadsurf_last_error", "roadsurf_device_count", "roa
            "roadsurf_version",
            "roadsurf_run_ensemble_device", "roadsurf_ensemble_stats", "roadsurf_run_ensemble_host_soa",
            "roadsurf_ensemble_area_events", "roadsurf_run_ensemble_host_soa_areas",
-           "roadsurf_ensemble_onset", "roadsurf_run_ensemble_host_soa_onset")
+           "roadsurf_ensemble_onset", "roadsurf_run_ensemble_host_soa_onset",
+           "roadsurf_ensemble_extremes", "roadsurf_run_ensemble_host_soa_extremes")
 (PRIM_EXP, PRIM_EXP_SMEM, PRIM_LOG, PRIM_LOG_SMEM, PRIM_EXP_FLAT, PRIM_EXP_FLAT_SMEM, PRIM_PSIH_UNSTABLE,
  PRIM_PSIH_UNSTABLE_SMEM, PRIM_FRCP, PRIM_FDIV, PRIM_DIV_CONST, PRIM_N) = range(12)
 ENS_MAX_MEMBERS, ENS_MAX_QUANTILES, ENS_MAX_THRESHOLDS = 128, 8, 8
@@ -50,6 +51,9 @@ ENS_MAX_EVENTS, ENS_MAX_CONDITIONS = 8, 4
 ENS_NVALID, ENS_MEAN, ENS_STD, ENS_MIN, ENS_MAX, ENS_NFIXED = range(6)
 ENS_LT, ENS_LE, ENS_GT, ENS_GE = range(4)
 ENS_OPS = {"<": ENS_LT, "<=": ENS_LE, ">": ENS_GT, ">=": ENS_GE}
+ENS_MAX_EXTREMES = 8
+ENS_WMIN, ENS_WMAX = 0, 1
+ENS_KINDS = {"min": ENS_WMIN, "max": ENS_WMAX}
 
 
 def state_nplanes(nlayers):
@@ -135,6 +139,29 @@ def ensemble_areas(station_lists):
     areas = RsEnsembleAreas(n_areas=len(lists), offsets=offsets.ctypes.data, stations=stations.ctypes.data)
     areas.offsets_array, areas.stations_array = offsets, stations
     return areas
+
+
+class RsEnsembleExtreme(C.Structure):
+    _fields_ = [("plane", C.c_int), ("kind", C.c_int), ("window", C.c_int)]
+
+
+class RsEnsembleExtremes(C.Structure):
+    _fields_ = [("n_extremes", C.c_int), ("extremes", RsEnsembleExtreme * ENS_MAX_EXTREMES)]
+
+
+def ensemble_extremes(extremes):
+    """RsEnsembleExtremes from [(plane, kind, window), ...], kind "min" or "max" (or an ENS_W* code): the minimum or
+    maximum of the plane over the window of output slots starting at each slot."""
+    extremes = list(extremes)
+    if not 1 <= len(extremes) <= ENS_MAX_EXTREMES:
+        raise ValueError("1 to 8 extremes")
+    ext = RsEnsembleExtremes(n_extremes=len(extremes))
+    for x, (plane, kind, window) in enumerate(extremes):
+        code = ENS_KINDS.get(kind, kind)
+        if code not in (ENS_WMIN, ENS_WMAX) or isinstance(code, bool):
+            raise ValueError(f"unknown extreme kind {kind!r}: 'min', 'max', ENS_WMIN or ENS_WMAX")
+        ext.extremes[x] = RsEnsembleExtreme(int(plane), code, int(window))
+    return ext
 
 
 def stats_spec(quantiles=(), thresholds=(), events=()):
@@ -250,6 +277,16 @@ def load():
                                                          C.c_void_p, P(RsEnsembleAreas), C.c_void_p, C.c_void_p,
                                                          C.c_void_p, P(IS), P(IPa)]
     lib.roadsurf_run_ensemble_host_soa_onset.restype = C.c_int
+    lib.roadsurf_ensemble_extremes.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                                               P(RsEnsembleStatsSpec), P(RsEnsembleExtremes), C.c_void_p, C.c_int,
+                                               P(RsEnsembleAreas), C.c_void_p, C.c_void_p]
+    lib.roadsurf_ensemble_extremes.restype = C.c_int
+    lib.roadsurf_run_ensemble_host_soa_extremes.argtypes = [P(RsHostBatch), C.c_void_p, C.c_int, C.c_int, C.c_void_p,
+                                                            P(RsEnsembleStatsSpec), C.c_void_p, C.c_void_p,
+                                                            C.c_void_p, C.c_void_p, P(RsEnsembleAreas), C.c_void_p,
+                                                            C.c_void_p, C.c_void_p, P(RsEnsembleExtremes),
+                                                            C.c_void_p, C.c_void_p, P(IS), P(IPa)]
+    lib.roadsurf_run_ensemble_host_soa_extremes.restype = C.c_int
     _lib = lib
     return lib
 
@@ -712,6 +749,28 @@ def ensemble_onset(member_out, npoints, members, spec, areas=None, onset=True, s
     return (None if on is None else on[..., :npoints]), area_on
 
 
+def ensemble_extremes_device(member_out, npoints, members, spec, ext, areas=None, stream=None):
+    """roadsurf_ensemble_extremes on a torch CUDA tensor member_out [out_nvar, n_out, ld_members] (lane
+    p * members + m); ext an RsEnsembleExtremes (ensemble_extremes), areas an RsEnsembleAreas (ensemble_areas) or None.
+    Returns (ext_stats [5 + n_quantiles, n_extremes, n_out, npoints], area_ext_stats
+    [5 + n_quantiles, n_extremes, n_out, n_areas] or None without areas) as CUDA tensors (synchronised)."""
+    import torch
+    out_nvar, n_out, ldm = member_out.shape
+    ld = max(32, (npoints + 31) // 32 * 32)
+    f64 = dict(dtype=torch.float64, device=member_out.device)
+    rows = (ENS_NFIXED + spec.n_quantiles, ext.n_extremes, n_out)
+    xs = torch.full(rows + (ld,), 12345.0, **f64)
+    area_xs = torch.full(rows + (areas.n_areas,), 12345.0, **f64) if areas is not None else None
+    st = stream if stream is not None else torch.cuda.current_stream()
+    _check(load().roadsurf_ensemble_extremes(member_out.data_ptr(), out_nvar, n_out, ldm, int(npoints), int(members),
+                                             C.byref(spec), C.byref(ext), xs.data_ptr(), ld,
+                                             None if areas is None else C.byref(areas),
+                                             None if area_xs is None else area_xs.data_ptr(),
+                                             C.c_void_p(st.cuda_stream)))
+    torch.cuda.synchronize()
+    return xs[..., :npoints], area_xs
+
+
 def fork_record(record_step, fork_step):
     """r_f: the last record at or before 0-based step fork_step - 1."""
     rs = np.asarray(record_step)
@@ -836,20 +895,24 @@ class EnsembleBatch:
 def run_ensemble_host_soa(settings, params, forcing, record_step, time_fields, local, member_records, members,
                           fork_step, spec, horizons=None, out_stride=1, coupling_window_end=0, out=None,
                           member_out=False, member_status=False, latest_obs_index=None, areas=None, prob=True,
-                          onset=False, area_prob=True):
-    """roadsurf_run_ensemble_host_soa_onset on host arrays: forcing [n_records, nvar, P], record_step [n_records],
+                          onset=False, area_prob=True, extremes=None, stats=True):
+    """roadsurf_run_ensemble_host_soa_extremes on host arrays: forcing [n_records, nvar, P], record_step [n_records],
     local [L_NLOCAL, P], member_records [n_records - r_f - 1, nvar, P * members], latest_obs_index [P] int32 (the
     relaxation rule of read_input_derive_records; None = no observations), areas an RsEnsembleAreas (ensemble_areas)
     or None.  Returns a dict with stats [5 + nq, 6, n_out_m, P], prob [nt + n_events, n_out_m, P] (unless prob=False:
     NULL is passed) and, when asked for, member_out [6, n_out_m, P * M], member_status [P * M] and area_prob
     [n_events, n_out_m, n_areas] (unless area_prob=False: NULL is passed).  With onset=True it also returns
-    onset [n_events, n_out_m, P] and, with areas, area_onset [n_events, n_out_m, n_areas]."""
+    onset [n_events, n_out_m, P] and, with areas, area_onset [n_events, n_out_m, n_areas].  With extremes (an
+    RsEnsembleExtremes, ensemble_extremes) it also returns ext_stats [5 + nq, n_extremes, n_out_m, P] and, with areas,
+    area_ext_stats [5 + nq, n_extremes, n_out_m, n_areas].  stats=False passes NULL for stats."""
     n_records, nvar, npoints = forcing.shape
     sim_len = time_fields.shape[1]
     k0 = fork_step - 1
     slot0 = (k0 + out_stride - 1) // out_stride
     n_m = (sim_len + out_stride - 1) // out_stride - slot0
-    res = dict(stats=np.zeros((ENS_NFIXED + spec.n_quantiles, O_NVAR, n_m, npoints)))
+    res = {}
+    if stats:
+        res["stats"] = np.zeros((ENS_NFIXED + spec.n_quantiles, O_NVAR, n_m, npoints))
     if prob:
         res["prob"] = np.zeros((spec.n_prob, n_m, npoints))
     if member_out:
@@ -862,14 +925,19 @@ def run_ensemble_host_soa(settings, params, forcing, record_step, time_fields, l
         res["onset"] = np.zeros((spec.n_events, n_m, npoints))
         if areas is not None:
             res["area_onset"] = np.zeros((spec.n_events, n_m, areas.n_areas))
+    if extremes is not None:
+        res["ext_stats"] = np.zeros((ENS_NFIXED + spec.n_quantiles, extremes.n_extremes, n_m, npoints))
+        if areas is not None:
+            res["area_ext_stats"] = np.zeros((ENS_NFIXED + spec.n_quantiles, extremes.n_extremes, n_m, areas.n_areas))
     hb = RsHostBatch(npoints=npoints, sim_len=sim_len, forcing_mode=1, n_records=n_records, nvar=nvar,
                      out_stride=out_stride, forcing=_ptr(forcing), record_step=_ptr(record_step),
                      time_fields=_ptr(time_fields), local=_ptr(local), horizons=_ptr(horizons), out=_ptr(out),
                      coupling_window_end=int(coupling_window_end))
     lat = None if latest_obs_index is None else np.ascontiguousarray(latest_obs_index, dtype=np.int32)
-    _check(load().roadsurf_run_ensemble_host_soa_onset(
-        C.byref(hb), _ptr(member_records), int(members), int(fork_step), _ptr(lat), C.byref(spec), _ptr(res["stats"]),
-        _ptr(res.get("prob")), _ptr(res.get("member_out")), _ptr(res.get("member_status")),
+    _check(load().roadsurf_run_ensemble_host_soa_extremes(
+        C.byref(hb), _ptr(member_records), int(members), int(fork_step), _ptr(lat), C.byref(spec),
+        _ptr(res.get("stats")), _ptr(res.get("prob")), _ptr(res.get("member_out")), _ptr(res.get("member_status")),
         None if areas is None else C.byref(areas), _ptr(res.get("area_prob")), _ptr(res.get("onset")),
-        _ptr(res.get("area_onset")), C.byref(settings), C.byref(params)))
+        _ptr(res.get("area_onset")), None if extremes is None else C.byref(extremes), _ptr(res.get("ext_stats")),
+        _ptr(res.get("area_ext_stats")), C.byref(settings), C.byref(params)))
     return res
